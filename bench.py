@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched with torchrun)
     python bench.py --impl reference --steps K --warmup W    (CPU oracle port on the host cores)
+    python bench.py --steps K --warmup W --dump-outputs DIR  (also writes the last timed step's outputs to DIR/*.npy)
 
 A "step" is one tracking iteration of BASELINE.json configs[1] (Replica room0-shaped 1200x680,
 ~1.0 M view-tied Gaussians): fused six-plane render -> masked-L1 tracking loss -> backward to
@@ -262,6 +263,30 @@ def load_counters(name):
         return {}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, solver, N):
+    """Writes what the timed path's last step handed its caller as float32 <name>.npy files: the pose after the step's
+    Adam update, the step's pose gradient and loss terms, the best (loss, pose) so far, and the step's six-plane render
+    and radii.  Arrays of more than 4096 elements are replaced by a fixed seeded sample of their flattened elements
+    (sorted indices) when the whole would exceed DUMP_BYTES, so two builds can be compared output for output."""
+    outs = {"cam_unnorm_rot": solver.cam_q, "cam_trans": solver.cam_t, "pose_grad": solver.msg[0:7],
+            "loss_terms": solver.loss_terms(), "best": solver.best, "image6": solver.r.image6, "radii": solver.r.radii[:N]}
+    arrs = {k: t.detach().cpu().numpy().astype(np.float32) for k, t in outs.items()}
+    big = sorted(k for k, a in arrs.items() if a.size > 4096)
+    room = DUMP_BYTES - sum(a.nbytes for k, a in arrs.items() if k not in big)
+    big_bytes = sum(arrs[k].nbytes for k in big)
+    if big_bytes > room:
+        for k in big:
+            n = arrs[k].size
+            idx = np.sort(np.random.default_rng(0).choice(n, n * room // big_bytes, replace=False))
+            arrs[k] = arrs[k].reshape(-1)[idx]
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def run_tracking(args, wl, rank, world, dev, pg):
     """The headline leg.  -> dict of everything measured (rank 0 assembles the JSON line)."""
     import torch
@@ -316,6 +341,8 @@ def run_tracking(args, wl, rank, world, dev, pg):
         solver.step()
     e1.record()
     sync_all()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, solver, N)
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -879,6 +906,7 @@ def run_ours(args, wl):
 
 
 def main():
+    sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (it may be read-only)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=200)
@@ -894,7 +922,16 @@ def main():
     ap.add_argument("--mode", default="tracking", choices=["tracking", "mapping"],
                     help="tracking = configs[1] (the driver's line, which also carries the mapping block); mapping = only the keyframe-sharded leg")
     ap.add_argument("--keyframes", type=int, default=8, help="--mode mapping: keyframes per mapping iteration (configs[2]: 8)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed tracking step computed as DIR/<name>.npy "
+                         "(float32, at most 64 MB; rank 0's arrays when --gpus > 1, whose render covers its tile band only). "
+                         "The order of the backward's float atomics moves them slightly from run to run; with --deterministic "
+                         "they repeat bitwise")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.mode == "mapping"):
+        ap.error("--dump-outputs writes the outputs of the GPU tracking path: not with --impl reference or --mode mapping")
     rank, world, local = dist_env()
     kind = "small" if args.small else args.workload
     if args.impl == "reference":
