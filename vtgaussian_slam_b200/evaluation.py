@@ -13,7 +13,7 @@ import torch
 
 from . import _lib, metrics
 from .fused import FusedRenderer
-from .rasterizer import _ptr, _stream_ptr
+from .rasterizer import _ptr, _stream_ptr, run_fitting
 from .slam_loop import quat_from_matrix
 
 
@@ -38,10 +38,7 @@ class FrameEvaluator:
         q = torch.as_tensor(quat_from_matrix(M[:3, :3]), dtype=torch.float32, device=self.device)
         t = torch.as_tensor(M[:3, 3], dtype=torch.float32, device=self.device)
         r = self.renderer(int(params["means3D"].shape[0]))
-        for _ in range(3):
-            image6, _ = r.forward(params, q, t)
-            if not r.ensure_capacity():
-                break
+        image6, _ = run_fitting(lambda: r.forward(params, q, t), [r])
         return image6
 
     def frame_metrics(self, image6, gt_rgb, gt_depth, sil_thres, use_presence=False, want_ssim=True):

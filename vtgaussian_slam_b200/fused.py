@@ -18,7 +18,8 @@ import os
 import torch
 
 from . import _lib
-from .rasterizer import _PAIR_RATIO, Workspace, _ptr, _require_cuda, _stream_ptr, camera_struct
+from .rasterizer import (Workspace, _ptr, _require_cuda, _stream_ptr, _tensor_bytes, camera_struct, grown_pair_capacity,
+                         initial_pair_capacity, run_fitting)
 
 PARAM_KEYS = ("means3D", "rgb_colors", "unnorm_rotations", "logit_opacities", "log_scales")
 
@@ -26,9 +27,9 @@ PARAM_KEYS = ("means3D", "rgb_colors", "unnorm_rotations", "logit_opacities", "l
 class FusedRenderer:
     """Persistent buffers for rendering N view-tied Gaussians into a W x H frame.
 
-    pair_capacity bounds R = sum(tiles_touched); the library never reads R back.  Poll
-    `overflowed()` (one tiny D2H) when convenient -- e.g. once per frame -- and call
-    `reserve_pairs` to grow."""
+    pair_capacity bounds R = sum(tiles_touched); the library never reads R back.  Run the work
+    through `run_fitting` with a poll when a blocking read is cheap -- e.g. once per frame --
+    and it is repeated with grown pair buffers if a render was truncated."""
 
     def __init__(self, settings, num_gaussians, device="cuda:0", pair_capacity=None, tile_rows=(0, 0),
                  depth_row=(0.0, 0.0, 1.0, 0.0), deterministic=None):
@@ -38,9 +39,7 @@ class FusedRenderer:
         self.cam = camera_struct(settings, tile_rows=tile_rows)
         self.W, self.H, self.N = self.cam.image_width, self.cam.image_height, int(num_gaussians)
         if pair_capacity is None:
-            # R / N observed on this device so far (view-tied sections: ~2 tiles per Gaussian), with head room; a
-            # renderer that still overflows is grown by ensure_capacity() and the forward repeated
-            pair_capacity = int(self.N * max(6.0, 1.5 * _PAIR_RATIO.get(self.device, 0.0))) + 65536
+            pair_capacity = initial_pair_capacity(self.device, self.N)
         # deterministic: fixed-point gradient accumulation (rasterizer.set_deterministic is the default when None)
         self.ws = Workspace(self.device, self.W, self.H, self.N, pair_capacity, deterministic=deterministic)
         self.ws.ensure_grad_geom()
@@ -56,36 +55,33 @@ class FusedRenderer:
         self._map_scratch = None
         self._median_state = None
         self._sil = None                    # [0:10] ladder sums, [10] chosen threshold, [11] its MSE
-        self._bufs = self.ws.struct()
+        self._bufs, self._bufs_generation = self.ws.struct(), self.ws.generation
         self.polls = 0
         self._step_graphs = {}              # tracking_step_cached: pointer set -> captured launch sequence
         self._cap_stream = None
 
     # -- helpers ---------------------------------------------------------------------------
-    def reserve_pairs(self, cap):
-        self.ws.reserve_pairs(cap)
-        self._bufs = self.ws.struct()
-        self._step_graphs.clear()           # the captured launches point into the old buffers
+    def _buffers(self):
+        """The workspace's VtgsBuffers.  When the pair buffers have been reallocated since it was built, it is rebuilt
+        and the step graphs, whose launches point into the old buffers, are dropped."""
+        if self._bufs_generation != self.ws.generation:
+            self._bufs, self._bufs_generation = self.ws.struct(), self.ws.generation
+            self._step_graphs.clear()
+        return self._bufs
 
     def overflowed(self):
         R, overflow, _ = self.ws.read_counters()
-        if self.N > 0:
-            _PAIR_RATIO[self.device] = max(_PAIR_RATIO.get(self.device, 0.0), R / self.N)
         return bool(overflow), R
 
     def ensure_capacity(self):
         """One blocking read of the device counters.  -> True if the last forward overflowed the pair buffers: they
         have been enlarged and the forward (and everything derived from it) must be repeated."""
-        overflow, R = self.overflowed()
-        if overflow:
-            self.reserve_pairs(int(R * 1.5) + 65536)
-        return overflow
+        return self.ws.ensure_capacity()
 
     @property
     def nbytes(self):
-        """Approximate device memory held by this renderer (pool accounting in slam_ops)."""
-        cap, P = self.ws.pair_capacity, self.W * self.H
-        return int(self.N * (64 + 4 + 64 + 4) + cap * (8 + 4 + 64 + 32) + P * (6 + 4 + 2 + 12) * 4)
+        """Device memory held by this renderer's tensors and its workspace's (pool accounting in slam_ops)."""
+        return self.ws.nbytes + _tensor_bytes(self)
 
     def median_state(self, image6=None, gt_depth=None, process_group=None, num_pixels_total=None):
         """Radix-select state of median(|gt - depth| (gt > 0)) over the frame (reference :525-527, :757-758) for the
@@ -166,7 +162,7 @@ class FusedRenderer:
         p, ps = self._params_struct(params), self._pose_struct(cam_q, cam_t)
         with torch.cuda.device(self.device):
             _lib.check(_lib.lib().vtgs_fused_forward(C.byref(self.cam), C.byref(p), C.byref(ps), _ptr(self.image6),
-                                                     _ptr(self.radii), C.byref(self._bufs), _stream_ptr(self.device)))
+                                                     _ptr(self.radii), C.byref(self._buffers()), _stream_ptr(self.device)))
         return self.image6, self.radii[:self.N]
 
     def tracking_loss(self, gt_rgb, gt_depth, w_im=0.5, w_depth=0.025, use_sil_for_loss=True, sil_thres=0.99,
@@ -216,7 +212,7 @@ class FusedRenderer:
             _lib.check(_lib.lib().vtgs_fused_tracking_step(
                 C.byref(self.cam), C.byref(p), C.byref(ps), C.byref(cfg), _ptr(gt_rgb), _ptr(gt_depth), _ptr(self.image6),
                 _ptr(self.radii), _ptr(self.dL_dimage4), _ptr(self.loss_terms), _ptr(self._loss_scratch), C.byref(g),
-                _ptr(max_2D_radius), _ptr(seen), C.byref(self._bufs), _stream_ptr(self.device)))
+                _ptr(max_2D_radius), _ptr(seen), C.byref(self._buffers()), _stream_ptr(self.device)))
         return self.loss_terms, self.radii[:self.N]
 
     STEP_GRAPHS_MAX = 8
@@ -227,6 +223,7 @@ class FusedRenderer:
         settings captures the launch sequence in a CUDA graph, later ones replay it (one launch, and back-to-back kernels
         overlap their tails as in TrackingSolver).  The entry owns the outputs that must not move: -> (loss_terms, radii,
         pose_grad[7] = d_cam_q | d_cam_t, seen or None), valid until the entry's next call."""
+        self._buffers()                     # (drops the graphs of reallocated pair buffers)
         pm = cfg.get("pixel_mask")
         key = (tuple(params[k].data_ptr() for k in PARAM_KEYS), cam_q.data_ptr(), cam_t.data_ptr(), gt_rgb.data_ptr(), gt_depth.data_ptr(),
                0 if pm is None else pm.data_ptr(), 0 if max_2D_radius is None else max_2D_radius.data_ptr(),
@@ -300,7 +297,7 @@ class FusedRenderer:
         dL = self.dL_dimage4 if dL_dimage4 is None else dL_dimage4
         with torch.cuda.device(self.device):
             _lib.check(_lib.lib().vtgs_fused_backward(C.byref(self.cam), C.byref(p), C.byref(ps), _ptr(dL), int(bool(accumulate)),
-                                                      C.byref(g), C.byref(self._bufs), _stream_ptr(self.device)))
+                                                      C.byref(g), C.byref(self._buffers()), _stream_ptr(self.device)))
 
 
 def book_radii(radii, max_2D_radius, seen=None):
@@ -400,6 +397,7 @@ class TrackingSolver:
         self.use_graph = use_graph
         self._graph = None
         self._graph0 = None              # the frame's first iteration when it differs (replica_sil_search)
+        self._graph_generation = None    # the renderer's workspace generation the graphs were captured on
         self._it = 0                     # iterations since set_frame
         self._init = None
 
@@ -465,6 +463,9 @@ class TrackingSolver:
         if not self.use_graph:
             self._iteration(first)
             return
+        if self._graph_generation != self.r.ws.generation:          # captured launches point into the pair buffers
+            self._graph = self._graph0 = None
+            self._graph_generation = self.r.ws.generation
         if first:
             if self._graph0 is None:
                 self._graph0 = self._capture(True)
@@ -481,14 +482,13 @@ class TrackingSolver:
 
     def check(self, grow=True, raise_on_overflow=True):
         """One blocking read of the device counters (call once per frame, not per iteration).  If the pair buffers
-        overflowed (R > pair_capacity: the renders of this frame were truncated) they are enlarged (grow=True) and the
-        captured graphs dropped; then either raises or returns None so that the caller re-runs the frame
-        (`run_frame` does).  -> R otherwise."""
+        overflowed (R > pair_capacity: the renders of this frame were truncated) they are enlarged (grow=True; the
+        captured graphs follow them at the next step); then either raises or returns None so that the caller re-runs the
+        frame (`run_frame` does).  -> R otherwise."""
         overflow, R = self.r.overflowed()
         if overflow:
             if grow:
-                self.r.reserve_pairs(int(R * 1.5) + 65536)
-                self._graph = self._graph0 = None          # buffer addresses changed: re-capture
+                self.r.ws.reserve_pairs(grown_pair_capacity(R))
             if raise_on_overflow:
                 raise _lib.VtgsError(f"pair buffer overflow: R = {R} > capacity; buffers "
                                      f"{'were grown -- re-run the frame' if grow else 'unchanged'}")
@@ -499,14 +499,7 @@ class TrackingSolver:
         """num_iters iterations from the pose given to set_frame, one blocking read of the result, and -- if the pair
         buffers turned out too small for this frame -- a transparent re-run with larger ones.
         -> best[8] on the host: (best loss, best cam_unnorm_rot[4], best cam_trans[3])."""
-        for attempt in range(3):
-            for _ in range(num_iters):
-                self.step()
-            best = self.best.cpu()
-            if self.check(grow=True, raise_on_overflow=False) is not None:
-                return best
-            self._reset_pose()
-        raise _lib.VtgsError("pair buffer overflow persisted after regrowing")
+        return self.run_frame_with_metric(num_iters, None)
 
     def run_frame_with_metric(self, num_iters, metric_fn):
         """run_frame with the reference's `choose_metric` of a section's base frame (:1891-1970): after every Adam step
@@ -514,19 +507,18 @@ class TrackingSolver:
         to the overlapping keyframe, keyframes.point2plane_dist) ranks the candidate, and the pose with the smallest
         metric is kept.  One blocking pose read per iteration -- the reference runs an Open3D KD-tree there.
         -> best[8] on the host: (best metric, cam_unnorm_rot[4], cam_trans[3])."""
-        for attempt in range(3):
+        def frame():
             best = torch.full((8,), float("inf"))
             for _ in range(num_iters):
                 self.step()
-                q, t = self.cam_q.cpu(), self.cam_t.cpu()
-                m = float(metric_fn(q, t))
-                if m < float(best[0]):
-                    best[0] = m
-                    best[1:5], best[5:8] = q, t
-            if self.check(grow=True, raise_on_overflow=False) is not None:
-                return best
-            self._reset_pose()
-        raise _lib.VtgsError("pair buffer overflow persisted after regrowing")
+                if metric_fn is not None:
+                    q, t = self.cam_q.cpu(), self.cam_t.cpu()
+                    m = float(metric_fn(q, t))
+                    if m < float(best[0]):
+                        best[0] = m
+                        best[1:5], best[5:8] = q, t
+            return self.best.cpu() if metric_fn is None else best
+        return run_fitting(frame, [self.r], on_regrow=self._reset_pose)
 
 
 class MappingSolver:
@@ -665,53 +657,47 @@ class MappingSolver:
         self.total_loss += loss
         r.backward(params, kf["cam_q"], kf["cam_t"], dL_dimage4=dL4, param_grads=grads, pose_grads=pose, accumulate=accumulate)
 
+    def _gradients(self, keyframes, loss_fn, w_im, w_depth, do_ba):
+        """Loss and gradients of one iteration over `keyframes`, nothing updated yet: repeatable."""
+        self.total_loss.zero_()
+        first = True
+        for kf in keyframes:
+            pose = None
+            if do_ba:
+                st = kf.setdefault("_ba", None)
+                if st is None:
+                    z = lambda n: torch.zeros(n, dtype=torch.float32, device=self.device)
+                    st = kf["_ba"] = dict(d_q=z(4), d_t=z(3), m_q=z(4), v_q=z(4), m_t=z(3), v_t=z(3), old_q=z(4), old_t=z(3),
+                                          step=torch.zeros(1, dtype=torch.int32, device=self.device))
+                pose = (st["d_q"], st["d_t"])
+            self._render_backward(self.r, self.params, kf, self.grads, not first, loss_fn, w_im, w_depth, pose)
+            first = False
+            if self.r_global is not None and kf.get("global", True):
+                N = self.params["means3D"].shape[0]
+                if not self._global_aliases:
+                    for k in PARAM_KEYS:
+                        self.gparams[k][-N:].copy_(self.params[k])
+                gpose = None
+                if do_ba:
+                    st = kf["_ba"]
+                    gpose = (st.setdefault("gd_q", torch.zeros_like(st["d_q"])), st.setdefault("gd_t", torch.zeros_like(st["d_t"])))
+                self._render_backward(self.r_global, self.gparams, kf, self.ggrads, False, loss_fn, w_im, w_depth, gpose)
+                for k in self.lrs:
+                    self.grads[k] += self.ggrads[k][-N:]
+                if do_ba:
+                    st["d_q"] += st["gd_q"]
+                    st["d_t"] += st["gd_t"]
+        if first:
+            for g in self.grads.values():
+                g.zero_()
+
     def iteration(self, keyframes, loss_fn=None, w_im=1.0, w_depth=1.0, do_ba=False):
         """keyframes: list of dict(cam_q, cam_t, gt_rgb, gt_depth[, global=True][, retie_last=n]) owned by THIS rank.
         loss_fn=None uses the fused mapping loss kernels (FusedRenderer.mapping_loss)."""
         poll = self.poll_every > 0 and self._iters % self.poll_every == 0
-        for attempt in range(3):
-            self.total_loss.zero_()
-            first = True
-            for kf in keyframes:
-                pose = None
-                if do_ba:
-                    st = kf.setdefault("_ba", None)
-                    if st is None:
-                        z = lambda n: torch.zeros(n, dtype=torch.float32, device=self.device)
-                        st = kf["_ba"] = dict(d_q=z(4), d_t=z(3), m_q=z(4), v_q=z(4), m_t=z(3), v_t=z(3), old_q=z(4), old_t=z(3),
-                                              step=torch.zeros(1, dtype=torch.int32, device=self.device))
-                    pose = (st["d_q"], st["d_t"])
-                self._render_backward(self.r, self.params, kf, self.grads, not first, loss_fn, w_im, w_depth, pose)
-                first = False
-                if self.r_global is not None and kf.get("global", True):
-                    N = self.params["means3D"].shape[0]
-                    if not self._global_aliases:
-                        for k in PARAM_KEYS:
-                            self.gparams[k][-N:].copy_(self.params[k])
-                    gpose = None
-                    if do_ba:
-                        st = kf["_ba"]
-                        gpose = (st.setdefault("gd_q", torch.zeros_like(st["d_q"])), st.setdefault("gd_t", torch.zeros_like(st["d_t"])))
-                    self._render_backward(self.r_global, self.gparams, kf, self.ggrads, False, loss_fn, w_im, w_depth, gpose)
-                    for k in self.lrs:
-                        self.grads[k] += self.ggrads[k][-N:]
-                    if do_ba:
-                        st["d_q"] += st["gd_q"]
-                        st["d_t"] += st["gd_t"]
-            if first:
-                for g in self.grads.values():
-                    g.zero_()
-            if not poll:
-                break
-            # pair-buffer overflow check (one blocking read every `poll_every` iterations, before anything is updated):
-            # a truncated render would give a wrong loss and wrong gradients without any error
-            grew = self.r.ensure_capacity()
-            if self.r_global is not None:
-                grew = self.r_global.ensure_capacity() or grew
-            if not grew:
-                break
-        else:
-            raise _lib.VtgsError("pair buffer overflow persisted after regrowing")
+        # the overflow check (one blocking read every `poll_every` iterations) comes before anything is updated
+        run_fitting(lambda: self._gradients(keyframes, loss_fn, w_im, w_depth, do_ba),
+                    [self.r] if self.r_global is None else [self.r, self.r_global], poll=poll)
         self._iters += 1
         self.step_dev.add_(1)
         if self.sharded is not None:

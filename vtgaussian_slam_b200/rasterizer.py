@@ -105,19 +105,23 @@ def set_deterministic(on: bool):
     _DETERMINISTIC = bool(on)
 
 
+def _tensor_bytes(obj):
+    return sum(t.nbytes for t in vars(obj).values() if isinstance(t, torch.Tensor))
+
+
 class Workspace:
-    """Device buffers of one forward (VtgsBuffers), owned as torch tensors.  Pair buffers grow
-    geometrically; `grad_geom` must be zero on entry to a backward and is left zeroed by it."""
+    """Device buffers of one forward (VtgsBuffers), owned as torch tensors and sized by `vtgs_workspace_query`.
+    `generation` counts the reallocations of the pair buffers: what holds their addresses (a VtgsBuffers struct, a
+    captured CUDA graph) is stale when it changes.  `grad_geom` must be zero on entry to a backward and is left zeroed by it."""
 
     def __init__(self, device, width, height, n, pair_capacity, deterministic=None):
         self.device, self.W, self.H, self.N = device, int(width), int(height), int(n)
         self.deterministic = deterministic                 # None: follow set_deterministic()
-        sz = _lib.VtgsWorkspaceSizes()
-        _lib.check(_lib.lib().vtgs_workspace_query(self.W, self.H, self.N, int(pair_capacity), C.byref(sz)))
+        sz = self._query(pair_capacity)
         u8 = dict(dtype=torch.uint8, device=device)
         self.tiles = (sz.tiles_x, sz.tiles_y)
         self.geom = torch.empty(sz.geom_bytes, **u8)
-        self.tiles_touched = torch.empty(max(self.N, 1), dtype=torch.int32, device=device)
+        self.tiles_touched = torch.empty(sz.tiles_touched_bytes // 4, dtype=torch.int32, device=device)
         self.tile_counts = torch.empty(sz.tile_counts_bytes // 4, dtype=torch.int32, device=device)
         self.tile_ranges = torch.empty((sz.tile_ranges_bytes // 8, 2), dtype=torch.int32, device=device)
         self.final_T = torch.empty((self.H, self.W), dtype=torch.float32, device=device)
@@ -129,20 +133,31 @@ class Workspace:
         self.band_flags = torch.zeros(max(int(sz.band_flags_bytes), 1), dtype=torch.uint8, device=device)
         self.band_cand = torch.zeros(max(int(sz.band_cand_bytes) // 4, 1), dtype=torch.int32, device=device)
         self.tile_order = torch.zeros(max(int(sz.tile_order_bytes) // 4, 1), dtype=torch.int32, device=device)
-        self.region_pairs = self.region_masks = None
-        self._num_tiles = sz.tiles_x * sz.tiles_y
-        self.pair_capacity = 0
-        self.pair_keys = self.point_list = None
+        self.pair_keys = self.point_list = self.region_pairs = self.region_masks = None
+        self.pair_capacity = self.generation = 0
+        self.num_rendered = None                            # R of the last read_counters()
         self.reserve_pairs(pair_capacity)
+
+    def _query(self, pair_capacity):
+        sz = _lib.VtgsWorkspaceSizes()
+        _lib.check(_lib.lib().vtgs_workspace_query(self.W, self.H, self.N, int(pair_capacity), C.byref(sz)))
+        return sz
 
     def reserve_pairs(self, cap):
         cap = max(int(cap), 1)
         if cap > self.pair_capacity:
-            self.pair_keys = torch.empty(cap, dtype=torch.int64, device=self.device)
-            self.point_list = torch.empty(cap, dtype=torch.int32, device=self.device)
-            self.region_pairs = torch.empty((8 * cap, 2), dtype=torch.int32, device=self.device)
-            self.region_masks = torch.empty(8 * (cap + 32 * self._num_tiles), dtype=torch.int32, device=self.device)
+            sz = self._query(cap)
+            self.pair_keys = torch.empty(sz.pair_keys_bytes // 8, dtype=torch.int64, device=self.device)
+            self.point_list = torch.empty(sz.point_list_bytes // 4, dtype=torch.int32, device=self.device)
+            self.region_pairs = torch.empty((sz.region_pairs_bytes // 8, 2), dtype=torch.int32, device=self.device)
+            self.region_masks = torch.empty(sz.region_masks_bytes // 4, dtype=torch.int32, device=self.device)
             self.pair_capacity = cap
+            self.generation += 1
+
+    @property
+    def nbytes(self):
+        """Memory held by the workspace's tensors (a shared grad_geom included)."""
+        return _tensor_bytes(self)
 
     def ensure_grad_geom(self):
         if self.grad_geom is None:
@@ -174,15 +189,51 @@ class Workspace:
         return b
 
     def read_counters(self):
-        """Blocking D2H read of (num_rendered, overflow, max_tile_pairs)."""
+        """Blocking D2H read of (num_rendered, overflow, max_tile_pairs).  R / N also raises the device's estimate that
+        sizes new pair buffers (initial_pair_capacity)."""
         c = self.counters[:3].cpu().tolist()
-        return int(c[0]) & 0xFFFFFFFF, int(c[1]), int(c[2])
+        R = self.num_rendered = int(c[0]) & 0xFFFFFFFF
+        if self.N > 0:
+            _PAIR_RATIO[self.device] = max(_PAIR_RATIO.get(self.device, 0.0), R / self.N)
+        return R, int(c[1]), int(c[2])
+
+    def ensure_capacity(self):
+        """One blocking read of the device counters.  -> True if the last forward overflowed the pair buffers: they
+        have been enlarged and the forward (and everything derived from it) must be repeated."""
+        R, overflow, _ = self.read_counters()
+        if overflow:
+            self.reserve_pairs(grown_pair_capacity(R))
+        return bool(overflow)
 
 
 # grad_geom scratch is left zeroed by every backward: share one per (device, N)
 _GRAD_GEOM_CACHE: dict = {}
-# last observed pairs-per-Gaussian ratio per device: sizes the next forward's pair buffers
+# largest pairs-per-Gaussian ratio R / N read back on each device so far (it never decreases)
 _PAIR_RATIO: dict = {}
+
+
+def initial_pair_capacity(device, n):
+    """Pair capacity of a new workspace for n Gaussians: the device's R / N estimate (view-tied sections: ~2 tiles per
+    Gaussian) with head room.  A forward that still overflows is grown by ensure_capacity() and repeated."""
+    return int(n * max(6.0, 1.5 * _PAIR_RATIO.get(torch.device(device), 0.0))) + 65536
+
+
+def grown_pair_capacity(R):
+    """Pair capacity after a forward that needed R pairs."""
+    return int(R * 1.5) + 65536
+
+
+def run_fitting(work, renderers, poll=True, on_regrow=None, attempts=3):
+    """-> work(), run until its renders fit (a truncated render gives a wrong loss and wrong gradients without any
+    error).  With `poll` each of `renderers` (a Workspace, a fused.FusedRenderer) reads its counters once after the run;
+    if any overflowed, they grow, on_regrow() resets what the run advanced and work() runs again; VtgsError after `attempts`."""
+    for _ in range(attempts):
+        out = work()
+        if not poll or not any([r.ensure_capacity() for r in renderers]):
+            return out
+        if on_regrow is not None:
+            on_regrow()
+    raise _lib.VtgsError("pair buffer overflow persisted after regrowing")
 
 
 def _require_cuda(name, t):
@@ -199,8 +250,7 @@ def rasterize_forward(cam: _lib.VtgsCamera, means3D, scales, rotations, opacitie
     W, H = cam.image_width, cam.image_height
     f32 = lambda t: t.detach().contiguous().float()
     means3D, scales, rotations, opacities, colors = map(f32, (means3D, scales, rotations, opacities, colors))
-    ratio = _PAIR_RATIO.get(dev, 4.0)
-    ws = Workspace(dev, W, H, N, int(N * ratio * 1.25) + 4096)
+    ws = Workspace(dev, W, H, N, initial_pair_capacity(dev, N))
     key = (dev, N)
     gg = _GRAD_GEOM_CACHE.get(key)
     if gg is None:
@@ -212,22 +262,14 @@ def rasterize_forward(cam: _lib.VtgsCamera, means3D, scales, rotations, opacitie
     depth = torch.empty((1, H, W), dtype=torch.float32, device=dev)
     radii = torch.zeros(N, dtype=torch.int32, device=dev)
     L = _lib.lib()
+
+    def forward():
+        _lib.check(L.vtgs_forward(C.byref(cam), N, _ptr(means3D), _ptr(scales), _ptr(rotations), _ptr(opacities),
+                                  _ptr(colors), _ptr(color), _ptr(depth), _ptr(radii), C.byref(ws.struct()), _stream_ptr(dev)))
     with torch.cuda.device(dev):
-        for attempt in range(2):
-            b = ws.struct()
-            _lib.check(L.vtgs_forward(C.byref(cam), N, _ptr(means3D), _ptr(scales), _ptr(rotations), _ptr(opacities),
-                                      _ptr(colors), _ptr(color), _ptr(depth), _ptr(radii), C.byref(b), _stream_ptr(dev)))
-            # like the reference binding (one blocking D2H of num_rendered per forward): the drop-in
-            # API sizes its pair buffers from it.  The fused path (fused.py) never synchronises.
-            R, overflow, _ = ws.read_counters()
-            if N > 0:
-                _PAIR_RATIO[dev] = max(R / N, 0.5)
-            if not overflow:
-                break
-            ws.reserve_pairs(R + 1024)
-        else:
-            raise _lib.VtgsError("pair buffer overflow persisted after regrowing")
-    ws.num_rendered = R
+        # like the reference binding (one blocking D2H of num_rendered per forward): the drop-in API
+        # polls every forward.  The fused path (fused.py) never synchronises inside an iteration.
+        run_fitting(forward, [ws])
     ws.saved_inputs = (means3D, scales, rotations, opacities, colors)
     return color, depth, radii, ws
 

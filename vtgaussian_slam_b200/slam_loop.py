@@ -31,7 +31,7 @@ import numpy as np
 import torch
 
 from .fused import MappingSolver, TrackingSolver
-from .rasterizer import GaussianRasterizationSettings
+from .rasterizer import GaussianRasterizationSettings, run_fitting
 from . import synthetic
 
 
@@ -293,10 +293,7 @@ class ViewTiedSLAM:
         M = self.w2c[idx]
         q = torch.as_tensor(quat_from_matrix(M[:3, :3]), dtype=torch.float32, device=self.device)
         t = torch.as_tensor(M[:3, 3], dtype=torch.float32, device=self.device)
-        for _ in range(2):
-            tr.r.forward(tr.params, q, t)
-            if not tr.r.ensure_capacity():
-                break
+        run_fitting(lambda: tr.r.forward(tr.params, q, t), [tr.r])
         mask, count = tr.r.nonpresence_mask(depth, sil_thres=sil_thres)
         if int(count.item()) == 0:
             return 0

@@ -23,6 +23,7 @@ import torch.nn.functional as F
 
 from .rasterizer import GaussianRasterizationSettings as Camera
 from .rasterizer import GaussianRasterizer as Renderer
+from .rasterizer import run_fitting
 
 
 # ---------------------------------------------------------------------------- small ops
@@ -283,17 +284,6 @@ def _give_grad(means2D, grad):
         means2D.grad += grad
 
 
-def _forward_checked(renderer, params, q, t, poll):
-    """renderer.forward, repeated with larger pair buffers if it overflowed them (checked when `poll`: one blocking
-    read of the device counters -- a truncated render gives a wrong loss and wrong gradients without any error)."""
-    img, radii = renderer.forward(params, q, t)
-    if poll and renderer.ensure_capacity():
-        img, radii = renderer.forward(params, q, t)
-        if renderer.ensure_capacity():
-            raise RuntimeError("pair buffer overflow persisted after regrowing")
-    return img, radii
-
-
 def _poll_due(renderer, tracking_iteration=None):
     """Poll the overflow counter on a renderer's first use, at the first tracking iteration of a frame, and every 16th
     call otherwise."""
@@ -311,7 +301,7 @@ class _FusedRender(torch.autograd.Function):
                       unnorm_rotations=unnorm_rot.detach().contiguous(), logit_opacities=logit_op.detach().contiguous(),
                       log_scales=log_scales.detach().contiguous())
         q, t = cam_q.detach().contiguous().reshape(4), cam_t.detach().contiguous().reshape(3)
-        img, radii = _forward_checked(renderer, params, q, t, _poll_due(renderer))
+        img, radii = run_fitting(lambda: renderer.forward(params, q, t), [renderer], poll=_poll_due(renderer))
         renderer.pending_backward = any(ctx.needs_input_grad)
         ctx.renderer, ctx.params, ctx.q, ctx.t = renderer, params, q, t
         ctx.want = (want_gauss, want_pose)
@@ -366,18 +356,15 @@ class _FusedTrackingLoss(torch.autograd.Function):
         ctx.eager = thres_fn is None and (ctx.needs_input_grad[2] or ctx.needs_input_grad[3])
         if ctx.eager:
             rgb, dep = gt_rgb.contiguous(), gt_depth.contiguous()
-            for attempt in range(2):
-                terms, radii, g7, seen = renderer.tracking_step_cached(p, q, t, rgb, dep, max_2D_radius=book, **cfg)
-                if not (poll and renderer.ensure_capacity()):      # (the bookkeeping only reads the radii: repeatable)
-                    break
-                if attempt == 1:
-                    raise RuntimeError("pair buffer overflow persisted after regrowing")
+            # (the bookkeeping only reads the radii: repeatable)
+            terms, radii, g7, seen = run_fitting(lambda: renderer.tracking_step_cached(p, q, t, rgb, dep, max_2D_radius=book, **cfg),
+                                                 [renderer], poll=poll)
             ctx.g7 = g7.clone()                     # the renderer's entry is overwritten by its next step
             terms = terms.clone()
             seen_box.append(seen)
             ctx.mark_non_differentiable(radii, terms)
             return terms[0].clone(), terms, radii
-        img, radii = _forward_checked(renderer, p, q, t, poll)
+        img, radii = run_fitting(lambda: renderer.forward(p, q, t), [renderer], poll=poll)
         cfg = dict(cfg)
         if thres_fn is not None:
             cfg["sil_thres"] = thres_fn(renderer, gt_rgb.contiguous(), gt_depth.contiguous())
@@ -419,7 +406,7 @@ class _FusedMappingLoss(torch.autograd.Function):
                  unnorm_rotations=unnorm_rot.detach().contiguous(), logit_opacities=logit_op.detach().contiguous(),
                  log_scales=log_scales.detach().contiguous())
         q, t = cam_q.detach().contiguous().reshape(4), cam_t.detach().contiguous().reshape(3)
-        _, radii = _forward_checked(renderer, p, q, t, _poll_due(renderer))
+        _, radii = run_fitting(lambda: renderer.forward(p, q, t), [renderer], poll=_poll_due(renderer))
         terms = renderer.mapping_loss(gt_rgb.contiguous(), gt_depth.contiguous(), w_im=w_im, w_depth=w_depth).clone()
         renderer.pending_backward = any(ctx.needs_input_grad)
         ctx.renderer, ctx.p, ctx.q, ctx.t, ctx.want_pose = renderer, p, q, t, want_pose
