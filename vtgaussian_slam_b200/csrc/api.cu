@@ -1,4 +1,6 @@
-// api.cu -- the extern "C" boundary declared in include/vtgs.h.
+// api.cu -- the library-wide part of the extern "C" boundary declared in include/vtgs.h: errors, build info, workspace
+// sizes, PDL and profiling switches, and the composed tracking step.  Every other entry point is defined in the .cu
+// file that owns its kernels.
 #include <stdarg.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -50,31 +52,6 @@ ProfScope::~ProfScope() {
 
 using namespace vtgs;
 
-#define VTGS_REQUIRE(cond, msg)                   \
-    do {                                          \
-        if (!(cond)) {                            \
-            set_error("invalid argument: %s", msg); \
-            return VTGS_E_INVALID;                \
-        }                                         \
-    } while (0)
-
-static int check_cam(const VtgsCamera* cam) {
-    VTGS_REQUIRE(cam != nullptr, "cam is NULL");
-    VTGS_REQUIRE(cam->image_width > 0 && cam->image_height > 0, "image size must be positive");
-    VTGS_REQUIRE(cam->tanfovx > 0.f && cam->tanfovy > 0.f, "tanfov must be positive");
-    VTGS_REQUIRE(cam->radius_sigma_mult > 0.f, "radius_sigma_mult must be positive");
-    return VTGS_OK;
-}
-
-static int check_buf(const VtgsBuffers* b, int64_t N) {
-    VTGS_REQUIRE(b != nullptr, "buffers is NULL");
-    VTGS_REQUIRE(b->tile_counts && b->tile_ranges && b->final_T && b->n_contrib && b->counters && b->region_cnt && b->region_masks && b->region_done, "workspace pointer is NULL");
-    if (N > 0) VTGS_REQUIRE(b->geom && b->tiles_touched && b->grad_geom, "per-Gaussian workspace pointer is NULL");
-    VTGS_REQUIRE(b->pair_capacity == 0 || (b->pair_keys && b->point_list && b->region_pairs), "pair workspace pointer is NULL");
-    VTGS_REQUIRE(b->pair_capacity < 0xffffffffull, "pair_capacity must fit 32 bits");
-    return VTGS_OK;
-}
-
 #pragma GCC visibility push(default)
 extern "C" {
 
@@ -111,92 +88,6 @@ int vtgs_workspace_query(int32_t W, int32_t H, int64_t N, uint64_t pair_capacity
     return VTGS_OK;
 }
 
-int vtgs_forward(const VtgsCamera* cam, int64_t N, const float* means3D, const float* scales,
-                 const float* rotations, const float* opacities, const float* colors,
-                 float* out_color, float* out_depth, int32_t* radii, VtgsBuffers* buf, void* stream) {
-    if (int e = check_cam(cam)) return e;
-    if (int e = check_buf(buf, N)) return e;
-    VTGS_REQUIRE(N >= 0, "num_gaussians < 0");
-    VTGS_REQUIRE(out_color && out_depth, "output pointer is NULL");
-    if (N > 0) VTGS_REQUIRE(means3D && scales && rotations && opacities && colors && radii, "input pointer is NULL");
-    FrontEnd fe{};
-    return launch_forward(cam, N, false, fe, means3D, scales, rotations, opacities, colors, out_color, out_depth, radii, buf,
-                          (cudaStream_t)stream);
-}
-
-int vtgs_backward(const VtgsCamera* cam, int64_t N, const float* means3D, const float* scales,
-                  const float* rotations, const float* opacities, const float* colors,
-                  const float* dL_dout_color, float* dL_dmeans2D, float* dL_dcolors, float* dL_dopacity,
-                  float* dL_dmeans3D, float* dL_dscales, float* dL_drotations, VtgsBuffers* buf, void* stream) {
-    if (int e = check_cam(cam)) return e;
-    if (int e = check_buf(buf, N)) return e;
-    VTGS_REQUIRE(N >= 0, "num_gaussians < 0");
-    if (N > 0)
-        VTGS_REQUIRE(means3D && scales && rotations && dL_dout_color && dL_dmeans2D && dL_dcolors && dL_dopacity &&
-                         dL_dmeans3D && dL_dscales && dL_drotations,
-                     "pointer is NULL");
-    return launch_backward(cam, N, means3D, scales, rotations, opacities, colors, dL_dout_color, dL_dmeans2D, dL_dcolors,
-                           dL_dopacity, dL_dmeans3D, dL_dscales, dL_drotations, buf, (cudaStream_t)stream);
-}
-
-int vtgs_mark_visible(const VtgsCamera* cam, int64_t N, const float* means3D, uint8_t* present, void* stream) {
-    if (int e = check_cam(cam)) return e;
-    if (N > 0) VTGS_REQUIRE(means3D && present, "pointer is NULL");
-    return launch_mark_visible(cam, N, means3D, present, (cudaStream_t)stream);
-}
-
-int vtgs_export_sorted_keys(const VtgsCamera* cam, int64_t N, const VtgsBuffers* buf, uint64_t* keys_out,
-                            uint64_t keys_capacity, void* stream) {
-    (void)N;
-    if (int e = check_cam(cam)) return e;
-    VTGS_REQUIRE(buf && keys_out, "pointer is NULL");
-    return launch_export_keys(cam, buf, keys_out, keys_capacity, (cudaStream_t)stream);
-}
-
-int vtgs_export_geometry(int64_t N, const VtgsBuffers* buf, float* means2D, float* depths, float* conic_opacity, void* stream) {
-    VTGS_REQUIRE(buf != nullptr, "buffers is NULL");
-    return launch_export_geometry(N, buf, means2D, depths, conic_opacity, (cudaStream_t)stream);
-}
-
-static int check_fused(const VtgsCamera* cam, const VtgsParams* p, const VtgsPose* pose, const VtgsBuffers* buf) {
-    if (int e = check_cam(cam)) return e;
-    VTGS_REQUIRE(p && pose, "params / pose is NULL");
-    if (int e = check_buf(buf, p->num_gaussians)) return e;
-    VTGS_REQUIRE(p->num_gaussians >= 0, "num_gaussians < 0");
-    if (p->num_gaussians > 0)
-        VTGS_REQUIRE(p->means3D && p->rgb_colors && p->unnorm_rotations && p->logit_opacities && p->log_scales, "param pointer is NULL");
-    VTGS_REQUIRE(pose->cam_unnorm_rot && pose->cam_trans, "pose pointer is NULL");
-    if (p->log_scales_dim != 1) {
-        set_error("fused path supports isotropic Gaussians only (log_scales [N,1]); use vtgs_forward/backward for anisotropic");
-        return VTGS_E_UNSUPPORTED;
-    }
-    return VTGS_OK;
-}
-
-int vtgs_fused_forward(const VtgsCamera* cam, const VtgsParams* p, const VtgsPose* pose, float* out_image6, int32_t* radii,
-                       VtgsBuffers* buf, void* stream) {
-    if (int e = check_fused(cam, p, pose, buf)) return e;
-    VTGS_REQUIRE(out_image6 != nullptr, "out_image6 is NULL");
-    if (p->num_gaussians > 0) VTGS_REQUIRE(radii != nullptr, "radii is NULL");
-    FrontEnd fe{};
-    fe.cam_unnorm_rot = pose->cam_unnorm_rot;
-    fe.cam_trans = pose->cam_trans;
-    fe.counters = buf->counters;
-    if (p->num_gaussians <= 0)          // nothing to preprocess: still publish the pose for the backward
-        if (int e = launch_pose_matrix(pose, buf->counters, (cudaStream_t)stream)) return e;
-    for (int k = 0; k < 4; ++k) fe.depth_row[k] = pose->depth_row[k];
-    fe.log_scales_dim = p->log_scales_dim;
-    return launch_forward(cam, p->num_gaussians, true, fe, p->means3D, p->log_scales, p->unnorm_rotations, p->logit_opacities,
-                          p->rgb_colors, out_image6, nullptr, radii, buf, (cudaStream_t)stream);
-}
-
-int vtgs_fused_backward(const VtgsCamera* cam, const VtgsParams* p, const VtgsPose* pose, const float* dL_dimage4,
-                        int32_t accumulate, VtgsParamGrads* grads, VtgsBuffers* buf, void* stream) {
-    if (int e = check_fused(cam, p, pose, buf)) return e;
-    VTGS_REQUIRE(dL_dimage4 && grads, "pointer is NULL");
-    return launch_fused_backward(cam, p, pose, dL_dimage4, accumulate, grads, buf, (cudaStream_t)stream);
-}
-
 int vtgs_fused_tracking_step(const VtgsCamera* cam, const VtgsParams* p, const VtgsPose* pose, const VtgsLossConfig* cfg,
                              const float* gt_rgb, const float* gt_depth, float* out_image6, int32_t* radii, float* dL_dimage4,
                              float* loss_terms, float* loss_scratch, VtgsParamGrads* grads, float* max_2D_radius, uint8_t* seen,
@@ -211,142 +102,6 @@ int vtgs_fused_tracking_step(const VtgsCamera* cam, const VtgsParams* p, const V
     if (max_2D_radius != nullptr)
         if (int e = vtgs_book_radii(p->num_gaussians, radii, max_2D_radius, seen, stream)) return e;
     return VTGS_OK;
-}
-
-uint64_t vtgs_pose_scratch_floats(int64_t N) { return (uint64_t)((N + 255) / 256 + 1) * 12; }
-
-uint64_t vtgs_loss_scratch_floats(int32_t W, int32_t H, int32_t mode) {
-    const uint64_t P = (uint64_t)W * H;
-    if (mode == 1) return 9 * P + ((uint64_t)((W + 15) / 16) * ((H + 15) / 16) * 3 + 1) * 4;
-    /* [tracking loss: 4 floats per 1024-pixel block + ticket + the radix-select state of the outlier median (320 words)
-     *  | silhouette ladder: 10 floats per block + ticket] */
-    return ((P + 1023) / 1024) * 14 + 320 + 16;
-}
-
-int vtgs_retie(float* means3D, int64_t n, const float* w2c_old, const float* cam_unnorm_rot, const float* cam_trans, void* stream) {
-    VTGS_REQUIRE(n >= 0, "n < 0");
-    VTGS_REQUIRE(w2c_old && cam_unnorm_rot && cam_trans && (n == 0 || means3D), "pointer is NULL");
-    return launch_retie(means3D, n, w2c_old, cam_unnorm_rot, cam_trans, (cudaStream_t)stream);
-}
-
-int vtgs_retie_dev(float* means3D, int64_t n, const float* old_unnorm_rot, const float* old_trans, const float* cam_unnorm_rot,
-                   const float* cam_trans, void* stream) {
-    VTGS_REQUIRE(n >= 0, "n < 0");
-    VTGS_REQUIRE(old_unnorm_rot && old_trans && cam_unnorm_rot && cam_trans && (n == 0 || means3D), "pointer is NULL");
-    return launch_retie_dev(means3D, n, old_unnorm_rot, old_trans, cam_unnorm_rot, cam_trans, (cudaStream_t)stream);
-}
-
-int vtgs_loss(const VtgsCamera* cam, const VtgsLossConfig* cfg, const float* image6, const float* gt_rgb,
-              const float* gt_depth, float* dL_dimage4, float* loss_terms, float* scratch, void* stream) {
-    if (int e = check_cam(cam)) return e;
-    VTGS_REQUIRE(cfg && image6 && gt_rgb && gt_depth && dL_dimage4 && loss_terms && scratch, "pointer is NULL");
-    return launch_loss(cam, cfg, image6, gt_rgb, gt_depth, dL_dimage4, loss_terms, scratch, (cudaStream_t)stream);
-}
-
-int vtgs_adam(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1,
-              float beta2, float eps, int32_t step, const int32_t* step_dev, void* stream) {
-    VTGS_REQUIRE(n >= 0, "n < 0");
-    if (n > 0) VTGS_REQUIRE(param && grad && exp_avg && exp_avg_sq, "pointer is NULL");
-    VTGS_REQUIRE(step_dev != nullptr || step >= 1, "step must be >= 1");
-    return launch_adam(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, step, step_dev, (cudaStream_t)stream);
-}
-
-int vtgs_sharded_adam(int32_t world, int32_t rank, const uint64_t* peer_bases, uint64_t multicast_base, int64_t param_off, int64_t grad_off, int64_t loss_off,
-                      float* exp_avg, float* exp_avg_sq, int64_t n, int32_t nseg, const int64_t* seg_end, const float* lr, float beta1,
-                      float beta2, float eps, const int32_t* step_dev, float* loss_out, void* stream) {
-    VTGS_REQUIRE(world >= 1 && world <= 8 && rank >= 0 && rank < world, "world must be 1..8 and rank inside it");
-    VTGS_REQUIRE(peer_bases && exp_avg && exp_avg_sq && seg_end && lr && step_dev && loss_out, "pointer is NULL");
-    VTGS_REQUIRE(n >= 0 && n % 4 == 0 && param_off % 4 == 0 && grad_off % 4 == 0, "flat vectors must be multiples of 4 floats");
-    VTGS_REQUIRE(nseg >= 1 && nseg <= 4, "1..4 segments");
-    for (int k = 0; k < world; ++k) VTGS_REQUIRE(peer_bases[k] != 0 && (peer_bases[k] & 15) == 0, "peer base must be a 16-byte aligned address");
-    VTGS_REQUIRE((multicast_base & 15) == 0, "multicast base must be 16-byte aligned");
-    return launch_sharded_adam(world, rank, peer_bases, multicast_base, param_off, grad_off, loss_off, exp_avg, exp_avg_sq, n, nseg, seg_end, lr,
-                               beta1, beta2, eps, step_dev, loss_out, (cudaStream_t)stream);
-}
-
-int vtgs_tracking_update(float* cam_unnorm_rot, float* cam_trans, const float* msg, float* adam_state, int32_t* step_dev,
-                         float* best, float lr_rot, float lr_trans, float eps, int32_t flags, void* stream) {
-    VTGS_REQUIRE(cam_unnorm_rot && cam_trans && msg && adam_state && step_dev && best, "pointer is NULL");
-    return launch_tracking_update(cam_unnorm_rot, cam_trans, msg, adam_state, step_dev, best, lr_rot, lr_trans, eps, flags, (cudaStream_t)stream);
-}
-
-int vtgs_median_hist(const VtgsCamera* cam, const float* depth_plane, const float* gt_depth, int32_t pass, uint32_t* state, void* stream) {
-    if (int e = check_cam(cam)) return e;
-    VTGS_REQUIRE(depth_plane && gt_depth && state, "pointer is NULL");
-    VTGS_REQUIRE(pass >= 0 && pass < 4, "pass must be 0..3");
-    return launch_median_hist(cam, depth_plane, gt_depth, pass, state, (cudaStream_t)stream);
-}
-
-int vtgs_median_pick(int64_t num_pixels_total, int32_t pass, uint32_t* state, void* stream) {
-    VTGS_REQUIRE(state != nullptr && num_pixels_total > 0, "bad argument");
-    VTGS_REQUIRE(pass >= 0 && pass < 4, "pass must be 0..3");
-    return launch_median_pick(num_pixels_total, pass, state, (cudaStream_t)stream);
-}
-
-int vtgs_sil_ladder(const VtgsCamera* cam, const float* image6, const float* gt_rgb, const float* gt_depth, float* sums10,
-                    float* scratch, void* stream) {
-    if (int e = check_cam(cam)) return e;
-    VTGS_REQUIRE(image6 && gt_rgb && gt_depth && sums10 && scratch, "pointer is NULL");
-    return launch_sil_ladder(cam, image6, gt_rgb, gt_depth, sums10, scratch, (cudaStream_t)stream);
-}
-
-int vtgs_sil_select(const float* sums10, float* sil_thres_dev, float* min_mse_dev, void* stream) {
-    VTGS_REQUIRE(sums10 && sil_thres_dev, "pointer is NULL");
-    return launch_sil_select(sums10, sil_thres_dev, min_mse_dev, (cudaStream_t)stream);
-}
-
-int vtgs_nonpresence_mask(const VtgsCamera* cam, const float* image6, const float* gt_depth, float sil_thres,
-                          const uint32_t* median_state, uint8_t* mask_out, uint32_t* count_dev, void* stream) {
-    if (int e = check_cam(cam)) return e;
-    VTGS_REQUIRE(image6 && gt_depth && median_state && mask_out, "pointer is NULL");
-    return launch_nonpresence_mask(cam, image6, gt_depth, sil_thres, median_state, mask_out, count_dev, (cudaStream_t)stream);
-}
-
-uint64_t vtgs_eval_scratch_floats(void) { return eval_scratch_floats(); }
-
-int vtgs_eval_metrics(const VtgsCamera* cam, const float* image6, const float* gt_rgb, const float* gt_depth, float sil_thres,
-                      int32_t use_presence, float* out8, float* scratch, void* stream) {
-    if (int e = check_cam(cam)) return e;
-    VTGS_REQUIRE(image6 && gt_rgb && gt_depth && out8 && scratch, "pointer is NULL");
-    return launch_eval_metrics(cam, image6, gt_rgb, gt_depth, sil_thres, use_presence, out8, scratch, (cudaStream_t)stream);
-}
-
-int vtgs_p2p_prepare(int32_t W, int32_t H, const float* intr4, const float* c2w12, const float* other_w2c12, const float* depth,
-                     const uint8_t* mask, float* pts, float* nrm, uint8_t* valid, void* stream) {
-    VTGS_REQUIRE(W > 0 && H > 0 && (int64_t)W * H < (int64_t)1 << 31, "bad image size");
-    VTGS_REQUIRE(intr4 && c2w12 && depth && pts && valid, "pointer is NULL");
-    return launch_p2p_prepare(W, H, intr4, c2w12, other_w2c12, depth, mask, pts, nrm, valid, (cudaStream_t)stream);
-}
-
-int vtgs_p2p_match(int64_t n_tgt, const float* tgt_pts, const float* tgt_nrm, const uint8_t* tgt_valid, int64_t n_src,
-                   const float* src_pts, const uint8_t* src_valid, float max_dist, int32_t* table, int64_t table_size,
-                   int32_t* next, float* out_dist, int32_t* out_idx, void* stream) {
-    VTGS_REQUIRE(n_tgt >= 0 && n_src >= 0 && n_tgt < (int64_t)1 << 31, "bad point count");
-    VTGS_REQUIRE(max_dist > 0.0f, "max_dist must be positive");
-    VTGS_REQUIRE(table && table_size > 0 && (table_size & (table_size - 1)) == 0 && table_size <= (int64_t)1 << 31, "table_size must be a power of two");
-    if (n_tgt > 0) VTGS_REQUIRE(tgt_pts && tgt_nrm && tgt_valid && next, "pointer is NULL");
-    if (n_src > 0) VTGS_REQUIRE(src_pts && src_valid && out_dist, "pointer is NULL");
-    return launch_p2p_match(n_tgt, tgt_pts, tgt_nrm, tgt_valid, n_src, src_pts, src_valid, max_dist, table, table_size, next, out_dist,
-                            out_idx, (cudaStream_t)stream);
-}
-
-int vtgs_frame_convert(int32_t src_w, int32_t src_h, int32_t dst_w, int32_t dst_h, const uint8_t* rgb_hwc, const uint16_t* depth_u16,
-                       double png_depth_scale, float* im_chw, float* depth_out, void* stream) {
-    VTGS_REQUIRE(src_w > 0 && src_h > 0 && dst_w > 0 && dst_h > 0, "bad image size");
-    VTGS_REQUIRE((rgb_hwc == nullptr) == (im_chw == nullptr) && (depth_u16 == nullptr) == (depth_out == nullptr), "input / output pointers must come in pairs");
-    VTGS_REQUIRE(depth_u16 == nullptr || png_depth_scale > 0.0, "png_depth_scale must be positive");
-    return launch_frame_convert(src_w, src_h, dst_w, dst_h, rgb_hwc, depth_u16, png_depth_scale, im_chw, depth_out, (cudaStream_t)stream);
-}
-
-int vtgs_book_radii(int64_t n, const int32_t* radii, float* max_2D_radius, uint8_t* seen, void* stream) {
-    VTGS_REQUIRE(n >= 0, "n < 0");
-    if (n > 0) VTGS_REQUIRE(radii && max_2D_radius && seen, "pointer is NULL");
-    return launch_book_radii(n, radii, max_2D_radius, seen, (cudaStream_t)stream);
-}
-
-int vtgs_ffma_probe(int64_t iters, float* sink, uint64_t* threads_out, void* stream) {
-    VTGS_REQUIRE(iters > 0 && sink != nullptr, "bad argument");
-    return launch_ffma_probe(iters, sink, threads_out, (cudaStream_t)stream);
 }
 
 int vtgs_profile_enable(int32_t on) {

@@ -105,9 +105,7 @@ static int launch_dpix_max(const CamConst& cam, const float* dL_dpix, int nch, u
     const size_t begin = (size_t)cam.row0 * 16 * cam.W, end = std::min(P, (size_t)cam.row1 * 16 * cam.W);
     if (end <= begin) return VTGS_OK;
     const int blocks = (int)std::min<size_t>((end - begin + 1023) / 1024, 148 * 8);
-    { VTGS_PROF("dpix_max_kernel", stream); launch_k(dpix_max_kernel, dim3(blocks), dim3(256), 0, stream, dL_dpix, P, begin, end, nch, out_bits); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
+    return launch_k("dpix_max_kernel", Launch::pdl, dpix_max_kernel, dim3(blocks), dim3(256), 0, stream, dL_dpix, P, begin, end, nch, out_bits);
 }
 
 // =============================== K6': backward blend =======================================
@@ -576,64 +574,32 @@ preprocess_backward_kernel(const __grid_constant__ CamConst cam, int64_t N,
     for (int k = 0; k < 4; ++k) dL_drot[4 * i + k] = dq[k];
 }
 
+template <bool FUSED, bool BG, bool LITE>
+static auto blend_backward_det(bool det) {
+    return det ? blend_backward_kernel<FUSED, BG, LITE, true> : blend_backward_kernel<FUSED, BG, LITE, false>;
+}
+
 // dynamic shared memory of blend_backward_kernel: bwd_smem_bytes(LITE)
 // per warp: splat table 1280 + cells 8192 + pixel table 768 (384 in the 3-row form) bytes
-template <bool FUSED, bool BG, bool LITE, bool DET>
-static int launch_blend_backward_det(int blocks, cudaStream_t stream, const CamConst& cam, const VtgsBuffers* buf, const GeomRecord* geom,
-                                     const float* dL_dpix, const uint32_t* order, const float* dl_bound) {
-    static std::atomic<uint64_t> done{0};
-    if (first_call_on_device(done)) {
-        VTGS_CUDA_CHECK(cudaFuncSetAttribute(blend_backward_kernel<FUSED, BG, LITE, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, bwd_smem_bytes(LITE)));
-        VTGS_CUDA_CHECK(cudaFuncSetAttribute(blend_backward_kernel<FUSED, BG, LITE, DET>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+static int launch_blend_backward(bool fused, bool bg, bool lite, int blocks, cudaStream_t stream, const CamConst& cam, const VtgsBuffers* buf,
+                                 const GeomRecord* geom, const float* dL_dpix, const uint32_t* order, const float* dl_bound) {
+    const bool det = (buf->flags & VTGS_BUF_DETERMINISTIC) != 0;
+    // (API mode never asks for the pose-only form: there is no blend_backward_kernel<false, BG, true, DET>)
+    const auto k6 = !fused ? (bg ? blend_backward_det<false, true, false>(det) : blend_backward_det<false, false, false>(det))
+                  : lite   ? (bg ? blend_backward_det<true, true, true>(det) : blend_backward_det<true, false, true>(det))
+                           : (bg ? blend_backward_det<true, true, false>(det) : blend_backward_det<true, false, false>(det));
+    static std::atomic<uint64_t> attr_done[16];          // per instantiation (index: its flags), the devices it is set up on
+    if (first_call_on_device(attr_done[fused * 8 + bg * 4 + lite * 2 + det])) {
+        VTGS_CUDA_CHECK(cudaFuncSetAttribute(k6, cudaFuncAttributeMaxDynamicSharedMemorySize, bwd_smem_bytes(lite)));
+        VTGS_CUDA_CHECK(cudaFuncSetAttribute(k6, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     }
     uint32_t* scalars = buf->tile_counts + cam.gx * cam.gy + 1;         // {max |colour|, max |dL/dpixel|} bit patterns
-    if (DET && dl_bound == nullptr) {          // no caller-supplied bound of |dL/dpixel|: measure it
-        if (int e = launch_dpix_max(cam, dL_dpix, FUSED ? 4 : 3, scalars + 1, stream)) return e;
+    if (det && dl_bound == nullptr) {          // no caller-supplied bound of |dL/dpixel|: measure it
+        if (int e = launch_dpix_max(cam, dL_dpix, fused ? 4 : 3, scalars + 1, stream)) return e;
     }
-    VTGS_PROF("blend_backward_kernel", stream);
-    launch_k(blend_backward_kernel<FUSED, BG, LITE, DET>, dim3(blocks), dim3(32 * BWD_WARPS), bwd_smem_bytes(LITE), stream, 
-        cam, buf->tile_ranges, reinterpret_cast<const uint2*>(buf->region_pairs), buf->region_cnt, buf->region_masks, buf->region_done,
-        geom, buf->final_T, dL_dpix, buf->grad_geom, order, scalars, DET ? dl_bound : nullptr);
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
-}
-
-template <bool FUSED, bool BG, bool LITE>
-static int launch_blend_backward(int blocks, cudaStream_t stream, const CamConst& cam, const VtgsBuffers* buf, const GeomRecord* geom,
-                                 const float* dL_dpix, const uint32_t* order, const float* dl_bound = nullptr) {
-    return (buf->flags & VTGS_BUF_DETERMINISTIC) ? launch_blend_backward_det<FUSED, BG, LITE, true>(blocks, stream, cam, buf, geom, dL_dpix, order, dl_bound)
-                                                 : launch_blend_backward_det<FUSED, BG, LITE, false>(blocks, stream, cam, buf, geom, dL_dpix, order, dl_bound);
-}
-
-int launch_backward(const VtgsCamera* camera, int64_t N,
-                    const float* means3D, const float* scales, const float* rotations,
-                    const float* opacities, const float* colors, const float* dL_dout_color,
-                    float* dL_dmeans2D, float* dL_dcolors, float* dL_dopacity,
-                    float* dL_dmeans3D, float* dL_dscales, float* dL_drotations,
-                    VtgsBuffers* buf, cudaStream_t stream) {
-    (void)opacities; (void)colors;
-    const CamConst cam = make_cam_const(*camera);
-    const GeomRecord* geom = reinterpret_cast<const GeomRecord*>(buf->geom);
-    const int band_tiles = (cam.row1 - cam.row0) * cam.gx;
-    if (N <= 0) return VTGS_OK;
-    if (band_tiles > 0) {
-        const bool has_bg = cam.bg[0] != 0.0f || cam.bg[1] != 0.0f || cam.bg[2] != 0.0f;
-        const int blocks = band_tiles * (8 / BWD_WARPS);
-        const uint32_t* order = nullptr;                  // (the forward orders tiles only for the fused path's tile bands)
-        if (int e = has_bg ? launch_blend_backward<false, true, false>(blocks, stream, cam, buf, geom, dL_dout_color, order)
-                           : launch_blend_backward<false, false, false>(blocks, stream, cam, buf, geom, dL_dout_color, order)) return e;
-    }
-    if (buf->flags & VTGS_BUF_DETERMINISTIC) {
-        VTGS_PROF("preprocess_backward_kernel", stream);
-        preprocess_backward_kernel<true><<<(unsigned)((N + 255) / 256), 256, 0, stream>>>(cam, N, means3D, scales, rotations, nullptr, geom, buf->grad_geom, dL_dmeans2D,
-                                                                                          dL_dcolors, dL_dopacity, dL_dmeans3D, dL_dscales, dL_drotations);
-    } else {
-        VTGS_PROF("preprocess_backward_kernel", stream);
-        preprocess_backward_kernel<false><<<(unsigned)((N + 255) / 256), 256, 0, stream>>>(cam, N, means3D, scales, rotations, nullptr, geom, buf->grad_geom, dL_dmeans2D,
-                                                                                           dL_dcolors, dL_dopacity, dL_dmeans3D, dL_dscales, dL_drotations);
-    }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
+    return launch_k("blend_backward_kernel", Launch::pdl, k6, dim3(blocks), dim3(32 * BWD_WARPS),
+                    bwd_smem_bytes(lite), stream, cam, buf->tile_ranges, reinterpret_cast<const uint2*>(buf->region_pairs), buf->region_cnt,
+                    buf->region_masks, buf->region_done, geom, buf->final_T, dL_dpix, buf->grad_geom, order, scalars, det ? dl_bound : nullptr);
 }
 
 // =============================== fused path ==================================================
@@ -651,9 +617,8 @@ __global__ void pose_matrix_kernel(const float* __restrict__ q_un, const float* 
 }
 
 int launch_pose_matrix(const VtgsPose* pose, VtgsCounters* counters, cudaStream_t stream) {
-    { VTGS_PROF("pose_matrix_kernel", stream); pose_matrix_kernel<<<1, 32, 0, stream>>>(pose->cam_unnorm_rot, pose->cam_trans, counters); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
+    return launch_k("pose_matrix_kernel", Launch::plain, pose_matrix_kernel, dim3(1), dim3(32), 0, stream, pose->cam_unnorm_rot, pose->cam_trans,
+                    counters);
 }
 
 constexpr int POSE_TERMS = 12;       // sum g (3) and sum g p^T (9)
@@ -890,9 +855,48 @@ fused_preprocess_backward_kernel(const __grid_constant__ CamConst cam, int64_t N
     if (tid == 0) *ticket = 0u;
 }
 
-int launch_fused_backward(const VtgsCamera* camera, const VtgsParams* params, const VtgsPose* pose,
-                          const float* dL_dimage4, int accumulate, VtgsParamGrads* grads,
-                          VtgsBuffers* buf, cudaStream_t stream) {
+}  // namespace vtgs
+
+// =============================== C entry points (include/vtgs.h) ===========================
+using namespace vtgs;
+
+uint64_t vtgs_pose_scratch_floats(int64_t N) { return (uint64_t)((N + 255) / 256 + 1) * 12; }
+
+// API-mode backward (K6' + K7').
+int vtgs_backward(const VtgsCamera* camera, int64_t N, const float* means3D, const float* scales,
+                  const float* rotations, const float* opacities, const float* colors,
+                  const float* dL_dout_color, float* dL_dmeans2D, float* dL_dcolors, float* dL_dopacity,
+                  float* dL_dmeans3D, float* dL_dscales, float* dL_drotations, VtgsBuffers* buf, void* stream_) {
+    if (int e = check_cam(camera)) return e;
+    if (int e = check_buf(buf, N)) return e;
+    VTGS_REQUIRE(N >= 0, "num_gaussians < 0");
+    if (N > 0)
+        VTGS_REQUIRE(means3D && scales && rotations && dL_dout_color && dL_dmeans2D && dL_dcolors && dL_dopacity &&
+                         dL_dmeans3D && dL_dscales && dL_drotations,
+                     "pointer is NULL");
+    (void)opacities; (void)colors;
+    const cudaStream_t stream = (cudaStream_t)stream_;
+    const CamConst cam = make_cam_const(*camera);
+    const GeomRecord* geom = reinterpret_cast<const GeomRecord*>(buf->geom);
+    const int band_tiles = (cam.row1 - cam.row0) * cam.gx;
+    if (N <= 0) return VTGS_OK;
+    const bool det = (buf->flags & VTGS_BUF_DETERMINISTIC) != 0;
+    if (band_tiles > 0) {
+        const bool has_bg = cam.bg[0] != 0.0f || cam.bg[1] != 0.0f || cam.bg[2] != 0.0f;
+        const int blocks = band_tiles * (8 / BWD_WARPS);
+        const uint32_t* order = nullptr;                  // (the forward orders tiles only for the fused path's tile bands)
+        if (int e = launch_blend_backward(false, has_bg, false, blocks, stream, cam, buf, geom, dL_dout_color, order, nullptr)) return e;
+    }
+    return launch_k("preprocess_backward_kernel", Launch::plain, det ? preprocess_backward_kernel<true> : preprocess_backward_kernel<false>,
+                    dim3((unsigned)((N + 255) / 256)), dim3(256), 0, stream, cam, N, means3D, scales, rotations, nullptr, geom, buf->grad_geom,
+                    dL_dmeans2D, dL_dcolors, dL_dopacity, dL_dmeans3D, dL_dscales, dL_drotations);
+}
+
+int vtgs_fused_backward(const VtgsCamera* camera, const VtgsParams* params, const VtgsPose* pose, const float* dL_dimage4,
+                        int32_t accumulate, VtgsParamGrads* grads, VtgsBuffers* buf, void* stream_) {
+    if (int e = check_fused(camera, params, pose, buf)) return e;
+    VTGS_REQUIRE(dL_dimage4 && grads, "pointer is NULL");
+    const cudaStream_t stream = (cudaStream_t)stream_;
     const CamConst cam = make_cam_const(*camera);
     const int64_t N = params->num_gaussians;
     const GeomRecord* geom = reinterpret_cast<const GeomRecord*>(buf->geom);
@@ -909,13 +913,7 @@ int launch_fused_backward(const VtgsCamera* camera, const VtgsParams* params, co
             const int bblocks = band_tiles * (8 / BWD_WARPS);
             // the fused forward left the band's tiles in longest-list-first order (tile bands only: same condition there)
             const uint32_t* order = band_tiles < cam.gx * cam.gy ? buf->tile_order : nullptr;
-            int e;
-            const float* dlb = grads->dL_abs_bound;
-            if (has_bg) e = lite ? launch_blend_backward<true, true, true>(bblocks, stream, cam, buf, geom, dL_dimage4, order, dlb)
-                                 : launch_blend_backward<true, true, false>(bblocks, stream, cam, buf, geom, dL_dimage4, order, dlb);
-            else e = lite ? launch_blend_backward<true, false, true>(bblocks, stream, cam, buf, geom, dL_dimage4, order, dlb)
-                          : launch_blend_backward<true, false, false>(bblocks, stream, cam, buf, geom, dL_dimage4, order, dlb);
-            if (e) return e;
+            if (int e = launch_blend_backward(true, has_bg, lite, bblocks, stream, cam, buf, geom, dL_dimage4, order, grads->dL_abs_bound)) return e;
         }
         unsigned int* ticket = reinterpret_cast<unsigned int*>(grads->pose_scratch ? grads->pose_scratch + (size_t)blocks * POSE_TERMS : nullptr);
         const uint32_t* band_touch = band_tiles < cam.gx * cam.gy ? buf->tiles_touched : nullptr;
@@ -926,23 +924,15 @@ int launch_fused_backward(const VtgsCamera* camera, const VtgsParams* params, co
         const uint32_t* n_cand = buf->tile_counts + cam.gx * cam.gy;
         const bool shape = grads->log_scales != nullptr || grads->unnorm_rotations != nullptr;
         const bool det = (buf->flags & VTGS_BUF_DETERMINISTIC) != 0;
-        {
-            VTGS_PROF("fused_preprocess_backward_kernel", stream);
-#define VTGS_K7_LAUNCH(SHAPE_, DET_)                                                                                                             \
-    launch_k(fused_preprocess_backward_kernel<SHAPE_, DET_>, dim3(blocks), dim3(256), 0, stream, cam, N, *params, buf->counters->pose_R, pose->depth_row[0],         \
-                                                                               pose->depth_row[1], pose->depth_row[2], geom, buf->grad_geom, *grads, \
-                                                                               accumulate, want_pose, buf->counters, ticket, band_touch, band_flags, \
-                                                                               band_cand, n_cand)
-            if (shape) { if (det) VTGS_K7_LAUNCH(true, true); else VTGS_K7_LAUNCH(true, false); }
-            else { if (det) VTGS_K7_LAUNCH(false, true); else VTGS_K7_LAUNCH(false, false); }
-#undef VTGS_K7_LAUNCH
-        }
-        VTGS_LAUNCH_CHECK();
-    } else if (want_pose && !accumulate) {
+        auto k7 = shape ? (det ? fused_preprocess_backward_kernel<true, true> : fused_preprocess_backward_kernel<true, false>)
+                        : (det ? fused_preprocess_backward_kernel<false, true> : fused_preprocess_backward_kernel<false, false>);
+        return launch_k("fused_preprocess_backward_kernel", Launch::pdl, k7, dim3(blocks), dim3(256), 0, stream, cam, N, *params,
+                        buf->counters->pose_R, pose->depth_row[0], pose->depth_row[1], pose->depth_row[2], geom, buf->grad_geom, *grads,
+                        accumulate, want_pose, buf->counters, ticket, band_touch, band_flags, band_cand, n_cand);
+    }
+    if (want_pose && !accumulate) {
         VTGS_CUDA_CHECK(cudaMemsetAsync(grads->cam_unnorm_rot, 0, 4 * sizeof(float), stream));
         VTGS_CUDA_CHECK(cudaMemsetAsync(grads->cam_trans, 0, 3 * sizeof(float), stream));
     }
     return VTGS_OK;
 }
-
-}  // namespace vtgs

@@ -86,19 +86,6 @@ eval_metrics_kernel(size_t P, const float* __restrict__ image6, const float* __r
     }
 }
 
-int launch_eval_metrics(const VtgsCamera* camera, const float* image6, const float* gt_rgb, const float* gt_depth, float sil_thres,
-                        int use_presence, float* out8, float* scratch, cudaStream_t stream) {
-    const size_t P = (size_t)camera->image_width * camera->image_height;
-    unsigned int* ticket = reinterpret_cast<unsigned int*>(scratch + (size_t)EVAL_BLOCKS * EVAL_TERMS);
-    VTGS_CUDA_CHECK(cudaMemsetAsync(ticket, 0, sizeof(unsigned int), stream));
-    { VTGS_PROF("eval_metrics_kernel", stream);
-      eval_metrics_kernel<<<EVAL_BLOCKS, 256, 0, stream>>>(P, image6, gt_rgb, gt_depth, sil_thres, use_presence, scratch, ticket, out8); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
-}
-
-uint64_t eval_scratch_floats() { return (uint64_t)EVAL_BLOCKS * EVAL_TERMS + 4; }
-
 // =============================== point-to-plane metric =======================================
 struct P2PFrame {
     int W, H;
@@ -215,39 +202,6 @@ p2p_query_kernel(int64_t n_src, const float* __restrict__ src, const uint8_t* __
     if (out_idx) out_idx[j] = best_i;
 }
 
-int launch_p2p_prepare(int W, int H, const float* intr4, const float* c2w12, const float* other_w2c12, const float* depth,
-                       const uint8_t* mask, float* pts, float* nrm, uint8_t* valid, cudaStream_t stream) {
-    P2PFrame f{};
-    f.W = W; f.H = H;
-    f.fx = intr4[0]; f.fy = intr4[1]; f.cx = intr4[2]; f.cy = intr4[3];
-    for (int k = 0; k < 12; ++k) { f.c2w[k] = c2w12[k]; f.other_w2c[k] = other_w2c12 ? other_w2c12[k] : 0.0f; }
-    f.frustum = other_w2c12 != nullptr;
-    const int P = W * H;
-    { VTGS_PROF("p2p_prepare_kernel", stream); p2p_prepare_kernel<<<(P + 255) / 256, 256, 0, stream>>>(f, depth, mask, pts, nrm, valid); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
-}
-
-int launch_p2p_match(int64_t n_tgt, const float* tgt_pts, const float* tgt_nrm, const uint8_t* tgt_valid, int64_t n_src,
-                     const float* src_pts, const uint8_t* src_valid, float max_dist, int32_t* table, int64_t table_size,
-                     int32_t* next, float* out_dist, int32_t* out_idx, cudaStream_t stream) {
-    VTGS_CUDA_CHECK(cudaMemsetAsync(table, 0xFF, sizeof(int32_t) * (size_t)table_size, stream));
-    const float inv_cell = 1.0f / max_dist;
-    const uint32_t mask = (uint32_t)(table_size - 1);
-    if (n_tgt > 0) {
-        VTGS_PROF("p2p_insert_kernel", stream);
-        p2p_insert_kernel<<<(unsigned)((n_tgt + 255) / 256), 256, 0, stream>>>(n_tgt, tgt_pts, tgt_valid, inv_cell, table, mask, next);
-    }
-    VTGS_LAUNCH_CHECK();
-    if (n_src > 0) {
-        VTGS_PROF("p2p_query_kernel", stream);
-        p2p_query_kernel<<<(unsigned)((n_src + 127) / 128), 128, 0, stream>>>(n_src, src_pts, src_valid, tgt_pts, tgt_nrm, inv_cell,
-                                                                            max_dist * max_dist, table, mask, next, out_dist, out_idx);
-    }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
-}
-
 // =============================== frame conversion on the device ==============================
 // What the reference's dataset does to a decoded frame on the CPU before every use (datasets/gradslam_datasets/
 // basedataset.py:215-272 + src/vtgaussian_slam.py:198-202): colour uint8 HWC -> float64 -> cv2.resize(INTER_LINEAR) ->
@@ -301,15 +255,6 @@ frame_convert_kernel(const __grid_constant__ ResizeGeom g, const uint8_t* __rest
     }
 }
 
-int launch_frame_convert(int sw, int sh, int dw, int dh, const uint8_t* rgb, const uint16_t* depth, double depth_scale, float* im,
-                         float* depth_out, cudaStream_t stream) {
-    ResizeGeom g{sw, sh, dw, dh, 1.0 / ((double)dw / (double)sw), 1.0 / ((double)dh / (double)sh)};      // cv::resize: 1 / inv_scale
-    { VTGS_PROF("frame_convert_kernel", stream);
-      frame_convert_kernel<<<(dw * dh + 255) / 256, 256, 0, stream>>>(g, rgb, depth, depth_scale, im, depth_out); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
-}
-
 // ---- radius bookkeeping of get_loss (reference src/vtgaussian_slam.py:681-683) ---------------------------------------
 __global__ void __launch_bounds__(256)
 book_radii_kernel(int64_t n, const int32_t* __restrict__ radii, float* __restrict__ max_radius, uint8_t* __restrict__ seen) {
@@ -321,11 +266,74 @@ book_radii_kernel(int64_t n, const int32_t* __restrict__ radii, float* __restric
     if (rf > m) max_radius[i] = rf;
 }
 
-int launch_book_radii(int64_t n, const int32_t* radii, float* max_radius, uint8_t* seen, cudaStream_t stream) {
-    if (n <= 0) return VTGS_OK;
-    { VTGS_PROF("book_radii_kernel", stream); book_radii_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(n, radii, max_radius, seen); }
-    VTGS_LAUNCH_CHECK();
+}  // namespace vtgs
+
+// =============================== C entry points (include/vtgs.h) ===========================
+using namespace vtgs;
+
+uint64_t vtgs_eval_scratch_floats(void) { return (uint64_t)EVAL_BLOCKS * EVAL_TERMS + 4; }
+
+int vtgs_eval_metrics(const VtgsCamera* cam, const float* image6, const float* gt_rgb, const float* gt_depth, float sil_thres,
+                      int32_t use_presence, float* out8, float* scratch, void* stream_) {
+    if (int e = check_cam(cam)) return e;
+    VTGS_REQUIRE(image6 && gt_rgb && gt_depth && out8 && scratch, "pointer is NULL");
+    const cudaStream_t stream = (cudaStream_t)stream_;
+    const size_t P = (size_t)cam->image_width * cam->image_height;
+    unsigned int* ticket = reinterpret_cast<unsigned int*>(scratch + (size_t)EVAL_BLOCKS * EVAL_TERMS);
+    VTGS_CUDA_CHECK(cudaMemsetAsync(ticket, 0, sizeof(unsigned int), stream));
+    return launch_k("eval_metrics_kernel", Launch::plain, eval_metrics_kernel, dim3(EVAL_BLOCKS), dim3(256), 0, stream, P, image6, gt_rgb, gt_depth,
+                    sil_thres, use_presence, scratch, ticket, out8);
+}
+
+int vtgs_p2p_prepare(int32_t W, int32_t H, const float* intr4, const float* c2w12, const float* other_w2c12, const float* depth,
+                     const uint8_t* mask, float* pts, float* nrm, uint8_t* valid, void* stream) {
+    VTGS_REQUIRE(W > 0 && H > 0 && (int64_t)W * H < (int64_t)1 << 31, "bad image size");
+    VTGS_REQUIRE(intr4 && c2w12 && depth && pts && valid, "pointer is NULL");
+    P2PFrame f{};
+    f.W = W; f.H = H;
+    f.fx = intr4[0]; f.fy = intr4[1]; f.cx = intr4[2]; f.cy = intr4[3];
+    for (int k = 0; k < 12; ++k) { f.c2w[k] = c2w12[k]; f.other_w2c[k] = other_w2c12 ? other_w2c12[k] : 0.0f; }
+    f.frustum = other_w2c12 != nullptr;
+    const int P = W * H;
+    return launch_k("p2p_prepare_kernel", Launch::plain, p2p_prepare_kernel, dim3((P + 255) / 256), dim3(256), 0, (cudaStream_t)stream, f, depth,
+                    mask, pts, nrm, valid);
+}
+
+int vtgs_p2p_match(int64_t n_tgt, const float* tgt_pts, const float* tgt_nrm, const uint8_t* tgt_valid, int64_t n_src,
+                   const float* src_pts, const uint8_t* src_valid, float max_dist, int32_t* table, int64_t table_size,
+                   int32_t* next, float* out_dist, int32_t* out_idx, void* stream_) {
+    VTGS_REQUIRE(n_tgt >= 0 && n_src >= 0 && n_tgt < (int64_t)1 << 31, "bad point count");
+    VTGS_REQUIRE(max_dist > 0.0f, "max_dist must be positive");
+    VTGS_REQUIRE(table && table_size > 0 && (table_size & (table_size - 1)) == 0 && table_size <= (int64_t)1 << 31, "table_size must be a power of two");
+    if (n_tgt > 0) VTGS_REQUIRE(tgt_pts && tgt_nrm && tgt_valid && next, "pointer is NULL");
+    if (n_src > 0) VTGS_REQUIRE(src_pts && src_valid && out_dist, "pointer is NULL");
+    const cudaStream_t stream = (cudaStream_t)stream_;
+    VTGS_CUDA_CHECK(cudaMemsetAsync(table, 0xFF, sizeof(int32_t) * (size_t)table_size, stream));
+    const float inv_cell = 1.0f / max_dist;
+    const uint32_t mask = (uint32_t)(table_size - 1);
+    if (n_tgt > 0)
+        if (int e = launch_k("p2p_insert_kernel", Launch::plain, p2p_insert_kernel, dim3((unsigned)((n_tgt + 255) / 256)), dim3(256), 0, stream,
+                             n_tgt, tgt_pts, tgt_valid, inv_cell, table, mask, next)) return e;
+    if (n_src > 0)
+        return launch_k("p2p_query_kernel", Launch::plain, p2p_query_kernel, dim3((unsigned)((n_src + 127) / 128)), dim3(128), 0, stream, n_src,
+                        src_pts, src_valid, tgt_pts, tgt_nrm, inv_cell, max_dist * max_dist, table, mask, next, out_dist, out_idx);
     return VTGS_OK;
 }
 
-}  // namespace vtgs
+int vtgs_frame_convert(int32_t src_w, int32_t src_h, int32_t dst_w, int32_t dst_h, const uint8_t* rgb_hwc, const uint16_t* depth_u16,
+                       double png_depth_scale, float* im_chw, float* depth_out, void* stream) {
+    VTGS_REQUIRE(src_w > 0 && src_h > 0 && dst_w > 0 && dst_h > 0, "bad image size");
+    VTGS_REQUIRE((rgb_hwc == nullptr) == (im_chw == nullptr) && (depth_u16 == nullptr) == (depth_out == nullptr), "input / output pointers must come in pairs");
+    VTGS_REQUIRE(depth_u16 == nullptr || png_depth_scale > 0.0, "png_depth_scale must be positive");
+    ResizeGeom g{src_w, src_h, dst_w, dst_h, 1.0 / ((double)dst_w / (double)src_w), 1.0 / ((double)dst_h / (double)src_h)};   // cv::resize: 1 / inv_scale
+    return launch_k("frame_convert_kernel", Launch::plain, frame_convert_kernel, dim3((dst_w * dst_h + 255) / 256), dim3(256), 0, (cudaStream_t)stream,
+                    g, rgb_hwc, depth_u16, png_depth_scale, im_chw, depth_out);
+}
+
+int vtgs_book_radii(int64_t n, const int32_t* radii, float* max_2D_radius, uint8_t* seen, void* stream) {
+    VTGS_REQUIRE(n >= 0, "n < 0");
+    if (n > 0) VTGS_REQUIRE(radii && max_2D_radius && seen, "pointer is NULL");
+    if (n <= 0) return VTGS_OK;
+    return launch_k("book_radii_kernel", Launch::plain, book_radii_kernel, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, (cudaStream_t)stream, n,
+                    radii, max_2D_radius, seen);
+}

@@ -26,13 +26,20 @@ void set_error(const char* fmt, ...);
             return VTGS_E_CUDA;                                                      \
         }                                                                            \
     } while (0)
-#define VTGS_LAUNCH_CHECK() VTGS_CUDA_CHECK(cudaGetLastError())
+
+// RAII event bracket around one kernel launch (only when vtgs_profile_enable(1) was called).
+struct ProfScope {
+    ProfScope(const char* name, cudaStream_t stream);
+    ~ProfScope();
+    int slot;
+    cudaStream_t stream;
+};
 
 // ---- programmatic dependent launch (PDL) ------------------------------------------------------------------------
 // The kernels of an iteration form a chain in one stream / CUDA graph, and several of them are short.  Launched with
 // the programmatic-stream-serialization attribute, a kernel's launch and block scheduling overlap the drain of its
 // predecessor; its blocks then sit in pdl_wait() until the predecessor grid has completed and its memory is visible.
-// Every kernel launched through launch_k() therefore starts with pdl_wait() BEFORE it touches global memory: the
+// Every kernel launched with Launch::pdl therefore starts with pdl_wait() BEFORE it touches global memory: the
 // ordering is that of a plain stream.  (Without the attribute the instruction is a no-op.)  Measured at C2 on one
 // B200 (graph replay): +0.5 %; with an early `griddepcontrol.launch_dependents` in every kernel (dependent blocks
 // resident behind the predecessor's last wave) -0.4 %, so the trigger stays implicit.  VTGS_PDL=0 turns the attribute off.
@@ -41,19 +48,34 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 
 bool pdl_enabled();        // api.cu: environment VTGS_PDL (default on)
 
+// Launch::plain is for kernels without pdl_wait(): a launch with no attributes, the same as <<<>>>.
+enum class Launch { plain, pdl };
+
+// Every kernel launch of the library: `kernel` runs under the profile name `name` (vtgs_profile_summary; bench.py's
+// per_kernel_us keys on these names).  Returns VTGS_OK, or VTGS_E_CUDA when the launch failed.
 template <typename... KArgs, typename... Args>
-inline void launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args&&... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
-    (void)cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);      // errors surface in VTGS_LAUNCH_CHECK()
+inline int launch_k(const char* name, Launch mode, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
+                    cudaStream_t stream, Args&&... args) {
+    {
+        ProfScope prof(name, stream);
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = grid;
+        cfg.blockDim = block;
+        cfg.dynamicSmemBytes = smem;
+        cfg.stream = stream;
+        cudaLaunchAttribute attr[1];
+        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        attr[0].val.programmaticStreamSerializationAllowed = 1;
+        cfg.attrs = attr;
+        cfg.numAttrs = (mode == Launch::pdl && pdl_enabled()) ? 1 : 0;
+        (void)cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);      // its error is also cudaGetLastError()'s
+    }
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) {
+        set_error("launch of %s failed: %s", name, cudaGetErrorString(e));
+        return VTGS_E_CUDA;
+    }
+    return VTGS_OK;
 }
 
 // One-time kernel attribute setup PER DEVICE (a process may drive several GPUs): true for the first caller on the

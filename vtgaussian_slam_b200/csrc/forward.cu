@@ -28,6 +28,15 @@
 
 namespace vtgs {
 
+// Front end of the fused path (transform_to_frame + activations); unused in API mode.
+struct FrontEnd {
+    const float* cam_unnorm_rot;   // device [4]: the frame's un-normalised pose quaternion
+    const float* cam_trans;        // device [3]
+    VtgsCounters* counters;        // device: receives pose_R / pose_t / pose_q / pose_qnorm for the backward
+    float depth_row[4];
+    int log_scales_dim;
+};
+
 // Warp-collective walk over every lane's tile rect [minx,maxx) x [miny,maxy).  Each step all lanes
 // present their current tile (or none); lanes presenting the same tile are grouped with
 // match.any so that the callback can issue ONE atomic per distinct tile:
@@ -1129,11 +1138,12 @@ __global__ void fill_outside_band_kernel(const __grid_constant__ CamConst cam, i
 }
 
 // =============================== host orchestration ======================================
-int launch_forward(const VtgsCamera* camera, int64_t N, bool fused, const FrontEnd& fe,
-                   const float* means3D, const float* scales, const float* rotations,
-                   const float* opacities, const float* colors,
-                   float* out_color, float* out_depth, int32_t* radii, VtgsBuffers* buf,
-                   cudaStream_t stream) {
+// The forward of both paths: API mode (vtgs_forward) and the fused path (vtgs_fused_forward: `fused`, front end `fe`).
+static int launch_forward(const VtgsCamera* camera, int64_t N, bool fused, const FrontEnd& fe,
+                          const float* means3D, const float* scales, const float* rotations,
+                          const float* opacities, const float* colors,
+                          float* out_color, float* out_depth, int32_t* radii, VtgsBuffers* buf,
+                          cudaStream_t stream) {
     const CamConst cam = make_cam_const(*camera);
     const int num_tiles = cam.gx * cam.gy;
     if (cam.gx > 0xffff || cam.gy > 0xffff) { set_error("image too large for packed tile rects"); return VTGS_E_INVALID; }
@@ -1152,20 +1162,13 @@ int launch_forward(const VtgsCamera* camera, int64_t N, bool fused, const FrontE
     const int persistent = 148 * 3;
     if (N > 0) {
         const bool narrow_band = (cam.row1 - cam.row0) * 5 < cam.gy * 2;
-        if (use_cand) {
-            { VTGS_PROF("band_flags_kernel", stream); launch_k(band_flags_kernel, dim3((blocks + 3) / 4), dim3(256), 0, stream, cam, N, fe, means3D, scales, radii, buf->tiles_touched, buf->band_flags, buf->band_cand, n_cand); }
-            VTGS_LAUNCH_CHECK();
-        }
+        if (use_cand)
+            if (int e = launch_k("band_flags_kernel", Launch::pdl, band_flags_kernel, dim3((blocks + 3) / 4), dim3(256), 0, stream,
+                                 cam, N, fe, means3D, scales, radii, buf->tiles_touched, buf->band_flags, buf->band_cand, n_cand)) return e;
         const int k1_grid = use_cand ? std::min(blocks, persistent) : k1_blocks;
-        if (fused && narrow_band)
-            { VTGS_PROF("preprocess_kernel", stream); launch_k(preprocess_kernel<true, true>, dim3(k1_grid), dim3(256), 0, stream, cam, N, fe, means3D, scales, rotations, opacities, colors,
-                                                                 geom, radii, buf->tiles_touched, buf->tile_counts, cand, n_cand, cmax_bits); }
-        else if (fused)
-            { VTGS_PROF("preprocess_kernel", stream); launch_k(preprocess_kernel<true>, dim3(k1_grid), dim3(256), 0, stream, cam, N, fe, means3D, scales, rotations, opacities, colors,
-                                                                 geom, radii, buf->tiles_touched, buf->tile_counts, cand, n_cand, cmax_bits); }
-        else { VTGS_PROF("preprocess_kernel", stream); launch_k(preprocess_kernel<false>, dim3(k1_grid), dim3(256), 0, stream, cam, N, fe, means3D, scales, rotations, opacities, colors,
-                                                                  geom, radii, buf->tiles_touched, buf->tile_counts, nullptr, nullptr, cmax_bits); }
-        VTGS_LAUNCH_CHECK();
+        auto k1 = fused ? (narrow_band ? preprocess_kernel<true, true> : preprocess_kernel<true, false>) : preprocess_kernel<false, false>;
+        if (int e = launch_k("preprocess_kernel", Launch::pdl, k1, dim3(k1_grid), dim3(256), 0, stream, cam, N, fe, means3D, scales, rotations,
+                             opacities, colors, geom, radii, buf->tiles_touched, buf->tile_counts, cand, fused ? n_cand : nullptr, cmax_bits)) return e;
     }
     // only the band's tiles hold counts (tile-band sharding: K1' clips every rect to the band); the fused solvers never
     // look at another tile's range, so they scan the band alone -- API mode keeps (0,0) ranges for the other tiles
@@ -1174,22 +1177,20 @@ int launch_forward(const VtgsCamera* camera, int64_t N, bool fused, const FrontE
     // the tile order is relative to the scanned range: usable when that is exactly what the sort / blend kernels cover
     // (worth its ~4 us in the scan only when a launch is about one wave of blocks: tile bands)
     uint32_t* order = (fused && band_active) ? buf->tile_order : nullptr;
-    { VTGS_PROF("tile_scan_kernel", stream); launch_k(tile_scan_kernel, dim3(1), dim3(1024), 0, stream, buf->tile_counts + scan0, buf->tile_ranges + 2 * (size_t)scan0, scan_n, buf->pair_capacity, buf->counters, order); }
-    VTGS_LAUNCH_CHECK();
+    if (int e = launch_k("tile_scan_kernel", Launch::pdl, tile_scan_kernel, dim3(1), dim3(1024), 0, stream, buf->tile_counts + scan0,
+                         buf->tile_ranges + 2 * (size_t)scan0, scan_n, buf->pair_capacity, buf->counters, order)) return e;
     if (N > 0 && band_tiles > 0) {
-        { VTGS_PROF("scatter_kernel", stream); const int sb = use_cand ? std::min(blocks, 148 * 8) : blocks;
-          if (wide) launch_k(scatter_kernel<true>, dim3(sb), dim3(256), 0, stream, N, cam.gx, geom, buf->tiles_touched, buf->tile_ranges, buf->tile_counts, buf->pair_keys, cand, n_cand);
-          else launch_k(scatter_kernel<false>, dim3(sb), dim3(256), 0, stream, N, cam.gx, geom, buf->tiles_touched, buf->tile_ranges, buf->tile_counts, buf->pair_keys, cand, n_cand); }
-        VTGS_LAUNCH_CHECK();
+        const int sb = use_cand ? std::min(blocks, 148 * 8) : blocks;
+        if (int e = launch_k("scatter_kernel", Launch::pdl, wide ? scatter_kernel<true> : scatter_kernel<false>, dim3(sb), dim3(256), 0, stream,
+                             N, cam.gx, geom, buf->tiles_touched, buf->tile_ranges, buf->tile_counts, buf->pair_keys, cand, n_cand)) return e;
         static std::atomic<uint64_t> sort_attr{0};
         if (first_call_on_device(sort_attr)) {
             VTGS_CUDA_CHECK(cudaFuncSetAttribute(tile_sort_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SORT_SMEM_ELEMS * 8));
             VTGS_CUDA_CHECK(cudaFuncSetAttribute(tile_sort_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SORT_SMEM_ELEMS * 8));
         }
-        { VTGS_PROF("tile_sort_kernel", stream);
-          if (wide) launch_k(tile_sort_kernel<true>, dim3(band_tiles), dim3(256), SORT_SMEM_ELEMS * 8, stream, cam, buf->tile_ranges, cam.row0 * cam.gx, buf->pair_keys, buf->point_list, geom, reinterpret_cast<uint2*>(buf->region_pairs), buf->region_cnt, order);
-          else launch_k(tile_sort_kernel<false>, dim3(band_tiles), dim3(256), SORT_SMEM_ELEMS * 8, stream, cam, buf->tile_ranges, cam.row0 * cam.gx, buf->pair_keys, buf->point_list, geom, reinterpret_cast<uint2*>(buf->region_pairs), buf->region_cnt, order); }
-        VTGS_LAUNCH_CHECK();
+        if (int e = launch_k("tile_sort_kernel", Launch::pdl, wide ? tile_sort_kernel<true> : tile_sort_kernel<false>, dim3(band_tiles), dim3(256),
+                             SORT_SMEM_ELEMS * 8, stream, cam, buf->tile_ranges, cam.row0 * cam.gx, buf->pair_keys, buf->point_list, geom,
+                             reinterpret_cast<uint2*>(buf->region_pairs), buf->region_cnt, order)) return e;
     }
     if (N <= 0) VTGS_CUDA_CHECK(cudaMemsetAsync(buf->region_cnt, 0, sizeof(uint32_t) * 8 * num_tiles, stream));
     if (band_tiles > 0) {
@@ -1198,15 +1199,15 @@ int launch_forward(const VtgsCamera* camera, int64_t N, bool fused, const FrontE
             VTGS_CUDA_CHECK(cudaFuncSetAttribute(blend_forward_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
             VTGS_CUDA_CHECK(cudaFuncSetAttribute(blend_forward_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         }
-        if (fused)
-            { VTGS_PROF("blend_forward_kernel", stream); launch_k(blend_forward_kernel<true>, dim3(band_tiles * (8 / FWD_WARPS)), dim3(32 * FWD_WARPS), 0, stream, cam, buf->tile_ranges, reinterpret_cast<const uint2*>(buf->region_pairs), buf->region_cnt, buf->region_masks, buf->region_done, geom, out_color, out_depth, buf->final_T, buf->n_contrib, order); }
-        else { VTGS_PROF("blend_forward_kernel", stream); launch_k(blend_forward_kernel<false>, dim3(band_tiles * (8 / FWD_WARPS)), dim3(32 * FWD_WARPS), 0, stream, cam, buf->tile_ranges, reinterpret_cast<const uint2*>(buf->region_pairs), buf->region_cnt, buf->region_masks, buf->region_done, geom, out_color, out_depth, buf->final_T, buf->n_contrib, order); }
-        VTGS_LAUNCH_CHECK();
+        if (int e = launch_k("blend_forward_kernel", Launch::pdl, fused ? blend_forward_kernel<true> : blend_forward_kernel<false>,
+                             dim3(band_tiles * (8 / FWD_WARPS)), dim3(32 * FWD_WARPS), 0, stream, cam, buf->tile_ranges,
+                             reinterpret_cast<const uint2*>(buf->region_pairs), buf->region_cnt, buf->region_masks, buf->region_done, geom,
+                             out_color, out_depth, buf->final_T, buf->n_contrib, order)) return e;
     }
     if (band_tiles < num_tiles && !fused) {       // API mode returns complete planes; the fused solvers only ever read their band
         const size_t P = (size_t)cam.W * cam.H;
-        { VTGS_PROF("fill_outside_band_kernel", stream); launch_k(fill_outside_band_kernel, dim3((unsigned)((P + 255) / 256)), dim3(256), 0, stream, cam, fused ? 6 : 3, out_color, out_depth, buf->final_T, buf->n_contrib); }
-        VTGS_LAUNCH_CHECK();
+        if (int e = launch_k("fill_outside_band_kernel", Launch::pdl, fill_outside_band_kernel, dim3((unsigned)((P + 255) / 256)), dim3(256), 0,
+                             stream, cam, fused ? 6 : 3, out_color, out_depth, buf->final_T, buf->n_contrib)) return e;
     }
     return VTGS_OK;
 }
@@ -1221,14 +1222,6 @@ __global__ void export_keys_kernel(const uint32_t* __restrict__ ranges, int num_
         if (i < cap) out[i] = ((uint64_t)tile << 32) | (pair_keys[i] >> 32);
 }
 
-int launch_export_keys(const VtgsCamera* camera, const VtgsBuffers* buf, uint64_t* out, uint64_t cap, cudaStream_t stream) {
-    const CamConst cam = make_cam_const(*camera);
-    const int num_tiles = cam.gx * cam.gy;
-    { VTGS_PROF("export_keys_kernel", stream); export_keys_kernel<<<num_tiles, 128, 0, stream>>>(buf->tile_ranges, num_tiles, buf->pair_keys, out, cap); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
-}
-
 __global__ void export_geom_kernel(int64_t N, const GeomRecord* __restrict__ geom, float* means2D, float* depths, float* conic_opacity) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= N) return;
@@ -1238,25 +1231,70 @@ __global__ void export_geom_kernel(int64_t N, const GeomRecord* __restrict__ geo
     if (conic_opacity) { conic_opacity[4 * i] = r.q1.x; conic_opacity[4 * i + 1] = r.q1.y; conic_opacity[4 * i + 2] = r.q1.z; conic_opacity[4 * i + 3] = r.q1.w; }
 }
 
-int launch_export_geometry(int64_t N, const VtgsBuffers* buf, float* means2D, float* depths, float* conic_opacity, cudaStream_t stream) {
-    if (N <= 0) return VTGS_OK;
-    { VTGS_PROF("export_geom_kernel", stream); export_geom_kernel<<<(unsigned)((N + 255) / 256), 256, 0, stream>>>(N, reinterpret_cast<const GeomRecord*>(buf->geom), means2D, depths, conic_opacity); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
-}
-
 __global__ void mark_visible_kernel(const __grid_constant__ CamConst cam, int64_t N, const float* __restrict__ means3D, uint8_t* __restrict__ present) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= N) return;
     present[i] = xform_row(cam.view, 2, means3D[3 * i], means3D[3 * i + 1], means3D[3 * i + 2]) > VTGS_NEAR_CULL ? 1 : 0;
 }
 
-int launch_mark_visible(const VtgsCamera* camera, int64_t N, const float* means3D, uint8_t* present, cudaStream_t stream) {
-    if (N <= 0) return VTGS_OK;
-    const CamConst cam = make_cam_const(*camera);
-    { VTGS_PROF("mark_visible_kernel", stream); mark_visible_kernel<<<(unsigned)((N + 255) / 256), 256, 0, stream>>>(cam, N, means3D, present); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
+}  // namespace vtgs
+
+// =============================== C entry points (include/vtgs.h) ===========================
+using namespace vtgs;
+
+int vtgs_forward(const VtgsCamera* cam, int64_t N, const float* means3D, const float* scales,
+                 const float* rotations, const float* opacities, const float* colors,
+                 float* out_color, float* out_depth, int32_t* radii, VtgsBuffers* buf, void* stream) {
+    if (int e = check_cam(cam)) return e;
+    if (int e = check_buf(buf, N)) return e;
+    VTGS_REQUIRE(N >= 0, "num_gaussians < 0");
+    VTGS_REQUIRE(out_color && out_depth, "output pointer is NULL");
+    if (N > 0) VTGS_REQUIRE(means3D && scales && rotations && opacities && colors && radii, "input pointer is NULL");
+    FrontEnd fe{};
+    return launch_forward(cam, N, false, fe, means3D, scales, rotations, opacities, colors, out_color, out_depth, radii, buf,
+                          (cudaStream_t)stream);
 }
 
-}  // namespace vtgs
+int vtgs_fused_forward(const VtgsCamera* cam, const VtgsParams* p, const VtgsPose* pose, float* out_image6, int32_t* radii,
+                       VtgsBuffers* buf, void* stream) {
+    if (int e = check_fused(cam, p, pose, buf)) return e;
+    VTGS_REQUIRE(out_image6 != nullptr, "out_image6 is NULL");
+    if (p->num_gaussians > 0) VTGS_REQUIRE(radii != nullptr, "radii is NULL");
+    FrontEnd fe{};
+    fe.cam_unnorm_rot = pose->cam_unnorm_rot;
+    fe.cam_trans = pose->cam_trans;
+    fe.counters = buf->counters;
+    if (p->num_gaussians <= 0)          // nothing to preprocess: still publish the pose for the backward
+        if (int e = launch_pose_matrix(pose, buf->counters, (cudaStream_t)stream)) return e;
+    for (int k = 0; k < 4; ++k) fe.depth_row[k] = pose->depth_row[k];
+    fe.log_scales_dim = p->log_scales_dim;
+    return launch_forward(cam, p->num_gaussians, true, fe, p->means3D, p->log_scales, p->unnorm_rotations, p->logit_opacities,
+                          p->rgb_colors, out_image6, nullptr, radii, buf, (cudaStream_t)stream);
+}
+
+int vtgs_export_sorted_keys(const VtgsCamera* camera, int64_t N, const VtgsBuffers* buf, uint64_t* keys_out,
+                            uint64_t keys_capacity, void* stream) {
+    (void)N;
+    if (int e = check_cam(camera)) return e;
+    VTGS_REQUIRE(buf && keys_out, "pointer is NULL");
+    const CamConst cam = make_cam_const(*camera);
+    const int num_tiles = cam.gx * cam.gy;
+    return launch_k("export_keys_kernel", Launch::plain, export_keys_kernel, dim3(num_tiles), dim3(128), 0, (cudaStream_t)stream,
+                    buf->tile_ranges, num_tiles, buf->pair_keys, keys_out, keys_capacity);
+}
+
+int vtgs_export_geometry(int64_t N, const VtgsBuffers* buf, float* means2D, float* depths, float* conic_opacity, void* stream) {
+    VTGS_REQUIRE(buf != nullptr, "buffers is NULL");
+    if (N <= 0) return VTGS_OK;
+    return launch_k("export_geom_kernel", Launch::plain, export_geom_kernel, dim3((unsigned)((N + 255) / 256)), dim3(256), 0,
+                    (cudaStream_t)stream, N, reinterpret_cast<const GeomRecord*>(buf->geom), means2D, depths, conic_opacity);
+}
+
+int vtgs_mark_visible(const VtgsCamera* camera, int64_t N, const float* means3D, uint8_t* present, void* stream) {
+    if (int e = check_cam(camera)) return e;
+    if (N > 0) VTGS_REQUIRE(means3D && present, "pointer is NULL");
+    if (N <= 0) return VTGS_OK;
+    const CamConst cam = make_cam_const(*camera);
+    return launch_k("mark_visible_kernel", Launch::plain, mark_visible_kernel, dim3((unsigned)((N + 255) / 256)), dim3(256), 0,
+                    (cudaStream_t)stream, cam, N, means3D, present);
+}

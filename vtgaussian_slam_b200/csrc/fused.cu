@@ -79,22 +79,18 @@ static inline void band_pixel_range(const CamConst& cam, size_t& b, size_t& e) {
     if (b > e) b = e;
 }
 
-int launch_median_hist(const VtgsCamera* camera, const float* depth_plane, const float* gt_depth, int pass, uint32_t* state,
-                       cudaStream_t stream) {
+static int launch_median_hist(const VtgsCamera* camera, const float* depth_plane, const float* gt_depth, int pass, uint32_t* state,
+                              cudaStream_t stream) {
     const CamConst cam = make_cam_const(*camera);
     size_t b, e;
     band_pixel_range(cam, b, e);
     if (e <= b) return VTGS_OK;
     const int mb = (int)std::min<size_t>((e - b + 1023) / 1024, 148 * 4);
-    { VTGS_PROF("median_hist_kernel", stream); launch_k(median_hist_kernel, dim3(mb), dim3(256), 0, stream, depth_plane, gt_depth, b, e, pass, state); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
+    return launch_k("median_hist_kernel", Launch::pdl, median_hist_kernel, dim3(mb), dim3(256), 0, stream, depth_plane, gt_depth, b, e, pass, state);
 }
 
-int launch_median_pick(int64_t P_total, int pass, uint32_t* state, cudaStream_t stream) {
-    { VTGS_PROF("median_pick_kernel", stream); launch_k(median_pick_kernel, dim3(1), dim3(256), 0, stream, (unsigned long long)P_total, pass, state); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
+static int launch_median_pick(int64_t P_total, int pass, uint32_t* state, cudaStream_t stream) {
+    return launch_k("median_pick_kernel", Launch::pdl, median_pick_kernel, dim3(1), dim3(256), 0, stream, (unsigned long long)P_total, pass, state);
 }
 
 // ---- Replica iteration-0 silhouette-threshold search (reference src/vtgaussian_slam.py:472-510) --------------------
@@ -178,31 +174,6 @@ __global__ void sil_select_kernel(const float* __restrict__ sums10, float* __res
     if (mse_out) *mse_out = have ? best_mse : __uint_as_float(0x7fc00000u);
 }
 
-int launch_sil_ladder(const VtgsCamera* camera, const float* image6, const float* gt_rgb, const float* gt_depth, float* sums10,
-                      float* scratch, cudaStream_t stream) {
-    const CamConst cam = make_cam_const(*camera);
-    size_t b, e;
-    band_pixel_range(cam, b, e);
-    const int nblocks = (int)((e - b + 1023) / 1024);
-    if (nblocks <= 0) { VTGS_CUDA_CHECK(cudaMemsetAsync(sums10, 0, 10 * sizeof(float), stream)); return VTGS_OK; }
-    // the loss scratch (vtgs_loss_scratch_floats, mode 0) = [tracking-loss region: 4 floats per 1024-pixel block of the
-    // whole frame, its ticket, the median state | ladder region: 10 floats per block, its ticket]: the two never overlap,
-    // so the tracking loss's self-resetting ticket stays intact
-    const size_t nb_full = ((size_t)cam.W * cam.H + 1023) / 1024;
-    float* part = scratch + nb_full * 4 + 320;
-    unsigned int* ticket = reinterpret_cast<unsigned int*>(part + nb_full * 2 * LADDER_N);
-    VTGS_CUDA_CHECK(cudaMemsetAsync(ticket, 0, sizeof(unsigned int), stream));
-    { VTGS_PROF("sil_ladder_kernel", stream); sil_ladder_kernel<<<nblocks, 256, 0, stream>>>(cam, image6, gt_rgb, gt_depth, part, ticket, sums10); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
-}
-
-int launch_sil_select(const float* sums10, float* sil_thres_dev, float* min_mse_dev, cudaStream_t stream) {
-    { VTGS_PROF("sil_select_kernel", stream); sil_select_kernel<<<1, 32, 0, stream>>>(sums10, sil_thres_dev, min_mse_dev); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
-}
-
 // ---- non-presence mask of the silhouette-driven Gaussian addition (reference src/vtgaussian_slam.py:747-760) ----
 __global__ void __launch_bounds__(256)
 nonpresence_mask_kernel(size_t P, const float* __restrict__ image6, const float* __restrict__ gt_depth, float sil_thres,
@@ -222,15 +193,6 @@ nonpresence_mask_kernel(size_t P, const float* __restrict__ image6, const float*
     }
 }
 
-int launch_nonpresence_mask(const VtgsCamera* camera, const float* image6, const float* gt_depth, float sil_thres,
-                            const uint32_t* median_state, uint8_t* mask_out, uint32_t* count_dev, cudaStream_t stream) {
-    const size_t P = (size_t)camera->image_width * camera->image_height;
-    if (count_dev) VTGS_CUDA_CHECK(cudaMemsetAsync(count_dev, 0, sizeof(uint32_t), stream));
-    { VTGS_PROF("nonpresence_mask_kernel", stream); nonpresence_mask_kernel<<<(unsigned)((P + 255) / 256), 256, 0, stream>>>(P, image6, gt_depth, sil_thres, median_state, mask_out, count_dev); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
-}
-
 // ---- FP32 FMA throughput probe ------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
 ffma_probe_kernel(long long iters, float* __restrict__ sink) {
@@ -243,14 +205,6 @@ ffma_probe_kernel(long long iters, float* __restrict__ sink) {
     }
     const float r = a0 + a1 + a2 + a3 + a4 + a5 + a6 + a7;
     if (r == 123456.789f) *sink = r;                     // never true: keeps the loop alive
-}
-
-int launch_ffma_probe(int64_t iters, float* sink, uint64_t* threads_out, cudaStream_t stream) {
-    const int blocks = 148 * 8;                          // 8 resident blocks of 256 threads per SM: 64 warps / SM
-    if (threads_out) *threads_out = (uint64_t)blocks * 256;
-    { VTGS_PROF("ffma_probe_kernel", stream); ffma_probe_kernel<<<blocks, 256, 0, stream>>>((long long)iters, sink); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
 }
 
 // Tracking loss (mode 0): sums of masked absolute differences; dL/dplane = w * sign * mask.
@@ -645,80 +599,12 @@ retie_dev_kernel(float* __restrict__ means3D, int64_t n, const float* __restrict
     means3D[3 * i + 2] = Rn[2] * cx + Rn[5] * cy + Rn[8] * cz;
 }
 
-int launch_retie_dev(float* means3D, int64_t n, const float* q_old, const float* t_old, const float* q_un, const float* t, cudaStream_t stream) {
-    if (n <= 0) return VTGS_OK;
-    { VTGS_PROF("retie_kernel", stream); retie_dev_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(means3D, n, q_old, t_old, q_un, t); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
-}
-
-int launch_retie(float* means3D, int64_t n, const float* w2c_old_rowmajor12, const float* q_un, const float* t, cudaStream_t stream) {
-    if (n <= 0) return VTGS_OK;
-    Mat34 m;
-    for (int k = 0; k < 12; ++k) m.m[k] = w2c_old_rowmajor12[k];
-    { VTGS_PROF("retie_kernel", stream); retie_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(means3D, n, m, q_un, t); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
-}
-
 static inline size_t band_pixels(const CamConst& cam) {
     const size_t P = (size_t)cam.W * cam.H;
     const size_t b = (size_t)cam.row0 * 16 * cam.W;
     size_t e = (size_t)cam.row1 * 16 * cam.W;
     if (e > P) e = P;
     return e > b ? e - b : 0;
-}
-
-int launch_loss(const VtgsCamera* camera, const VtgsLossConfig* cfg, const float* image6,
-                const float* gt_rgb, const float* gt_depth, float* dL_dimage4, float* loss_terms,
-                float* scratch, cudaStream_t stream) {
-    const CamConst cam = make_cam_const(*camera);
-    if (cfg->ignore_outlier_depth && cfg->mode != 0) { set_error("ignore_outlier_depth_loss is a tracking option"); return VTGS_E_UNSUPPORTED; }
-    if (cfg->ignore_outlier_depth && cfg->median_state == nullptr && (cam.row0 != 0 || cam.row1 != cam.gy)) {
-        set_error("ignore_outlier_depth_loss with a tile-row band needs VtgsLossConfig.median_state (vtgs_median_hist / all-reduce / vtgs_median_pick)");
-        return VTGS_E_UNSUPPORTED;
-    }
-    if (!cfg->use_l1) { set_error("use_l1 = False is not supported"); return VTGS_E_UNSUPPORTED; }
-    if (cfg->mode == 1) {
-        if (cam.row0 != 0 || cam.row1 != cam.gy) { set_error("mapping loss is not band-sharded"); return VTGS_E_INVALID; }
-        static const SsimWindow win = make_window();
-        const size_t P = (size_t)cam.W * cam.H;
-        const dim3 grid((cam.W + SSIM_T - 1) / SSIM_T, (cam.H + SSIM_T - 1) / SSIM_T, 3), block(256);
-        const int nb = (int)(grid.x * grid.y * grid.z);
-        float* maps = scratch;                      // 9 P floats
-        float* partials = scratch + 9 * P;          // nb * 4
-        { VTGS_PROF("ssim_forward_kernel", stream); launch_k(ssim_forward_kernel, dim3(grid), dim3(block), 0, stream, cam.W, cam.H, win, image6, gt_rgb, gt_depth, maps, partials); }
-        VTGS_LAUNCH_CHECK();
-        { VTGS_PROF("mapping_finalize_kernel", stream); launch_k(mapping_finalize_kernel, dim3(1), dim3(1024), 0, stream, partials, nb, cam.W, cam.H, *cfg, loss_terms); }
-        VTGS_LAUNCH_CHECK();
-        { VTGS_PROF("ssim_backward_kernel", stream); launch_k(ssim_backward_kernel, dim3(grid), dim3(block), 0, stream, cam.W, cam.H, win, *cfg, image6, gt_rgb, gt_depth, maps, loss_terms, dL_dimage4); }
-        VTGS_LAUNCH_CHECK();
-        return VTGS_OK;
-    }
-    if (cfg->mode != 0) { set_error("unknown loss mode"); return VTGS_E_INVALID; }
-    const size_t npx = band_pixels(cam);
-    const int nblocks = (int)((npx + 256 * LOSS_PX_PER_THREAD - 1) / (256 * LOSS_PX_PER_THREAD));
-    if (nblocks > 0) {
-        unsigned int* ticket = reinterpret_cast<unsigned int*>(scratch + (size_t)nblocks * LOSS_TERMS);
-        const unsigned int* median_state = nullptr;
-        if (cfg->ignore_outlier_depth && cfg->median_state != nullptr) {
-            median_state = cfg->median_state;
-        } else if (cfg->ignore_outlier_depth) {
-            unsigned int* st = ticket + 16;
-            const size_t P = (size_t)cam.W * cam.H;
-            VTGS_CUDA_CHECK(cudaMemsetAsync(st, 0, MEDIAN_STATE_WORDS * sizeof(unsigned int), stream));
-            for (int pass = 0; pass < 4; ++pass) {
-                if (int e = launch_median_hist(camera, image6 + 3 * P, gt_depth, pass, st, stream)) return e;
-                if (int e = launch_median_pick((int64_t)P, pass, st, stream)) return e;
-            }
-            median_state = st;
-        }
-        { VTGS_PROF("tracking_loss_kernel", stream); launch_k(tracking_loss_kernel, dim3(nblocks), dim3(256), 0, stream, cam, *cfg, image6, gt_rgb, gt_depth, dL_dimage4, scratch, ticket, loss_terms, median_state); }
-        VTGS_LAUNCH_CHECK();
-    } else {
-        VTGS_CUDA_CHECK(cudaMemsetAsync(loss_terms, 0, 8 * sizeof(float), stream));
-    }
-    return VTGS_OK;
 }
 
 // ---- Adam -----------------------------------------------------------------------------------
@@ -916,26 +802,6 @@ sharded_adam_mc_kernel(const __grid_constant__ ShardedAdamArgs a, uint64_t mc_ba
     }
 }
 
-int launch_sharded_adam(int world, int rank, const uint64_t* bases, uint64_t mc_base, int64_t param_off, int64_t grad_off, int64_t loss_off,
-                        float* m, float* v, int64_t n, int nseg, const int64_t* seg_end, const float* lr, float b1, float b2,
-                        float eps, const int32_t* step_dev, float* loss_out, cudaStream_t stream) {
-    ShardedAdamArgs a{};
-    a.nseg = nseg; a.world = world; a.rank = rank;
-    for (int k = 0; k < world; ++k) a.base[k] = bases[k];
-    for (int k = 0; k < world; ++k) a.pbase[k] = bases[k];
-    for (int k = 0; k < nseg; ++k) { a.seg_end[k] = seg_end[k]; a.lr[k] = lr[k]; }
-    const int64_t n4 = n / 4;
-    int blocks = 148 * 4;
-    if (const char* e = getenv("VTGS_SHARD_BLOCKS")) blocks = std::max(1, atoi(e));      // tools/bench_sharded_step.py (8 B200: flat from 296 blocks on)
-    { VTGS_PROF("sharded_adam_kernel", stream);
-      if (mc_base != 0) sharded_adam_mc_kernel<<<blocks, 256, 0, stream>>>(a, mc_base, param_off, grad_off, loss_off, m, v, n4, b1, b2, eps, step_dev, loss_out);
-      else if (world <= 2) sharded_adam_kernel<2, 4><<<blocks, 256, 0, stream>>>(a, param_off, grad_off, loss_off, m, v, n4, b1, b2, eps, step_dev, loss_out);
-      else if (world <= 4) sharded_adam_kernel<4, 2><<<blocks, 256, 0, stream>>>(a, param_off, grad_off, loss_off, m, v, n4, b1, b2, eps, step_dev, loss_out);
-      else sharded_adam_kernel<8, 1><<<blocks, 256, 0, stream>>>(a, param_off, grad_off, loss_off, m, v, n4, b1, b2, eps, step_dev, loss_out); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
-}
-
 // ---- tracking pose update: best-candidate bookkeeping + Adam on the 7 pose numbers, one launch ----
 // Reference src/vtgaussian_slam.py:1890 (optimizer.step) and :1961-1970 (keep the candidate pose with
 // the smallest loss; the loss of an iteration belongs to the pose BEFORE that iteration's step).
@@ -971,21 +837,188 @@ __global__ void tracking_update_kernel(float* __restrict__ cam_q, float* __restr
     if (s_better && (flags & VTGS_TRACK_BOOK_POST_STEP)) best[1 + k] = pn;
 }
 
-int launch_tracking_update(float* cam_q, float* cam_t, const float* msg, float* adam, int32_t* step_dev, float* best,
-                           float lr_rot, float lr_trans, float eps, int flags, cudaStream_t stream) {
-    { VTGS_PROF("tracking_update_kernel", stream); launch_k(tracking_update_kernel, dim3(1), dim3(32), 0, stream, cam_q, cam_t, msg, adam, step_dev, best, lr_rot, lr_trans, 0.9f, 0.999f, eps, flags); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
-}
-
-int launch_adam(float* param, const float* grad, float* m, float* v, int64_t n, float lr, float b1,
-                float b2, float eps, int step, const int32_t* step_dev, cudaStream_t stream) {
-    if (n <= 0) return VTGS_OK;
-    const bool vec4 = (n % 4 == 0) && (((uintptr_t)param | (uintptr_t)grad | (uintptr_t)m | (uintptr_t)v) & 15) == 0;
-    const int64_t threads = vec4 ? n / 4 : n;
-    { VTGS_PROF("adam_kernel", stream); launch_k(adam_kernel, dim3((unsigned)((threads + 255) / 256)), dim3(256), 0, stream, param, grad, m, v, n, lr, b1, b2, eps, step, step_dev, vec4 ? 1 : 0); }
-    VTGS_LAUNCH_CHECK();
-    return VTGS_OK;
-}
-
 }  // namespace vtgs
+
+// =============================== C entry points (include/vtgs.h) ===========================
+using namespace vtgs;
+
+uint64_t vtgs_loss_scratch_floats(int32_t W, int32_t H, int32_t mode) {
+    const uint64_t P = (uint64_t)W * H;
+    if (mode == 1) return 9 * P + ((uint64_t)((W + 15) / 16) * ((H + 15) / 16) * 3 + 1) * 4;
+    /* [tracking loss: 4 floats per 1024-pixel block + ticket + the radix-select state of the outlier median (320 words)
+     *  | silhouette ladder: 10 floats per block + ticket] */
+    return ((P + 1023) / 1024) * 14 + 320 + 16;
+}
+
+int vtgs_loss(const VtgsCamera* camera, const VtgsLossConfig* cfg, const float* image6, const float* gt_rgb,
+              const float* gt_depth, float* dL_dimage4, float* loss_terms, float* scratch, void* stream_) {
+    if (int e = check_cam(camera)) return e;
+    VTGS_REQUIRE(cfg && image6 && gt_rgb && gt_depth && dL_dimage4 && loss_terms && scratch, "pointer is NULL");
+    const cudaStream_t stream = (cudaStream_t)stream_;
+    const CamConst cam = make_cam_const(*camera);
+    if (cfg->ignore_outlier_depth && cfg->mode != 0) { set_error("ignore_outlier_depth_loss is a tracking option"); return VTGS_E_UNSUPPORTED; }
+    if (cfg->ignore_outlier_depth && cfg->median_state == nullptr && (cam.row0 != 0 || cam.row1 != cam.gy)) {
+        set_error("ignore_outlier_depth_loss with a tile-row band needs VtgsLossConfig.median_state (vtgs_median_hist / all-reduce / vtgs_median_pick)");
+        return VTGS_E_UNSUPPORTED;
+    }
+    if (!cfg->use_l1) { set_error("use_l1 = False is not supported"); return VTGS_E_UNSUPPORTED; }
+    if (cfg->mode == 1) {
+        if (cam.row0 != 0 || cam.row1 != cam.gy) { set_error("mapping loss is not band-sharded"); return VTGS_E_INVALID; }
+        static const SsimWindow win = make_window();
+        const size_t P = (size_t)cam.W * cam.H;
+        const dim3 grid((cam.W + SSIM_T - 1) / SSIM_T, (cam.H + SSIM_T - 1) / SSIM_T, 3), block(256);
+        const int nb = (int)(grid.x * grid.y * grid.z);
+        float* maps = scratch;                      // 9 P floats
+        float* partials = scratch + 9 * P;          // nb * 4
+        if (int e = launch_k("ssim_forward_kernel", Launch::pdl, ssim_forward_kernel, grid, block, 0, stream, cam.W, cam.H, win, image6, gt_rgb,
+                             gt_depth, maps, partials)) return e;
+        if (int e = launch_k("mapping_finalize_kernel", Launch::pdl, mapping_finalize_kernel, dim3(1), dim3(1024), 0, stream, partials, nb, cam.W,
+                             cam.H, *cfg, loss_terms)) return e;
+        return launch_k("ssim_backward_kernel", Launch::pdl, ssim_backward_kernel, grid, block, 0, stream, cam.W, cam.H, win, *cfg, image6, gt_rgb,
+                        gt_depth, maps, loss_terms, dL_dimage4);
+    }
+    if (cfg->mode != 0) { set_error("unknown loss mode"); return VTGS_E_INVALID; }
+    const size_t npx = band_pixels(cam);
+    const int nblocks = (int)((npx + 256 * LOSS_PX_PER_THREAD - 1) / (256 * LOSS_PX_PER_THREAD));
+    if (nblocks > 0) {
+        unsigned int* ticket = reinterpret_cast<unsigned int*>(scratch + (size_t)nblocks * LOSS_TERMS);
+        const unsigned int* median_state = nullptr;
+        if (cfg->ignore_outlier_depth && cfg->median_state != nullptr) {
+            median_state = cfg->median_state;
+        } else if (cfg->ignore_outlier_depth) {
+            unsigned int* st = ticket + 16;
+            const size_t P = (size_t)cam.W * cam.H;
+            VTGS_CUDA_CHECK(cudaMemsetAsync(st, 0, MEDIAN_STATE_WORDS * sizeof(unsigned int), stream));
+            for (int pass = 0; pass < 4; ++pass) {
+                if (int e = launch_median_hist(camera, image6 + 3 * P, gt_depth, pass, st, stream)) return e;
+                if (int e = launch_median_pick((int64_t)P, pass, st, stream)) return e;
+            }
+            median_state = st;
+        }
+        return launch_k("tracking_loss_kernel", Launch::pdl, tracking_loss_kernel, dim3(nblocks), dim3(256), 0, stream, cam, *cfg, image6, gt_rgb,
+                        gt_depth, dL_dimage4, scratch, ticket, loss_terms, median_state);
+    }
+    VTGS_CUDA_CHECK(cudaMemsetAsync(loss_terms, 0, 8 * sizeof(float), stream));
+    return VTGS_OK;
+}
+
+int vtgs_median_hist(const VtgsCamera* cam, const float* depth_plane, const float* gt_depth, int32_t pass, uint32_t* state, void* stream) {
+    if (int e = check_cam(cam)) return e;
+    VTGS_REQUIRE(depth_plane && gt_depth && state, "pointer is NULL");
+    VTGS_REQUIRE(pass >= 0 && pass < 4, "pass must be 0..3");
+    return launch_median_hist(cam, depth_plane, gt_depth, pass, state, (cudaStream_t)stream);
+}
+
+int vtgs_median_pick(int64_t num_pixels_total, int32_t pass, uint32_t* state, void* stream) {
+    VTGS_REQUIRE(state != nullptr && num_pixels_total > 0, "bad argument");
+    VTGS_REQUIRE(pass >= 0 && pass < 4, "pass must be 0..3");
+    return launch_median_pick(num_pixels_total, pass, state, (cudaStream_t)stream);
+}
+
+int vtgs_sil_ladder(const VtgsCamera* camera, const float* image6, const float* gt_rgb, const float* gt_depth, float* sums10,
+                    float* scratch, void* stream_) {
+    if (int e = check_cam(camera)) return e;
+    VTGS_REQUIRE(image6 && gt_rgb && gt_depth && sums10 && scratch, "pointer is NULL");
+    const cudaStream_t stream = (cudaStream_t)stream_;
+    const CamConst cam = make_cam_const(*camera);
+    size_t b, e;
+    band_pixel_range(cam, b, e);
+    const int nblocks = (int)((e - b + 1023) / 1024);
+    if (nblocks <= 0) { VTGS_CUDA_CHECK(cudaMemsetAsync(sums10, 0, 10 * sizeof(float), stream)); return VTGS_OK; }
+    // the loss scratch (vtgs_loss_scratch_floats, mode 0) = [tracking-loss region: 4 floats per 1024-pixel block of the
+    // whole frame, its ticket, the median state | ladder region: 10 floats per block, its ticket]: the two never overlap,
+    // so the tracking loss's self-resetting ticket stays intact
+    const size_t nb_full = ((size_t)cam.W * cam.H + 1023) / 1024;
+    float* part = scratch + nb_full * 4 + 320;
+    unsigned int* ticket = reinterpret_cast<unsigned int*>(part + nb_full * 2 * LADDER_N);
+    VTGS_CUDA_CHECK(cudaMemsetAsync(ticket, 0, sizeof(unsigned int), stream));
+    return launch_k("sil_ladder_kernel", Launch::plain, sil_ladder_kernel, dim3(nblocks), dim3(256), 0, stream, cam, image6, gt_rgb, gt_depth,
+                    part, ticket, sums10);
+}
+
+int vtgs_sil_select(const float* sums10, float* sil_thres_dev, float* min_mse_dev, void* stream) {
+    VTGS_REQUIRE(sums10 && sil_thres_dev, "pointer is NULL");
+    return launch_k("sil_select_kernel", Launch::plain, sil_select_kernel, dim3(1), dim3(32), 0, (cudaStream_t)stream, sums10, sil_thres_dev,
+                    min_mse_dev);
+}
+
+int vtgs_nonpresence_mask(const VtgsCamera* camera, const float* image6, const float* gt_depth, float sil_thres,
+                          const uint32_t* median_state, uint8_t* mask_out, uint32_t* count_dev, void* stream_) {
+    if (int e = check_cam(camera)) return e;
+    VTGS_REQUIRE(image6 && gt_depth && median_state && mask_out, "pointer is NULL");
+    const cudaStream_t stream = (cudaStream_t)stream_;
+    const size_t P = (size_t)camera->image_width * camera->image_height;
+    if (count_dev) VTGS_CUDA_CHECK(cudaMemsetAsync(count_dev, 0, sizeof(uint32_t), stream));
+    return launch_k("nonpresence_mask_kernel", Launch::plain, nonpresence_mask_kernel, dim3((unsigned)((P + 255) / 256)), dim3(256), 0, stream,
+                    P, image6, gt_depth, sil_thres, median_state, mask_out, count_dev);
+}
+
+int vtgs_ffma_probe(int64_t iters, float* sink, uint64_t* threads_out, void* stream) {
+    VTGS_REQUIRE(iters > 0 && sink != nullptr, "bad argument");
+    const int blocks = 148 * 8;                          // 8 resident blocks of 256 threads per SM: 64 warps / SM
+    if (threads_out) *threads_out = (uint64_t)blocks * 256;
+    return launch_k("ffma_probe_kernel", Launch::plain, ffma_probe_kernel, dim3(blocks), dim3(256), 0, (cudaStream_t)stream, (long long)iters, sink);
+}
+
+int vtgs_retie(float* means3D, int64_t n, const float* w2c_old, const float* cam_unnorm_rot, const float* cam_trans, void* stream) {
+    VTGS_REQUIRE(n >= 0, "n < 0");
+    VTGS_REQUIRE(w2c_old && cam_unnorm_rot && cam_trans && (n == 0 || means3D), "pointer is NULL");
+    if (n <= 0) return VTGS_OK;
+    Mat34 m;
+    for (int k = 0; k < 12; ++k) m.m[k] = w2c_old[k];
+    return launch_k("retie_kernel", Launch::plain, retie_kernel, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, (cudaStream_t)stream, means3D, n,
+                    m, cam_unnorm_rot, cam_trans);
+}
+
+int vtgs_retie_dev(float* means3D, int64_t n, const float* old_unnorm_rot, const float* old_trans, const float* cam_unnorm_rot,
+                   const float* cam_trans, void* stream) {
+    VTGS_REQUIRE(n >= 0, "n < 0");
+    VTGS_REQUIRE(old_unnorm_rot && old_trans && cam_unnorm_rot && cam_trans && (n == 0 || means3D), "pointer is NULL");
+    if (n <= 0) return VTGS_OK;
+    return launch_k("retie_kernel", Launch::plain, retie_dev_kernel, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, (cudaStream_t)stream,
+                    means3D, n, old_unnorm_rot, old_trans, cam_unnorm_rot, cam_trans);
+}
+
+int vtgs_adam(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1,
+              float beta2, float eps, int32_t step, const int32_t* step_dev, void* stream) {
+    VTGS_REQUIRE(n >= 0, "n < 0");
+    if (n > 0) VTGS_REQUIRE(param && grad && exp_avg && exp_avg_sq, "pointer is NULL");
+    VTGS_REQUIRE(step_dev != nullptr || step >= 1, "step must be >= 1");
+    if (n <= 0) return VTGS_OK;
+    const bool vec4 = (n % 4 == 0) && (((uintptr_t)param | (uintptr_t)grad | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq) & 15) == 0;
+    const int64_t threads = vec4 ? n / 4 : n;
+    return launch_k("adam_kernel", Launch::pdl, adam_kernel, dim3((unsigned)((threads + 255) / 256)), dim3(256), 0, (cudaStream_t)stream, param,
+                    grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, step, step_dev, vec4 ? 1 : 0);
+}
+
+int vtgs_sharded_adam(int32_t world, int32_t rank, const uint64_t* peer_bases, uint64_t multicast_base, int64_t param_off, int64_t grad_off, int64_t loss_off,
+                      float* exp_avg, float* exp_avg_sq, int64_t n, int32_t nseg, const int64_t* seg_end, const float* lr, float beta1,
+                      float beta2, float eps, const int32_t* step_dev, float* loss_out, void* stream) {
+    VTGS_REQUIRE(world >= 1 && world <= 8 && rank >= 0 && rank < world, "world must be 1..8 and rank inside it");
+    VTGS_REQUIRE(peer_bases && exp_avg && exp_avg_sq && seg_end && lr && step_dev && loss_out, "pointer is NULL");
+    VTGS_REQUIRE(n >= 0 && n % 4 == 0 && param_off % 4 == 0 && grad_off % 4 == 0, "flat vectors must be multiples of 4 floats");
+    VTGS_REQUIRE(nseg >= 1 && nseg <= 4, "1..4 segments");
+    for (int k = 0; k < world; ++k) VTGS_REQUIRE(peer_bases[k] != 0 && (peer_bases[k] & 15) == 0, "peer base must be a 16-byte aligned address");
+    VTGS_REQUIRE((multicast_base & 15) == 0, "multicast base must be 16-byte aligned");
+    ShardedAdamArgs a{};
+    a.nseg = nseg; a.world = world; a.rank = rank;
+    for (int k = 0; k < world; ++k) a.base[k] = peer_bases[k];
+    for (int k = 0; k < world; ++k) a.pbase[k] = peer_bases[k];
+    for (int k = 0; k < nseg; ++k) { a.seg_end[k] = seg_end[k]; a.lr[k] = lr[k]; }
+    const int64_t n4 = n / 4;
+    int blocks = 148 * 4;
+    if (const char* e = getenv("VTGS_SHARD_BLOCKS")) blocks = std::max(1, atoi(e));      // tools/bench_sharded_step.py (8 B200: flat from 296 blocks on)
+    if (multicast_base != 0)
+        return launch_k("sharded_adam_kernel", Launch::plain, sharded_adam_mc_kernel, dim3(blocks), dim3(256), 0, (cudaStream_t)stream, a,
+                        multicast_base, param_off, grad_off, loss_off, exp_avg, exp_avg_sq, n4, beta1, beta2, eps, step_dev, loss_out);
+    auto k = world <= 2 ? sharded_adam_kernel<2, 4> : world <= 4 ? sharded_adam_kernel<4, 2> : sharded_adam_kernel<8, 1>;
+    return launch_k("sharded_adam_kernel", Launch::plain, k, dim3(blocks), dim3(256), 0, (cudaStream_t)stream, a, param_off, grad_off, loss_off,
+                    exp_avg, exp_avg_sq, n4, beta1, beta2, eps, step_dev, loss_out);
+}
+
+int vtgs_tracking_update(float* cam_unnorm_rot, float* cam_trans, const float* msg, float* adam_state, int32_t* step_dev,
+                         float* best, float lr_rot, float lr_trans, float eps, int32_t flags, void* stream) {
+    VTGS_REQUIRE(cam_unnorm_rot && cam_trans && msg && adam_state && step_dev && best, "pointer is NULL");
+    return launch_k("tracking_update_kernel", Launch::pdl, tracking_update_kernel, dim3(1), dim3(32), 0, (cudaStream_t)stream, cam_unnorm_rot,
+                    cam_trans, msg, adam_state, step_dev, best, lr_rot, lr_trans, 0.9f, 0.999f, eps, flags);
+}

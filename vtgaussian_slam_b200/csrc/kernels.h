@@ -1,82 +1,54 @@
-// kernels.h -- internal launch interface between the translation units of libvtgs_cuda.so.
+// kernels.h -- what the translation units of libvtgs_cuda.so share on the host: the argument checks of the C entry
+// points and the internal calls one file makes into another.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include "../../include/vtgs.h"
+#include "common.cuh"
 
 namespace vtgs {
 
-// RAII event bracket around one kernel launch (only when vtgs_profile_enable(1) was called).
-struct ProfScope {
-    ProfScope(const char* name, cudaStream_t stream);
-    ~ProfScope();
-    int slot;
-    cudaStream_t stream;
-};
-#define VTGS_PROF(name, stream) vtgs::ProfScope _prof_scope(name, stream)
+#define VTGS_REQUIRE(cond, msg)                           \
+    do {                                                  \
+        if (!(cond)) {                                    \
+            vtgs::set_error("invalid argument: %s", msg); \
+            return VTGS_E_INVALID;                        \
+        }                                                 \
+    } while (0)
 
-// Front end of the fused path (transform_to_frame + activations); unused in API mode.
-struct FrontEnd {
-    const float* cam_unnorm_rot;   // device [4]: the frame's un-normalised pose quaternion
-    const float* cam_trans;        // device [3]
-    VtgsCounters* counters;        // device: receives pose_R / pose_t / pose_q / pose_qnorm for the backward
-    float depth_row[4];
-    int log_scales_dim;
-};
+inline int check_cam(const VtgsCamera* cam) {
+    VTGS_REQUIRE(cam != nullptr, "cam is NULL");
+    VTGS_REQUIRE(cam->image_width > 0 && cam->image_height > 0, "image size must be positive");
+    VTGS_REQUIRE(cam->tanfovx > 0.f && cam->tanfovy > 0.f, "tanfov must be positive");
+    VTGS_REQUIRE(cam->radius_sigma_mult > 0.f, "radius_sigma_mult must be positive");
+    return VTGS_OK;
+}
 
-int launch_forward(const VtgsCamera* cam, int64_t N, bool fused, const FrontEnd& fe,
-                   const float* means3D, const float* scales, const float* rotations,
-                   const float* opacities, const float* colors,
-                   float* out_color, float* out_depth, int32_t* radii, VtgsBuffers* buf,
-                   cudaStream_t stream);
-int launch_export_keys(const VtgsCamera* cam, const VtgsBuffers* buf, uint64_t* out, uint64_t cap, cudaStream_t stream);
-int launch_export_geometry(int64_t N, const VtgsBuffers* buf, float* means2D, float* depths, float* conic_opacity, cudaStream_t stream);
-int launch_mark_visible(const VtgsCamera* cam, int64_t N, const float* means3D, uint8_t* present, cudaStream_t stream);
+inline int check_buf(const VtgsBuffers* b, int64_t N) {
+    VTGS_REQUIRE(b != nullptr, "buffers is NULL");
+    VTGS_REQUIRE(b->tile_counts && b->tile_ranges && b->final_T && b->n_contrib && b->counters && b->region_cnt && b->region_masks && b->region_done, "workspace pointer is NULL");
+    if (N > 0) VTGS_REQUIRE(b->geom && b->tiles_touched && b->grad_geom, "per-Gaussian workspace pointer is NULL");
+    VTGS_REQUIRE(b->pair_capacity == 0 || (b->pair_keys && b->point_list && b->region_pairs), "pair workspace pointer is NULL");
+    VTGS_REQUIRE(b->pair_capacity < 0xffffffffull, "pair_capacity must fit 32 bits");
+    return VTGS_OK;
+}
 
-// API-mode backward (K6 + K7).
-int launch_backward(const VtgsCamera* cam, int64_t N,
-                    const float* means3D, const float* scales, const float* rotations,
-                    const float* opacities, const float* colors, const float* dL_dout_color,
-                    float* dL_dmeans2D, float* dL_dcolors, float* dL_dopacity,
-                    float* dL_dmeans3D, float* dL_dscales, float* dL_drotations,
-                    VtgsBuffers* buf, cudaStream_t stream);
+inline int check_fused(const VtgsCamera* cam, const VtgsParams* p, const VtgsPose* pose, const VtgsBuffers* buf) {
+    if (int e = check_cam(cam)) return e;
+    VTGS_REQUIRE(p && pose, "params / pose is NULL");
+    if (int e = check_buf(buf, p->num_gaussians)) return e;
+    VTGS_REQUIRE(p->num_gaussians >= 0, "num_gaussians < 0");
+    if (p->num_gaussians > 0)
+        VTGS_REQUIRE(p->means3D && p->rgb_colors && p->unnorm_rotations && p->logit_opacities && p->log_scales, "param pointer is NULL");
+    VTGS_REQUIRE(pose->cam_unnorm_rot && pose->cam_trans, "pose pointer is NULL");
+    if (p->log_scales_dim != 1) {
+        set_error("fused path supports isotropic Gaussians only (log_scales [N,1]); use vtgs_forward/backward for anisotropic");
+        return VTGS_E_UNSUPPORTED;
+    }
+    return VTGS_OK;
+}
 
-// Fused path.
+// backward.cu: publishes the frame's pose for the backward when the fused forward has no Gaussian to preprocess.
 int launch_pose_matrix(const VtgsPose* pose, VtgsCounters* counters, cudaStream_t stream);
-int launch_fused_backward(const VtgsCamera* cam, const VtgsParams* params, const VtgsPose* pose,
-                          const float* dL_dimage4, int accumulate, VtgsParamGrads* grads,
-                          VtgsBuffers* buf, cudaStream_t stream);
-int launch_loss(const VtgsCamera* cam, const VtgsLossConfig* cfg, const float* image6,
-                const float* gt_rgb, const float* gt_depth, float* dL_dimage4, float* loss_terms,
-                float* scratch, cudaStream_t stream);
-int launch_tracking_update(float* cam_q, float* cam_t, const float* msg, float* adam, int32_t* step_dev, float* best,
-                           float lr_rot, float lr_trans, float eps, int flags, cudaStream_t stream);
-int launch_median_hist(const VtgsCamera* cam, const float* depth_plane, const float* gt_depth, int pass, uint32_t* state, cudaStream_t stream);
-int launch_median_pick(int64_t P_total, int pass, uint32_t* state, cudaStream_t stream);
-int launch_sil_ladder(const VtgsCamera* cam, const float* image6, const float* gt_rgb, const float* gt_depth, float* sums10,
-                      float* scratch, cudaStream_t stream);
-int launch_sil_select(const float* sums10, float* sil_thres_dev, float* min_mse_dev, cudaStream_t stream);
-int launch_nonpresence_mask(const VtgsCamera* cam, const float* image6, const float* gt_depth, float sil_thres,
-                            const uint32_t* median_state, uint8_t* mask_out, uint32_t* count_dev, cudaStream_t stream);
-int launch_eval_metrics(const VtgsCamera* cam, const float* image6, const float* gt_rgb, const float* gt_depth, float sil_thres,
-                        int use_presence, float* out8, float* scratch, cudaStream_t stream);
-uint64_t eval_scratch_floats();
-int launch_p2p_prepare(int W, int H, const float* intr4, const float* c2w12, const float* other_w2c12, const float* depth,
-                       const uint8_t* mask, float* pts, float* nrm, uint8_t* valid, cudaStream_t stream);
-int launch_p2p_match(int64_t n_tgt, const float* tgt_pts, const float* tgt_nrm, const uint8_t* tgt_valid, int64_t n_src,
-                     const float* src_pts, const uint8_t* src_valid, float max_dist, int32_t* table, int64_t table_size,
-                     int32_t* next, float* out_dist, int32_t* out_idx, cudaStream_t stream);
-int launch_frame_convert(int sw, int sh, int dw, int dh, const uint8_t* rgb, const uint16_t* depth, double depth_scale, float* im,
-                         float* depth_out, cudaStream_t stream);
-int launch_book_radii(int64_t n, const int32_t* radii, float* max_radius, uint8_t* seen, cudaStream_t stream);
-int launch_ffma_probe(int64_t iters, float* sink, uint64_t* threads_out, cudaStream_t stream);
-int launch_retie(float* means3D, int64_t n, const float* w2c_old_rowmajor12, const float* q_un, const float* t, cudaStream_t stream);
-int launch_retie_dev(float* means3D, int64_t n, const float* q_old, const float* t_old, const float* q_un, const float* t, cudaStream_t stream);
-int launch_adam(float* param, const float* grad, float* m, float* v, int64_t n, float lr, float b1,
-                float b2, float eps, int step, const int32_t* step_dev, cudaStream_t stream);
-int launch_sharded_adam(int world, int rank, const uint64_t* bases, uint64_t mc_base, int64_t param_off, int64_t grad_off, int64_t loss_off,
-                        float* m, float* v, int64_t n, int nseg, const int64_t* seg_end, const float* lr, float b1, float b2,
-                        float eps, const int32_t* step_dev, float* loss_out, cudaStream_t stream);
 
 }  // namespace vtgs
