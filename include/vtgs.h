@@ -439,6 +439,24 @@ VTGS_API int vtgs_retie_dev(float* means3D, int64_t n, const float* old_unnorm_r
                             const float* cam_unnorm_rot, const float* cam_trans, void* stream);
 
 /*
+ * The re-ties of a keyframe-sharded bundle-adjustment iteration, every rank's in one launch and without a host round
+ * trip.  Each rank writes one record per keyframe whose pose it stepped into its table of records_per_rank records:
+ *   words  0-3   int32 valid (0 = empty slot), id (the keyframe's frame index), n_last (rows to re-tie, 0 = none), reserved
+ *   words  4-10  float old_q[4], old_t[3]: the pose before the step
+ *   words 11-17  float new_q[4], new_t[3]: the pose after the step
+ *   words 18-19  pad (a record is VTGS_BA_RECORD_WORDS words; tables are 16-byte aligned)
+ *   table_bases[world]  HOST array: device address, in THIS process, of rank r's table (a peer mapping, or a local copy)
+ *   means3D[n_rows, 3]  re-tied in place
+ *   table_out           NULL, or [world * records_per_rank * VTGS_BA_RECORD_WORDS] words: receives the tables in rank order
+ * For every rank r, then every slot s, in that order, a record with valid != 0 and n_last > 0 re-ties the rows
+ * [n_rows - min(n_last, n_rows), n_rows) exactly as vtgs_retie_dev(old -> new) does.  A row covered by several records goes
+ * through them in (rank, slot) order, so one call gives the bits of the same sequence of vtgs_retie_dev calls.  world <= 8.
+ */
+#define VTGS_BA_RECORD_WORDS 20
+VTGS_API int vtgs_retie_records(int32_t world, const uint64_t* table_bases, int32_t records_per_rank, float* means3D,
+                                int64_t n_rows, uint32_t* table_out, void* stream);
+
+/*
  * Tracking pose update in one launch: the reference's `optimizer.step()` on the frame's pose slices
  * (src/vtgaussian_slam.py:1890, Adam betas (0.9, 0.999)) plus its best-candidate bookkeeping (:1961-1970).
  *   msg[16]        = {dL/dq[4], dL/dt[3], pad, loss_terms[8]}  (the all-reduced message of an iteration)

@@ -1,6 +1,7 @@
 """torchrun --nproc-per-node 2 tools/check_multi_gpu.py : tile-band sharded tracking == the unsharded solver, for the
 plain loss, Replica's iteration-0 threshold search (10 floats all-reduced) and the frame-wide outlier median (radix-select
-histograms all-reduced); keyframe-sharded mapping == the unsharded solver."""
+histograms all-reduced); keyframe-sharded mapping == the unsharded solver, also with bundle adjustment and re-tie
+(`do_ba`, `retie_last`: every rank's means3D and ba_poses() bitwise equal to rank 0's)."""
 import os
 import sys
 
@@ -78,6 +79,46 @@ ok &= good
 if rank == 0:
     print("mapping", "OK" if good else "MISMATCH", [o[0] for o in out], [float(np.abs(out[0][1] - o[1]).max()) for o in out[1:]],
           "fused vs nccl:", float(np.abs(out[1][1] - out[2][1]).max()), flush=True)
+
+# keyframe-sharded mapping with bundle adjustment: the owners step the poses, the records are exchanged and every rank
+# re-ties the section's newest Gaussians (two overlapping ranges) to them.  The keyframes are dealt rank-major, so the
+# (rank, slot) order of the re-ties is the single run's keyframe order.
+lrs = dict(rgb_colors=0.0025, logit_opacities=0.05, log_scales=0.005, cam_unnorm_rots=1e-4, cam_trans=1e-3)
+N = p["means3D"].shape[0]
+per = (len(kfs) + world - 1) // world
+out = []
+for mode in ("single", "nccl", "fused"):
+    print(f"[rank {rank}] mapping do_ba {mode}", file=sys.stderr, flush=True)
+    sharded = mode != "single"
+    ms = MappingSolver(settings, {k: torch.tensor(v, device=dev) for k, v in p.items()}, device=dev, lrs=lrs,
+                       process_group=pg if sharded else None, sharded_step=(mode == "fused") and "auto")
+    if mode == "fused" and rank == 0:
+        print("do_ba fused step:", "ON" if ms.sharded is not None else f"unavailable: {ms.sharded_error}", flush=True)
+    ba = [dict(kf, cam_q=kf["cam_q"].clone(), cam_t=kf["cam_t"].clone(), id=k) for k, kf in enumerate(kfs)]
+    ba[1]["retie_last"], ba[3]["retie_last"] = N // 3, N // 4
+    mine = ba[rank * per:(rank + 1) * per] if sharded else ba
+    for _ in range(5):
+        loss = ms.iteration(mine, do_ba=True)
+    poses = ms.ba_poses() if sharded else {kf["id"]: (kf["cam_q"].cpu(), kf["cam_t"].cpu()) for kf in ba}
+    pose_vec = torch.cat([torch.cat(poses[k]) for k in sorted(poses)]).to(dev)
+    means = ms.params["means3D"]
+    same = True
+    if sharded:                                           # every replica bitwise equal to rank 0's
+        for v in (means.reshape(-1), pose_vec):
+            allv = [torch.empty_like(v) for _ in range(world)]
+            dist.all_gather(allv, v.contiguous(), group=pg)
+            same &= all(torch.equal(allv[0], a) for a in allv)
+    out.append((float(loss.item()), ms.params["rgb_colors"].cpu().numpy().copy(), ms.params["log_scales"].cpu().numpy().copy(),
+                pose_vec.cpu().numpy(), means.cpu().numpy().copy(), same, sorted(poses)))
+good = True
+for o in out[1:]:
+    good &= o[5] and o[6] == out[0][6] and abs(out[0][0] - o[0]) <= 1e-4 * abs(out[0][0])
+    good &= all(np.abs(out[0][i] - o[i]).max() <= 2e-3 for i in (1, 2, 3, 4))
+ok &= good
+if rank == 0:
+    print("mapping do_ba + retie", "OK" if good else "MISMATCH", [o[0] for o in out], "replicas equal:", [o[5] for o in out[1:]],
+          "max |d| params / poses / means3D:", [[float(np.abs(out[0][i] - o[i]).max()) for i in (1, 3, 4)] for o in out[1:]],
+          flush=True)
 flag = torch.tensor([1.0 if ok else 0.0], device=dev)
 dist.all_reduce(flag, op=dist.ReduceOp.MIN)
 passed = flag.item() == 1.0

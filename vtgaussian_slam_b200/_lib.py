@@ -19,6 +19,7 @@ TRACK_CALLER_METRIC = 2
 GEOM_RECORD_BYTES = 64
 GRAD_GEOM_FLOATS = 32
 BUF_DETERMINISTIC = 1
+BA_RECORD_WORDS = 20
 
 
 class VtgsCamera(C.Structure):
@@ -112,6 +113,7 @@ SYMBOLS = {
                                     C.c_float, C.c_float, C.c_float, _P, _P, _P]),
     "vtgs_retie": (C.c_int, [_P, C.c_int64, C.POINTER(C.c_float * 12), _P, _P, _P]),
     "vtgs_retie_dev": (C.c_int, [_P, C.c_int64, _P, _P, _P, _P, _P]),
+    "vtgs_retie_records": (C.c_int, [C.c_int32, _P, C.c_int32, _P, C.c_int64, _P, _P]),
     "vtgs_tracking_update": (C.c_int, [_P, _P, _P, _P, _P, _P, C.c_float, C.c_float, C.c_float, C.c_int32, _P]),
     "vtgs_median_hist": (C.c_int, [C.POINTER(VtgsCamera), _P, _P, C.c_int32, _P, _P]),
     "vtgs_median_pick": (C.c_int, [C.c_int64, C.c_int32, _P, _P]),

@@ -569,12 +569,10 @@ retie_kernel(float* __restrict__ means3D, int64_t n, const Mat34 old, const floa
 }
 
 // The same with the OLD pose on the device too (the mapping step snapshots the pose before its Adam update): no host
-// round trip, so the mapping iteration stays free of synchronisation.
-__global__ void __launch_bounds__(256)
-retie_dev_kernel(float* __restrict__ means3D, int64_t n, const float* __restrict__ q_old, const float* __restrict__ t_old,
-                 const float* __restrict__ q_un, const float* __restrict__ t) {
-    const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
-    if (i >= n) return;
+// round trip, so the mapping iteration stays free of synchronisation.  retie_row re-ties row i; retie_dev_kernel and
+// retie_records_kernel both go through it, so their results agree bit for bit.
+__device__ __forceinline__ void retie_row(float* __restrict__ means3D, int64_t i, const float* __restrict__ q_old,
+                                          const float* __restrict__ t_old, const float* __restrict__ q_un, const float* __restrict__ t) {
     float Ro[9], Rn[9];
     {
         const float u0 = q_old[0], u1 = q_old[1], u2 = q_old[2], u3 = q_old[3];
@@ -597,6 +595,61 @@ retie_dev_kernel(float* __restrict__ means3D, int64_t n, const float* __restrict
     means3D[3 * i] = Rn[0] * cx + Rn[3] * cy + Rn[6] * cz;          // R_new^T (p_cam - t_new)
     means3D[3 * i + 1] = Rn[1] * cx + Rn[4] * cy + Rn[7] * cz;
     means3D[3 * i + 2] = Rn[2] * cx + Rn[5] * cy + Rn[8] * cz;
+}
+
+__global__ void __launch_bounds__(256)
+retie_dev_kernel(float* __restrict__ means3D, int64_t n, const float* __restrict__ q_old, const float* __restrict__ t_old,
+                 const float* __restrict__ q_un, const float* __restrict__ t) {
+    const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (i >= n) return;
+    retie_row(means3D, i, q_old, t_old, q_un, t);
+}
+
+// ---- the re-ties of a keyframe-sharded bundle-adjustment iteration, every rank's records in one launch ----------------
+// Record (VTGS_BA_RECORD_WORDS 32-bit words, include/vtgs.h): valid, id, n_last, reserved | old_q[4] old_t[3] |
+// new_q[4] new_t[3] | pad[2].  Each block stages the records in shared memory, RECORD_CHUNK at a time, and walks the
+// rows from the lowest one a staged record re-ties.  A row always belongs to the same thread (its index modulo the grid's
+// thread count), so the chunks reach it in (rank, slot) order: the order of the unsharded solver's retie_dev calls.
+constexpr int RECORD_WORDS = VTGS_BA_RECORD_WORDS;
+constexpr int RECORD_CHUNK = 64;                  // 8 ranks x 8 records: the mapping solver's whole exchange in one chunk
+constexpr int RECORDS_MAX_WORLD = 8;
+static_assert(RECORD_WORDS % 4 == 0, "records are read as 16-byte vectors");
+struct RecordTables { uint64_t base[RECORDS_MAX_WORLD]; };
+
+__global__ void __launch_bounds__(256)
+retie_records_kernel(const __grid_constant__ RecordTables tabs, int world, int records_per_rank, float* __restrict__ means3D,
+                     int64_t n_rows, uint32_t* __restrict__ table_out) {
+    __shared__ uint4 s_rec[RECORD_CHUNK * RECORD_WORDS / 4];
+    const uint32_t* rec = reinterpret_cast<const uint32_t*>(s_rec);
+    const int64_t total = (int64_t)world * records_per_rank, stride = (int64_t)gridDim.x * 256;
+    for (int64_t c0 = 0; c0 < total; c0 += RECORD_CHUNK) {
+        const int nrec = (int)min((int64_t)RECORD_CHUNK, total - c0);
+        for (int k = threadIdx.x; k < nrec * (RECORD_WORDS / 4); k += 256) {
+            const int64_t r = (c0 + k / (RECORD_WORDS / 4)) / records_per_rank, s = (c0 + k / (RECORD_WORDS / 4)) % records_per_rank;
+            const uint4 w = reinterpret_cast<const uint4*>(tabs.base[r])[s * (RECORD_WORDS / 4) + k % (RECORD_WORDS / 4)];
+            s_rec[k] = w;
+            if (table_out != nullptr && blockIdx.x == 0) {
+                uint32_t* o = table_out + c0 * RECORD_WORDS + 4 * (int64_t)k;
+                o[0] = w.x; o[1] = w.y; o[2] = w.z; o[3] = w.w;
+            }
+        }
+        __syncthreads();
+        int64_t lo = n_rows;
+        for (int j = 0; j < nrec; ++j) {
+            const int32_t n_last = (int32_t)rec[j * RECORD_WORDS + 2];
+            if (rec[j * RECORD_WORDS] != 0u && n_last > 0) lo = min(lo, n_rows - min((int64_t)n_last, n_rows));
+        }
+        for (int64_t i = lo / stride * stride + (int64_t)blockIdx.x * 256 + threadIdx.x; i < n_rows; i += stride) {
+            for (int j = 0; j < nrec; ++j) {
+                const uint32_t* R = rec + j * RECORD_WORDS;
+                const int32_t n_last = (int32_t)R[2];
+                if (R[0] == 0u || n_last <= 0 || i < n_rows - min((int64_t)n_last, n_rows)) continue;
+                const float* f = reinterpret_cast<const float*>(R);
+                retie_row(means3D, i, f + 4, f + 8, f + 11, f + 15);
+            }
+        }
+        __syncthreads();
+    }
 }
 
 static inline size_t band_pixels(const CamConst& cam) {
@@ -977,6 +1030,21 @@ int vtgs_retie_dev(float* means3D, int64_t n, const float* old_unnorm_rot, const
     if (n <= 0) return VTGS_OK;
     return launch_k("retie_kernel", Launch::plain, retie_dev_kernel, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, (cudaStream_t)stream,
                     means3D, n, old_unnorm_rot, old_trans, cam_unnorm_rot, cam_trans);
+}
+
+int vtgs_retie_records(int32_t world, const uint64_t* table_bases, int32_t records_per_rank, float* means3D, int64_t n_rows,
+                       uint32_t* table_out, void* stream) {
+    VTGS_REQUIRE(world >= 1 && world <= RECORDS_MAX_WORLD, "world must be 1..8");
+    VTGS_REQUIRE(records_per_rank >= 1, "records_per_rank must be >= 1");
+    VTGS_REQUIRE(n_rows >= 0, "n_rows < 0");
+    VTGS_REQUIRE(table_bases && (n_rows == 0 || means3D), "pointer is NULL");
+    for (int k = 0; k < world; ++k) VTGS_REQUIRE(table_bases[k] != 0 && (table_bases[k] & 15) == 0, "table base must be a 16-byte aligned address");
+    if (n_rows == 0 && table_out == nullptr) return VTGS_OK;
+    RecordTables tabs{};
+    for (int k = 0; k < world; ++k) tabs.base[k] = table_bases[k];
+    const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>((n_rows + 255) / 256, 148 * 2));
+    return launch_k("retie_records_kernel", Launch::plain, retie_records_kernel, dim3(blocks), dim3(256), 0, (cudaStream_t)stream, tabs, (int)world,
+                    (int)records_per_rank, means3D, n_rows, table_out);
 }
 
 int vtgs_adam(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1,

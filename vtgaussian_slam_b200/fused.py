@@ -13,6 +13,7 @@ All compute is in libvtgs_cuda.so (include/vtgs.h); no CPU path.
 from __future__ import annotations
 
 import ctypes as C
+import operator
 import os
 
 import torch
@@ -22,6 +23,7 @@ from .rasterizer import (Workspace, _ptr, _require_cuda, _stream_ptr, _tensor_by
                          initial_pair_capacity, run_fitting)
 
 PARAM_KEYS = ("means3D", "rgb_colors", "unnorm_rotations", "logit_opacities", "log_scales")
+BA_RECORDS_PER_RANK = 8         # keyframes one rank may step with do_ba in a sharded mapping iteration (its record table)
 
 
 class FusedRenderer:
@@ -347,6 +349,46 @@ def retie_dev(means3D, old_q, old_t, cam_q, cam_t):
     return means3D
 
 
+def ba_record_table(keyframes, num_gaussians):
+    """This rank's record table of a keyframe-sharded bundle-adjustment iteration (`vtgs_retie_records`, include/vtgs.h),
+    on the host: [BA_RECORDS_PER_RANK, BA_RECORD_WORDS] int32 with one record per keyframe in list order -- valid = 1, the
+    keyframe's "id", its `retie_last` -- and the pose words and the unused slots zero.  Raises ValueError when a keyframe
+    has no integer "id", two keyframes share one, there are more keyframes than records or `retie_last` is not in 0..N."""
+    if len(keyframes) > BA_RECORDS_PER_RANK:
+        raise ValueError(f"do_ba under keyframe sharding steps at most {BA_RECORDS_PER_RANK} keyframes per rank and iteration, "
+                         f"got {len(keyframes)}")
+    table = torch.zeros((BA_RECORDS_PER_RANK, _lib.BA_RECORD_WORDS), dtype=torch.int32)
+    ids = set()
+    for s, kf in enumerate(keyframes):
+        try:
+            k = operator.index(kf["id"])
+        except (KeyError, TypeError):
+            raise ValueError("do_ba under keyframe sharding needs an integer 'id' on every keyframe") from None
+        if not -2 ** 31 <= k < 2 ** 31 or k in ids:
+            raise ValueError(f"keyframe id {k} is repeated or does not fit 32 bits")
+        ids.add(k)
+        n_last = int(kf.get("retie_last", 0))
+        if not 0 <= n_last <= num_gaussians:
+            raise ValueError(f"retie_last = {n_last} of keyframe {k} is not in 0..{num_gaussians}")
+        table[s, 0], table[s, 1], table[s, 2] = 1, k, n_last
+    return table
+
+
+def decode_ba_poses(tables):
+    """{id: (cam_q[4], cam_t[3])}: the stepped poses of the valid records of host tables [..., BA_RECORD_WORDS] int32.
+    Raises ValueError when an id appears twice."""
+    words = tables.reshape(-1, _lib.BA_RECORD_WORDS)
+    floats = words.view(torch.float32)
+    poses = {}
+    for rec, f in zip(words.tolist(), floats):
+        if rec[0] == 0:
+            continue
+        if rec[1] in poses:
+            raise ValueError(f"keyframe id {rec[1]} appears in two bundle-adjustment records")
+        poses[rec[1]] = (f[11:15].clone(), f[15:18].clone())
+    return poses
+
+
 class TrackingSolver:
     """The reference's per-frame tracking loop (src/vtgaussian_slam.py:1794-1970) for one frame:
     num_iters x (get_loss(tracking=True) -> backward -> Adam on the 7 pose numbers), keeping
@@ -539,7 +581,12 @@ class MappingSolver:
         The frozen rows get no update (their `fixed_lrs` are 0, configs/replica/room0.py:108-116).
     do_ba (per iteration): the keyframes' poses get gradients and an Adam step of their own (`do_ba`, :2545-2548; LRs
         `cam_unnorm_rots` / `cam_trans` of `lrs`); a keyframe carrying `retie_last=n` has the newest n Gaussians re-tied
-        to its pose after the step (:2706-2727)."""
+        to its pose after the step (:2706-2727).
+    do_ba with a process group: every keyframe needs an "id", an int unique across the ranks (e.g. its frame index); a
+        rank steps at most BA_RECORDS_PER_RANK keyframes per iteration.  The owner of a keyframe steps its pose and writes
+        a record (id, retie_last, old and new pose); the ranks exchange the records after the parameter step and every
+        rank applies every re-tie, in (rank, keyframe) order, to its replica of means3D, so the replicas stay bitwise
+        equal.  `ba_poses()` returns the poses all ranks stepped in the last such iteration."""
 
     def __init__(self, settings, params, device="cuda:0", lrs=None, eps=1e-15, pair_capacity=None, process_group=None,
                  global_params=None, poll_every=16, deterministic=None, sharded_step="auto"):
@@ -580,6 +627,8 @@ class MappingSolver:
                 self.sharded, self.sharded_error = None, repr(e)[:300]
         self.poll_every = int(poll_every)
         self._iters = 0
+        self._ba_iters = 0                  # keyframe-sharded do_ba iterations: their parity picks the fused step's record table
+        self._ba_mine = self._ba_tables = None
         self.gparams = self.r_global = self.ggrads = None
         if global_params is not None:
             self.set_global(global_params)
@@ -599,7 +648,8 @@ class MappingSolver:
             raise RuntimeError("vtgs_sharded_adam supports up to 8 ranks")
         n = sum(sizes.values())
         n_pad = (n + 3) // 4 * 4
-        block = symm.empty(2 * n_pad + 4, dtype=torch.float32, device=self.device)
+        tab = BA_RECORDS_PER_RANK * _lib.BA_RECORD_WORDS
+        block = symm.empty(2 * n_pad + 4 + 2 * tab, dtype=torch.float32, device=self.device)
         hdl = symm.rendezvous(block, self.pg)
         block.zero_()
         pflat, gflat = block[:n_pad], block[n_pad:2 * n_pad]
@@ -623,7 +673,12 @@ class MappingSolver:
             bases=(C.c_uint64 * world)(*[int(p_) for p_ in hdl.buffer_ptrs]),
             seg_end=(C.c_int64 * nseg)(*seg_end), lr=(C.c_float * nseg)(*[float(self.lrs[k]) for k in sizes]),
             m=torch.zeros(per, dtype=torch.float32, device=self.device), v=torch.zeros(per, dtype=torch.float32, device=self.device),
-            loss=torch.zeros(1, dtype=torch.float32, device=self.device))
+            loss=torch.zeros(1, dtype=torch.float32, device=self.device),
+            # the bundle-adjustment record tables, double-buffered by the parity of the do_ba iteration.  A rank writes its
+            # table before the step's first barrier and the peers read it after the second, with nothing ordering those
+            # reads against the rank's next write; with two tables that write goes to the other one, and the write after
+            # it comes behind the next step's barriers, which no peer reaches before its re-tie from this table is done
+            ba=block[2 * n_pad + 4:].view(torch.int32).view(2, BA_RECORDS_PER_RANK, _lib.BA_RECORD_WORDS))
         self.m = self.v = None                          # the moments are sharded: this rank keeps its slice only
         torch.cuda.synchronize(self.device)
         hdl.barrier(channel=0)
@@ -637,6 +692,57 @@ class MappingSolver:
                                                     float(self.eps), _ptr(self.step_dev), _ptr(sh["loss"]),
                                                     _stream_ptr(self.device)))
         sh["hdl"].barrier(channel=0)                    # every rank's new parameters have landed
+
+    def _ba_step(self, keyframes, header):
+        """Keyframe sharding, do_ba: the pose Adam steps of this rank's keyframes, each recorded (old and new pose) in this
+        rank's table -> that table on the device."""
+        if self.sharded is not None:
+            table = self.sharded["ba"][self._ba_iters % 2]
+        else:
+            if self._ba_mine is None:
+                self._ba_mine = torch.empty(header.shape, dtype=torch.int32, device=self.device)
+            table = self._ba_mine
+        table.copy_(header, non_blocking=True)
+        poses = table.view(torch.float32)
+        for s, kf in enumerate(keyframes):
+            st = kf["_ba"]
+            poses[s, 4:8].copy_(kf["cam_q"])
+            poses[s, 8:11].copy_(kf["cam_t"])
+            st["step"].add_(1)
+            if self.pose_lrs[0] != 0.0:
+                adam_step(kf["cam_q"], st["d_q"], st["m_q"], st["v_q"], self.pose_lrs[0], step_dev=st["step"], eps=self.eps)
+            if self.pose_lrs[1] != 0.0:
+                adam_step(kf["cam_t"], st["d_t"], st["m_t"], st["v_t"], self.pose_lrs[1], step_dev=st["step"], eps=self.eps)
+            poses[s, 11:15].copy_(kf["cam_q"])
+            poses[s, 15:18].copy_(kf["cam_t"])
+        return table
+
+    def _ba_retie(self, table):
+        """Keyframe sharding, do_ba, after the parameter step: every rank's records reach every rank -- read from the peers'
+        symmetric blocks (fused step) or one all-gather -- and `vtgs_retie_records` applies all their re-ties to this
+        rank's means3D in (rank, slot) order, leaving the gathered tables in `_ba_tables`."""
+        world = torch.distributed.get_world_size(self.pg)
+        if self._ba_tables is None:
+            self._ba_tables = torch.empty((world,) + tuple(table.shape), dtype=torch.int32, device=self.device)
+        if self.sharded is not None:
+            off = table.data_ptr() - self.sharded["block"].data_ptr()           # the same offset in every rank's block
+            bases, out = (C.c_uint64 * world)(*[b + off for b in self.sharded["bases"]]), self._ba_tables
+        else:
+            torch.distributed.all_gather_into_tensor(self._ba_tables.view(-1, table.shape[1]), table, group=self.pg)
+            bases, out = (C.c_uint64 * world)(*[self._ba_tables[r].data_ptr() for r in range(world)]), None
+        means3D = self.params["means3D"]
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().vtgs_retie_records(world, bases, table.shape[0], _ptr(means3D), means3D.shape[0], _ptr(out),
+                                                     _stream_ptr(self.device)))
+        self._ba_iters += 1
+
+    def ba_poses(self):
+        """{id: (cam_q[4], cam_t[3])} on the host: the pose every rank's keyframe got in the last bundle-adjustment iteration
+        under keyframe sharding, from this rank's gathered tables (one blocking read).  Raises ValueError if an id appears
+        twice among the ranks."""
+        if self._ba_tables is None:
+            raise RuntimeError("ba_poses: no do_ba iteration has run under a process group")
+        return decode_ba_poses(self._ba_tables.cpu())
 
     def set_global(self, global_params):
         gp = {k: global_params[k].detach().to(self.device).float().contiguous() for k in PARAM_KEYS}
@@ -692,14 +798,20 @@ class MappingSolver:
                 g.zero_()
 
     def iteration(self, keyframes, loss_fn=None, w_im=1.0, w_depth=1.0, do_ba=False):
-        """keyframes: list of dict(cam_q, cam_t, gt_rgb, gt_depth[, global=True][, retie_last=n]) owned by THIS rank.
-        loss_fn=None uses the fused mapping loss kernels (FusedRenderer.mapping_loss)."""
+        """keyframes: list of dict(cam_q, cam_t, gt_rgb, gt_depth[, global=True][, retie_last=n][, id]) owned by THIS rank
+        ("id" is required with do_ba and a process group).  loss_fn=None uses the fused mapping loss kernels
+        (FusedRenderer.mapping_loss)."""
+        # (a sharded do_ba iteration's keyframes are checked before anything is updated)
+        ba_header = ba_record_table(keyframes, self.params["means3D"].shape[0]) if do_ba and self.pg is not None else None
         poll = self.poll_every > 0 and self._iters % self.poll_every == 0
         # the overflow check (one blocking read every `poll_every` iterations) comes before anything is updated
         run_fitting(lambda: self._gradients(keyframes, loss_fn, w_im, w_depth, do_ba),
                     [self.r] if self.r_global is None else [self.r, self.r_global], poll=poll)
         self._iters += 1
         self.step_dev.add_(1)
+        # keyframe sharding: the pose steps come before the parameter step (they touch disjoint tensors), so that the fused
+        # step's barriers publish the records
+        ba_table = self._ba_step(keyframes, ba_header) if ba_header is not None else None
         if self.sharded is not None:
             self._sharded_step()
         else:
@@ -708,13 +820,12 @@ class MappingSolver:
                 torch.distributed.all_reduce(self.flat, group=self.pg)
             for k, lr in self.lrs.items():
                 adam_step(self.params[k], self.grads[k], self.m[k], self.v[k], lr, step_dev=self.step_dev, eps=self.eps)
-        if do_ba:
+        if ba_table is not None:
+            self._ba_retie(ba_table)
+        elif do_ba:
             for kf in keyframes:
                 st = kf["_ba"]
                 n_last = int(kf.get("retie_last", 0))
-                if n_last > 0 and self.pg is not None:
-                    raise NotImplementedError("retie_last under keyframe sharding: the re-tied keyframe's pose lives on its "
-                                              "owner rank only; replicate that keyframe on every rank or broadcast its pose")
                 if n_last > 0:
                     st["old_q"].copy_(kf["cam_q"])
                     st["old_t"].copy_(kf["cam_t"])
