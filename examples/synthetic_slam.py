@@ -2,6 +2,9 @@
 
 Synthetic (BASELINE config 4: TUM fr1_desk-shaped 640x480 tracking + mapping over synthetic frames):
     python examples/synthetic_slam.py --shape tum_fr1 --frames 600 --track-iters 200 --map-iters 30 --baseframe-every 30
+Add `--align-sections 2` to bundle-adjust every base frame against the two sections it was tracked against (with
+`--track-sections 2`; one otherwise): the JSON line then lists each base frame's correction.  At the default
+`--align-lr-*` (the tracking rates) this currently raises the ATE (see slam_loop.LoopConfig.align_sections).
 On-disk sequences in the reference's layouts (camera parameters from the reference's configs/data/*.yaml):
     python examples/synthetic_slam.py --source replica --basedir data/Replica --sequence room0 --camera-yaml configs/data/replica.yaml
     python examples/synthetic_slam.py --source tum --basedir data/TUM_RGBD --sequence rgbd_dataset_freiburg1_desk \
@@ -37,6 +40,11 @@ def main():
     ap.add_argument("--step-deg", type=float, default=0.3)
     ap.add_argument("--track-sections", type=int, default=1, help="track against the newest k sections")
     ap.add_argument("--no-graph", action="store_true")
+    ap.add_argument("--align-sections", type=int, default=0,
+                    help="bundle-adjust each base frame against the last N sections it was tracked against (0: off)")
+    # the tracking rates: the reference's own mapping pose LRs (1e-8 / 1e-7) leave the pose where it is
+    ap.add_argument("--align-lr-rot", type=float, default=4e-4, help="mapping LR of cam_unnorm_rots with --align-sections")
+    ap.add_argument("--align-lr-trans", type=float, default=2e-3, help="mapping LR of cam_trans with --align-sections")
     a = ap.parse_args()
 
     import torch
@@ -60,7 +68,10 @@ def main():
     W, H, K = src.W, src.H, src.K.astype(np.float64)
     poses = src.c2w.numpy().astype(np.float64)
     cfg = LoopConfig(track_iters=a.track_iters, map_iters=a.map_iters, baseframe_every=a.baseframe_every,
-                     map_every=a.map_every, use_graph=not a.no_graph, track_sections=a.track_sections)
+                     map_every=a.map_every, use_graph=not a.no_graph, track_sections=a.track_sections,
+                     align_sections=a.align_sections)
+    if a.align_sections > 0:
+        cfg.map_lrs = dict(cfg.map_lrs, cam_unnorm_rots=a.align_lr_rot, cam_trans=a.align_lr_trans)
     slam = ViewTiedSLAM(W, H, K, cfg)
     t0 = time.perf_counter()
     gen = 0.0                                                       # decoding runs on the prefetch thread
@@ -78,6 +89,8 @@ def main():
         ate_mean_after_alignment_m=ate_after_alignment(list(poses), list(est)),        # the reference's evaluate_ate
         track_iters=st["track_iters"], track_iters_per_s=st["track_iters"] / max(st["track_s"], 1e-9),
         map_keyframe_iters=st["map_iters"], map_keyframe_iters_per_s=st["map_iters"] / max(st["map_s"], 1e-9),
+        align_sections=a.align_sections, align_share_of_map_s=st["align_s"] / max(st["map_s"], 1e-9),
+        align_corrections=[dict(frame=i, frozen=f, shift_m=dt, angle_deg=da) for i, f, dt, da in st["align"]],
         frames_per_s=n / wall, wall_s=wall)))
 
 

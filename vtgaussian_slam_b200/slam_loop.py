@@ -15,10 +15,16 @@ What it mirrors of the reference's `rgbd_slam` (src/vtgaussian_slam.py:1574-2876
   * section choice at a section's base frame (:1526-1553, :1891-1970; LoopConfig.section_selection = "overlap"): the
     earliest sections that still overlap the new frame (keyframes.keyframe_selection_overlap_visbased_earliest_dynamic_
     new_topkbase) are rendered together with the newest one, candidates ranked by the device point-to-plane metric;
+  * section-start mapping (:2530-2552, :2706-2727; LoopConfig.align_sections = k > 0): at every base frame but frame 0
+    the first mapping call maps the base keyframe alone with bundle adjustment (do_ba, pose LRs from map_lrs) and the
+    frozen-section term `loss_global` over the last k sections the frame was tracked against, re-tying the new section
+    to the stepped pose after every step; the stepped pose replaces the frame's estimate.  The section's later mapping
+    calls run without either, as the reference's do away from section starts;
   * silhouette-driven Gaussian addition (:732-813): add_missing_gaussians.
   Left out (not on the hot path, SURVEY.md 8 "out of scope" / later rows): edge-mask densification on the 2x grid inside
-  the loop (densified_section builds such a section), the frozen-section loss inside the loop (MappingSolver has it),
-  checkpoints.
+  the loop (densified_section builds such a section), Gaussian addition inside `process`, checkpoints.  The loop runs
+  on one GPU: keyframe-sharded mapping with `MappingSolver.ba_poses()` keeping one trajectory on every rank is not wired
+  into it.
 
 Everything on the device runs through the CUDA library; there is no CPU fallback.
 """
@@ -66,6 +72,26 @@ class LoopConfig:
     base_metric: str = "loss"             # "p2p": rank the base frame's candidate poses by the point-to-plane distance
                                           # to the earliest overlapping section's base frame (reference choose_metric)
     p2p_method: str = "sum"
+    # -- section-start mapping with bundle adjustment (reference :2530-2552, :2706-2727; SURVEY.md 3.3) --
+    align_sections: int = 0               # k > 0: at every base frame but frame 0 the first mapping call steps the base pose
+                                          # (do_ba, LRs map_lrs["cam_unnorm_rots"] / ["cam_trans"]) against the frozen
+                                          # earlier sections -- the last k of those it was tracked against -- plus the new
+                                          # one, re-tying the new section to the stepped pose after every step.  The
+                                          # reference's own mapping pose LRs (1e-8 / 1e-7, room0.py:99-107) make that step
+                                          # negligible; whether alignment helps at those rates is not measured.  At the
+                                          # tracking rates (4e-4 / 2e-3) it currently HURTS (measured on a B200): the own
+                                          # term's pose gradient is not zero at the tied pose and the re-tie keeps it so,
+                                          # so Adam walks the pose ~one LR per step in a fixed direction (tests/
+                                          # test_gpu_slam_align.py: a 1 cm base error grows to ~35 mm)
+
+
+def base_frame_sections(k, track_sections, align_sections, selected=None):
+    """Section k's base frame -> (the sections it was tracked against, the frozen sections its section-start mapping
+    aligns it to).  Tracked against: `selected` (section_selection "overlap": the choice of `_track_base_frame`), else
+    the newest `track_sections` sections before k (the tracker's consecutive rows).  Frozen: the last `align_sections`
+    of those, none when 0."""
+    tracked = sorted(selected) if selected is not None else list(range(max(0, k - max(1, track_sections)), k))
+    return tracked, tracked[max(0, len(tracked) - align_sections):] if align_sections > 0 else []
 
 
 def quat_from_matrix(R):
@@ -242,6 +268,11 @@ class ViewTiedSLAM:
     def __init__(self, W, H, K, cfg: LoopConfig | None = None, device="cuda:0"):
         self.W, self.H, self.K = int(W), int(H), np.asarray(K, np.float64)
         self.cfg = cfg or LoopConfig()
+        if self.cfg.align_sections < 0:
+            raise ValueError(f"align_sections must be >= 0, got {self.cfg.align_sections}")
+        if self.cfg.align_sections > 0 and not (self.cfg.map_lrs.get("cam_unnorm_rots") or self.cfg.map_lrs.get("cam_trans")):
+            raise ValueError("align_sections > 0 steps the base pose with the mapping LRs map_lrs['cam_unnorm_rots'] / "
+                             "map_lrs['cam_trans']; with both missing or zero the alignment would do nothing")
         self.device = torch.device(device)
         s = synthetic.setup_camera(self.W, self.H, self.K, np.eye(4))
         t = lambda a: torch.as_tensor(a, dtype=torch.float32, device=self.device)
@@ -250,7 +281,8 @@ class ViewTiedSLAM:
             bg=t(s["bg"]), scale_modifier=s["scale_modifier"], viewmatrix=t(s["viewmatrix"]), projmatrix=t(s["projmatrix"]),
             sh_degree=0, campos=t(s["campos"]), prefiltered=False)
         self.w2c = []                      # estimated poses, one 4x4 per frame
-        self.sections = []                 # dict(params (arena views), index, base, keyframes=[(idx, rgb, depth)])
+        self.sections = []                 # dict(params (arena views), index, base, keyframes=[(idx, rgb, depth)],
+                                           #      tracked_against, frozen: base_frame_sections of its base frame)
         self.store = None                  # SectionStore, created with the first section
         self.tracker = None
         self.mapper = None
@@ -258,7 +290,9 @@ class ViewTiedSLAM:
             raise ValueError("overlap-driven section choice needs baseframe_every to be a multiple of overlap_every")
         self.keyframe_list = []            # every `overlap_every` frames: dict(id, est_w2c, depth) for the section choice
         self.section_choices = []          # per base frame: the sections it was tracked against
-        self.stats = dict(track_iters=0, map_iters=0, track_s=0.0, map_s=0.0, track_loss=[])
+        # align: per aligned base frame (idx, frozen sections, |camera centre shift| m, |rotation change| deg); align_s is
+        # the part of map_s spent in section-start mapping with bundle adjustment
+        self.stats = dict(track_iters=0, map_iters=0, track_s=0.0, map_s=0.0, track_loss=[], align=[], align_s=0.0)
 
     # -- sections -------------------------------------------------------------------------------------------
     def _new_section(self, idx, rgb, depth):
@@ -267,15 +301,19 @@ class ViewTiedSLAM:
         if self.store is None:
             self.store = SectionStore(4 * fresh["means3D"].shape[0], self.device)
         k = self.store.append(fresh)
-        sec = dict(params=self.store.rows(k), index=k, base=idx, keyframes=[])
+        c = self.cfg
+        choice = self.section_choices[-1][1] if self.section_choices and self.section_choices[-1][0] == idx else None
+        tracked, frozen = base_frame_sections(k, c.track_sections, c.align_sections, choice)
+        sec = dict(params=self.store.rows(k), index=k, base=idx, keyframes=[], tracked_against=tracked, frozen=frozen)
         self.sections.append(sec)
         for s_ in self.sections:                         # the arena may have moved: refresh every view
             s_["params"] = self.store.rows(s_["index"])
-        c = self.cfg
         # the solvers alias the arena rows (contiguous float32 CUDA row slices are used in place): mapping updates the
         # newest section where it lives, and the tracker -- over the newest `track_sections` consecutive sections --
-        # sees them without a copy
-        self.mapper = MappingSolver(self.settings, sec["params"], device=self.device, lrs=c.map_lrs)
+        # sees them without a copy, re-tied rows included.  The frozen-section term renders frozen + new rows: views of
+        # the arena when they are consecutive, otherwise one gathered copy whose new rows the mapper refreshes
+        gp = self.store.gather(frozen + [k]) if frozen else None
+        self.mapper = MappingSolver(self.settings, sec["params"], device=self.device, lrs=c.map_lrs, global_params=gp)
         first = max(0, k - max(1, c.track_sections) + 1)
         self.tracker = TrackingSolver(self.settings, self.store.rows(first, k), device=self.device, lr_rot=c.lr_rot,
                                       lr_trans=c.lr_trans, w_im=c.track_w_im, w_depth=c.track_w_depth,
@@ -322,15 +360,39 @@ class ViewTiedSLAM:
         chosen = [sec["keyframes"][0]] + sec["keyframes"][1:][-(c.keyframes_per_map - 1):] if c.keyframes_per_map > 1 else sec["keyframes"][-1:]
         for idx, rgb, depth in chosen:
             M = self.w2c[idx]
-            kfs.append(dict(cam_q=torch.as_tensor(quat_from_matrix(M[:3, :3]), dtype=torch.float32, device=self.device),
-                            cam_t=torch.as_tensor(M[:3, 3], dtype=torch.float32, device=self.device),
-                            gt_rgb=rgb, gt_depth=depth))
+            kfs.append({"cam_q": torch.as_tensor(quat_from_matrix(M[:3, :3]), dtype=torch.float32, device=self.device),
+                        "cam_t": torch.as_tensor(M[:3, 3], dtype=torch.float32, device=self.device),
+                        "gt_rgb": rgb, "gt_depth": depth, "global": False})
+        # the section start (its base keyframe alone) with frozen sections: bundle adjustment of the base pose against
+        # them, the whole section re-tied to the stepped pose after every step (reference :2530-2552, :2706-2727)
+        align = bool(sec["frozen"]) and len(sec["keyframes"]) == 1
+        if align:
+            kfs[0].update({"global": True, "retie_last": int(sec["params"]["means3D"].shape[0]), "id": sec["base"]})
         t0 = time.perf_counter()
         for _ in range(c.map_iters):
-            self.mapper.iteration(kfs, w_im=c.map_w_im, w_depth=c.map_w_depth)
+            self.mapper.iteration(kfs, w_im=c.map_w_im, w_depth=c.map_w_depth, do_ba=align)
+        if align:
+            self._adopt_aligned_pose(sec, kfs[0])
         torch.cuda.synchronize(self.device)
-        self.stats["map_s"] += time.perf_counter() - t0
+        dt = time.perf_counter() - t0
+        self.stats["map_s"] += dt
         self.stats["map_iters"] += c.map_iters * len(kfs)
+        if align:
+            self.stats["align_s"] += dt
+
+    def _adopt_aligned_pose(self, sec, kf):
+        """The base pose stepped by the section-start mapping (one blocking read) becomes the frame's estimate: for the
+        constant-velocity propagation, the export and, through `keyframe_list`, the overlap choice and the p2p anchor."""
+        idx = sec["base"]
+        pose = torch.cat((kf["cam_q"], kf["cam_t"])).cpu().numpy()
+        old, new = self.w2c[idx], matrix_from_quat(pose[:4], pose[4:])
+        self.w2c[idx] = new
+        for e in self.keyframe_list:
+            if e["id"] == idx:
+                e["est_w2c"] = torch.as_tensor(new, dtype=torch.float32, device=self.device)
+        shift = float(np.linalg.norm(np.linalg.inv(new)[:3, 3] - np.linalg.inv(old)[:3, 3]))
+        cos = (np.trace(new[:3, :3] @ old[:3, :3].T) - 1.0) / 2.0
+        self.stats["align"].append((idx, list(sec["frozen"]), shift, float(np.degrees(np.arccos(np.clip(cos, -1.0, 1.0))))))
 
     # -- tracking -------------------------------------------------------------------------------------------
     def _track(self, idx, rgb, depth):
