@@ -23,6 +23,9 @@ E = matrix_from_quat([np.cos(np.radians(0.25)), 0.0, np.sin(np.radians(0.25)), 0
 # zero at the pose the section is tied to, and re-tying the section after every step keeps it so: Adam walks the pose
 # about one LR per step in a fixed direction (the own term alone, re-tied, drifts ~40 mm in 20 steps; not re-tied, a few
 # mm), and the frozen-section term does not hold it back.
+# That gradient is a property of the method, not a kernel error: test_gpu_mapping_reference.py::
+# test_own_term_pose_gradient_at_the_tied_pose_matches_fp64 finds the kernels' own-term pose gradient at the tied pose equal
+# to fp64 autograd through the reference's chain (to 5e-5), and far from zero (|dL/dt| = 0.89 on a 100x70 section).
 RUNAWAY = "section-start BA with re-tie drifts under the own term's pose gradient at the tracking LRs"
 
 

@@ -272,15 +272,19 @@ def _torch_inputs(sc, dtype=torch.float64):
     return t
 
 
-@pytest.mark.parametrize("seed,aniso,bg", [(3, True, (0, 0, 0)), (4, False, (0.3, 0.1, 0.6)), (11, True, (0, 0, 0))])
-def test_forward_and_backward_match_autograd(seed, aniso, bg):
+@pytest.mark.parametrize("seed,aniso,bg,tiled", [pytest.param(3, True, (0, 0, 0), False, id="3-True-bg0"),
+                                                 pytest.param(4, False, (0.3, 0.1, 0.6), False, id="4-False-bg1"),
+                                                 pytest.param(11, True, (0, 0, 0), False, id="11-True-bg2"),
+                                                 pytest.param(4, False, (0.3, 0.1, 0.6), True, id="4-False-bg1-tiled")])
+def test_forward_and_backward_match_autograd(seed, aniso, bg, tiled):
+    """tiled: torch_ref's tile-by-tile evaluation, which must also equal its dense form to fp64 rounding."""
     W, H = 48, 40
     K, sc = synthetic.random_scene(160, W, H, seed=seed, anisotropic=aniso, scale_px=(0.7, 5.0))
     cam, s = oracle_camera(W, H, K, bg=bg)
     o, out = _run(cam, sc)
     t = _torch_inputs(sc)
     ref = torch_ref.render(cam_dict(s), t["means3D"], t["scales"], t["rotations"], t["opacities"], t["colors"],
-                           out["rects"], means2D=t["means2D"])
+                           out["rects"], means2D=t["means2D"], tiled=tiled)
     assert np.array_equal(ref["n_contrib"].numpy(), out["n_contrib"])
     np.testing.assert_allclose(out["color"], ref["color"].detach().numpy(), atol=2e-5)
     np.testing.assert_allclose(out["depth"], ref["depth"].detach().numpy(), atol=5e-5)
@@ -298,6 +302,16 @@ def test_forward_and_backward_match_autograd(seed, aniso, bg):
         want = t[key].grad.numpy()
         got = g[name]
         assert rel_err(got, want) < 1e-3, (name, rel_err(got, want))
+    if tiled:
+        td = _torch_inputs(sc)
+        dense = torch_ref.render(cam_dict(s), td["means3D"], td["scales"], td["rotations"], td["opacities"], td["colors"],
+                                 out["rects"], means2D=td["means2D"])
+        assert torch.equal(dense["n_contrib"], ref["n_contrib"])
+        for k in ("color", "depth", "final_T"):
+            assert rel_err(ref[k].detach().numpy(), dense[k].detach().numpy()) <= 1e-12, k
+        (dense["color"] * torch.tensor(dL, dtype=torch.float64)).sum().backward()
+        for k in td:
+            assert rel_err(t[k].grad.numpy(), td[k].grad.numpy(), floor=1e-300) <= 1e-12, k
 
 
 def test_view_tied_frame_statistics():
