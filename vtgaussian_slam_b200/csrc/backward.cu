@@ -102,7 +102,8 @@ dpix_max_kernel(const float* __restrict__ dL_dpix, size_t P, size_t begin, size_
 
 static int launch_dpix_max(const CamConst& cam, const float* dL_dpix, int nch, uint32_t* out_bits, cudaStream_t stream) {
     const size_t P = (size_t)cam.W * cam.H;
-    const size_t begin = (size_t)cam.row0 * 16 * cam.W, end = std::min(P, (size_t)cam.row1 * 16 * cam.W);
+    size_t begin, end;
+    band_pixel_range(cam, begin, end);
     if (end <= begin) return VTGS_OK;
     const int blocks = (int)std::min<size_t>((end - begin + 1023) / 1024, 148 * 8);
     return launch_k("dpix_max_kernel", Launch::pdl, dpix_max_kernel, dim3(blocks), dim3(256), 0, stream, dL_dpix, P, begin, end, nch, out_bits);
@@ -623,29 +624,14 @@ int launch_pose_matrix(const VtgsPose* pose, VtgsCounters* counters, cudaStream_
 
 constexpr int POSE_TERMS = 12;       // sum g (3) and sum g p^T (9)
 
-// Deterministic final reduction of the block partials (fixed slice order, fp64) and the chain
-// dL/dR, dL/dt -> cam_unnorm_rot, cam_trans through build_rotation and the two normalisations.
-// Executed by the K7' block that finishes last (256 threads): no extra launch.
-__device__ __forceinline__ void pose_finalize_block(const float* __restrict__ partials, int nblocks,
-                                                    const VtgsCounters* __restrict__ c, float* __restrict__ d_rot,
-                                                    float* __restrict__ d_trans, int accumulate, double (*s_sum)[21],
+// The chain dL/dR, dL/dt -> cam_unnorm_rot, cam_trans through build_rotation and the two normalisations, from the
+// pose sums over the grid.  Executed by the K7' block that finishes last: no extra launch.
+__device__ __forceinline__ void pose_finalize_block(const LastBlockSum<POSE_TERMS>& red, const VtgsCounters* __restrict__ c,
+                                                    float* __restrict__ d_rot, float* __restrict__ d_trans, int accumulate,
                                                     const float* __restrict__ out_scale) {
-    constexpr int SLICES = 21;                    // 12 terms x 21 slices = 252 threads, coalesced reads
-    const int tid = threadIdx.x;
-    if (tid < POSE_TERMS * SLICES) {
-        const int term = tid % POSE_TERMS, sl = tid / POSE_TERMS;
-        double acc = 0.0;
-        for (int b = sl; b < nblocks; b += SLICES) acc += (double)__ldcg(&partials[(size_t)b * POSE_TERMS + term]);
-        s_sum[term][sl] = acc;
-    }
-    __syncthreads();
-    if (tid == 0) {
+    if (threadIdx.x == 0) {
         double tot[POSE_TERMS];
-        for (int k = 0; k < POSE_TERMS; ++k) {
-            double a = 0.0;
-            for (int l = 0; l < SLICES; ++l) a += s_sum[k][l];
-            tot[k] = a;
-        }
+        for (int k = 0; k < POSE_TERMS; ++k) tot[k] = red.total(k);
         // D[r][k] = dL/dR[r][k] = sum g_r p_k
         const double D[3][3] = {{tot[3], tot[4], tot[5]}, {tot[6], tot[7], tot[8]}, {tot[9], tot[10], tot[11]}};
         const double n1 = c->pose_qnorm[0], n2 = c->pose_qnorm[1];
@@ -722,9 +708,7 @@ fused_preprocess_backward_kernel(const __grid_constant__ CamConst cam, int64_t N
                                  const uint32_t* __restrict__ tiles_touched, const uint8_t* __restrict__ band_flags,
                                  const uint32_t* __restrict__ cand, const uint32_t* __restrict__ n_cand) {
     VTGS_PDL_PROLOGUE();
-    __shared__ float s_part[8][POSE_TERMS];
-    __shared__ double s_sum[POSE_TERMS][21];
-    __shared__ bool s_last;
+    __shared__ LastBlockSum<POSE_TERMS> red;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int64_t stride = (int64_t)gridDim.x * 256;
     const bool rot_aligned = (reinterpret_cast<uintptr_t>(prm.unnorm_rotations) & 15) == 0;
@@ -837,22 +821,9 @@ fused_preprocess_backward_kernel(const __grid_constant__ CamConst cam, int64_t N
     }
     if (!want_pose) return;
     const float tot = warp_transpose_reduce<POSE_TERMS>(pose_v, lane);
-    if ((lane & 1) == 0 && (lane >> 1) < POSE_TERMS) s_part[warp][lane >> 1] = tot;
-    __syncthreads();
-    if (tid < POSE_TERMS) {
-        float s = 0.0f;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) s += s_part[w][tid];
-        out.pose_scratch[(size_t)blockIdx.x * POSE_TERMS + tid] = s;
-        __threadfence();
-    }
-    __syncthreads();
-    if (tid == 0) s_last = atomicAdd(ticket, 1u) == gridDim.x - 1;
-    __syncthreads();
-    if (!s_last) return;
-    __threadfence();
-    pose_finalize_block(out.pose_scratch, (int)gridDim.x, counters, out.cam_unnorm_rot, out.cam_trans, accumulate, s_sum, out.pose_scale);
-    if (tid == 0) *ticket = 0u;
+    if ((lane & 1) == 0 && (lane >> 1) < POSE_TERMS) red.part[warp][lane >> 1] = tot;
+    if (!red.reduce(out.pose_scratch, ticket)) return;
+    pose_finalize_block(red, counters, out.cam_unnorm_rot, out.cam_trans, accumulate, out.pose_scale);
 }
 
 }  // namespace vtgs

@@ -9,7 +9,7 @@ namespace vtgs {
 
 // =============================== evaluation metrics ==========================================
 // One pass over the frame: per-channel squared error of the weighted images, masked depth L1, valid count; the last
-// block reduces the per-block partials in a fixed order (fp64) and derives PSNR / depth L1.
+// block derives PSNR / depth L1 from the sums over the frame.
 constexpr int EVAL_BLOCKS = 592;          // 4 blocks per SM
 constexpr int EVAL_TERMS = 8;             // 5 used
 
@@ -17,9 +17,7 @@ __global__ void __launch_bounds__(256)
 eval_metrics_kernel(size_t P, const float* __restrict__ image6, const float* __restrict__ gt_rgb, const float* __restrict__ gt_depth,
                     float sil_thres, int use_presence, float* __restrict__ partials, unsigned int* __restrict__ ticket,
                     float* __restrict__ out8) {
-    __shared__ float s_part[8][EVAL_TERMS];
-    __shared__ double s_sum[EVAL_TERMS][32];
-    __shared__ bool s_last;
+    __shared__ LastBlockSum<EVAL_TERMS> red;
     float acc[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
     for (size_t pid = (size_t)blockIdx.x * 256 + threadIdx.x; pid < P; pid += (size_t)gridDim.x * 256) {
         const float gd = __ldg(gt_depth + pid);
@@ -45,33 +43,12 @@ eval_metrics_kernel(size_t P, const float* __restrict__ image6, const float* __r
     for (int k = 0; k < 5; ++k) acc[k] = warp_sum(acc[k]);
     if (lane == 0) {
 #pragma unroll
-        for (int k = 0; k < EVAL_TERMS; ++k) s_part[warp][k] = k < 5 ? acc[k] : 0.0f;
+        for (int k = 0; k < EVAL_TERMS; ++k) red.part[warp][k] = k < 5 ? acc[k] : 0.0f;
     }
-    __syncthreads();
-    if (tid < EVAL_TERMS) {
-        float s = 0.f;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) s += s_part[w][tid];
-        partials[(size_t)blockIdx.x * EVAL_TERMS + tid] = s;
-        __threadfence();
-    }
-    __syncthreads();
-    if (tid == 0) s_last = atomicAdd(ticket, 1u) == gridDim.x - 1;
-    __syncthreads();
-    if (!s_last) return;
-    __threadfence();
-    const int term = tid & (EVAL_TERMS - 1), sl = tid >> 3;            // 32 slices of blocks
-    double a = 0.0;
-    for (int b = sl; b < (int)gridDim.x; b += 32) a += (double)__ldcg(&partials[(size_t)b * EVAL_TERMS + term]);
-    s_sum[term][sl] = a;
-    __syncthreads();
+    if (!red.reduce(partials, ticket)) return;
     if (tid == 0) {
         double tot[5];
-        for (int k = 0; k < 5; ++k) {
-            double t = 0.0;
-            for (int i = 0; i < 32; ++i) t += s_sum[k][i];
-            tot[k] = t;
-        }
+        for (int k = 0; k < 5; ++k) tot[k] = red.total(k);
         double psnr = 0.0;
         for (int c = 0; c < 3; ++c) {
             out8[c] = (float)tot[c];
@@ -82,7 +59,6 @@ eval_metrics_kernel(size_t P, const float* __restrict__ image6, const float* __r
         out8[5] = (float)(psnr / 3.0);
         out8[6] = (float)(tot[3] / tot[4]);                            // depth L1
         out8[7] = out8[6];                                             // the reference's "rmse": sqrt(x^2) = |x|, same sum
-        *ticket = 0u;
     }
 }
 

@@ -137,6 +137,15 @@ inline CamConst make_cam_const(const VtgsCamera& c) {
     return k;
 }
 
+// Pixels [b, e) of the camera's tile-row band, clamped to the frame (b <= e; the whole frame without a band).
+__host__ __device__ __forceinline__ void band_pixel_range(const CamConst& cam, size_t& b, size_t& e) {
+    const size_t P = (size_t)cam.W * cam.H;
+    b = (size_t)cam.row0 * 16 * cam.W;
+    e = (size_t)cam.row1 * 16 * cam.W;
+    if (e > P) e = P;
+    if (b > e) b = e;
+}
+
 // ---- spec'd elementary functions (device) -------------------------------------------------
 __device__ __forceinline__ float fmul(float a, float b) { return __fmul_rn(a, b); }
 __device__ __forceinline__ float fadd(float a, float b) { return __fadd_rn(a, b); }
@@ -347,5 +356,71 @@ __device__ __forceinline__ T warp_sum(T v) {
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(VTGS_FULL_MASK, v, o);
     return v;
 }
+
+// ---- fixed-order sum of T terms over the blocks of a grid -------------------------------------------------------------
+// Each block leaves one fp32 partial per term, its warps' values summed in warp order.  SLICES = THREADS / T threads
+// per term then form fp64 slice sums: slice s sums the blocks b = s (mod SLICES) in ascending order, and a term's total
+// sums its slices in ascending order.  The result is the same whatever order the blocks ran in.
+template <int T, int WARPS>
+__device__ __forceinline__ float warp_order_sum(const float (&part)[WARPS][T], int term) {
+    float s = 0.f;
+#pragma unroll
+    for (int w = 0; w < WARPS; ++w) s += part[w][term];
+    return s;
+}
+
+// SAME_GRID: the partials were written by other blocks of the running grid, so they are read from L2 (__ldcg), not
+// through this SM's L1; otherwise an earlier launch wrote them.
+template <int T, int THREADS, bool SAME_GRID = true>
+__device__ __forceinline__ void slice_sums(const float* partials, int nblocks, double (&slice)[T][THREADS / T]) {
+    constexpr int SLICES = THREADS / T;
+    const int tid = threadIdx.x;
+    if (tid < T * SLICES) {
+        const int term = tid % T, sl = tid / T;          // consecutive threads read consecutive partials
+        double acc = 0.0;
+        for (int b = sl; b < nblocks; b += SLICES) {
+            const float* p = &partials[(size_t)b * T + term];
+            acc += (double)(SAME_GRID ? __ldcg(p) : *p);
+        }
+        slice[term][sl] = acc;
+    }
+}
+
+template <int T, int SLICES>
+__device__ __forceinline__ double slices_total(const double (&slice)[T][SLICES], int term) {
+    double a = 0.0;
+    for (int s = 0; s < SLICES; ++s) a += slice[term][s];
+    return a;
+}
+
+// The same in one launch: the block whose ticket comes last sums every block's partials.  Declared __shared__ by the
+// kernel, which leaves each warp's values in part[warp][term] and calls reduce() with all its threads.  reduce()
+// returns true in the last block only, with the slice sums formed and the ticket (zero on entry) reset to zero;
+// total(term) is then the term's sum over the grid.
+template <int T, int THREADS = 256>
+struct LastBlockSum {
+    float part[THREADS / 32][T];
+    double slice[T][THREADS / T];
+    bool last;
+
+    __device__ __forceinline__ bool reduce(float* partials, unsigned int* ticket) {
+        const int tid = threadIdx.x;
+        __syncthreads();
+        if (tid < T) {
+            partials[(size_t)blockIdx.x * T + tid] = warp_order_sum(part, tid);
+            __threadfence();                             // the partial is visible before the ticket is taken
+        }
+        __syncthreads();
+        if (tid == 0) last = atomicAdd(ticket, 1u) == gridDim.x - 1;
+        __syncthreads();
+        if (!last) return false;
+        if (tid == 0) *ticket = 0u;                      // every block has taken its ticket
+        __threadfence();
+        slice_sums<T, THREADS>(partials, gridDim.x, slice);
+        __syncthreads();
+        return true;
+    }
+    __device__ __forceinline__ double total(int term) const { return slices_total(slice, term); }
+};
 
 }  // namespace vtgs

@@ -71,14 +71,6 @@ median_pick_kernel(unsigned long long P_total, int pass, unsigned int* __restric
     }
 }
 
-static inline void band_pixel_range(const CamConst& cam, size_t& b, size_t& e) {
-    const size_t P = (size_t)cam.W * cam.H;
-    b = (size_t)cam.row0 * 16 * cam.W;
-    e = (size_t)cam.row1 * 16 * cam.W;
-    if (e > P) e = P;
-    if (b > e) b = e;
-}
-
 static int launch_median_hist(const VtgsCamera* camera, const float* depth_plane, const float* gt_depth, int pass, uint32_t* state,
                               cudaStream_t stream) {
     const CamConst cam = make_cam_const(*camera);
@@ -95,20 +87,17 @@ static int launch_median_pick(int64_t P_total, int pass, uint32_t* state, cudaSt
 
 // ---- Replica iteration-0 silhouette-threshold search (reference src/vtgaussian_slam.py:472-510) --------------------
 // The five masks are nested (0.990 < 0.993 < ... < 0.999), so a pixel is binned by the number of thresholds its
-// silhouette exceeds and the per-threshold sums are suffix sums of the bins.  Per-block partials + a deterministic
-// (fixed slice order, fp64) final reduction by the block that finishes last.
+// silhouette exceeds and the per-threshold sums are suffix sums of the bins.
 constexpr int LADDER_N = 5;
 __device__ __constant__ float c_sil_ladder[LADDER_N] = {0.990f, 0.993f, 0.995f, 0.997f, 0.999f};
 __global__ void __launch_bounds__(256)
 sil_ladder_kernel(const __grid_constant__ CamConst cam, const float* __restrict__ image6, const float* __restrict__ gt_rgb,
                   const float* __restrict__ gt_depth, float* __restrict__ partials, unsigned int* __restrict__ ticket,
                   float* __restrict__ sums10) {
-    __shared__ float s_part[8][2 * LADDER_N];
-    __shared__ double s_sum[2 * LADDER_N][25];
-    __shared__ bool s_last;
+    __shared__ LastBlockSum<2 * LADDER_N> red;
     const size_t P = (size_t)cam.W * cam.H;
-    const size_t row_begin = (size_t)cam.row0 * 16 * cam.W;
-    const size_t row_end = min(P, (size_t)cam.row1 * 16 * cam.W);
+    size_t row_begin, row_end;
+    band_pixel_range(cam, row_begin, row_end);
     float sq[LADDER_N], cnt[LADDER_N];
 #pragma unroll
     for (int k = 0; k < LADDER_N; ++k) { sq[k] = 0.f; cnt[k] = 0.f; }
@@ -128,35 +117,10 @@ sil_ladder_kernel(const __grid_constant__ CamConst cam, const float* __restrict_
     for (int k = 0; k < LADDER_N; ++k) { sq[k] = warp_sum(sq[k]); cnt[k] = warp_sum(cnt[k]); }
     if (lane == 0) {
 #pragma unroll
-        for (int k = 0; k < LADDER_N; ++k) { s_part[warp][k] = sq[k]; s_part[warp][LADDER_N + k] = cnt[k]; }
+        for (int k = 0; k < LADDER_N; ++k) { red.part[warp][k] = sq[k]; red.part[warp][LADDER_N + k] = cnt[k]; }
     }
-    __syncthreads();
-    if (tid < 2 * LADDER_N) {
-        float s = 0.f;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) s += s_part[w][tid];
-        partials[(size_t)blockIdx.x * 2 * LADDER_N + tid] = s;
-        __threadfence();
-    }
-    __syncthreads();
-    if (tid == 0) s_last = atomicAdd(ticket, 1u) == gridDim.x - 1;
-    __syncthreads();
-    if (!s_last) return;
-    __threadfence();
-    const int nblocks = gridDim.x;
-    if (tid < 250) {
-        const int term = tid % (2 * LADDER_N), sl = tid / (2 * LADDER_N);          // 25 slices
-        double acc = 0.0;
-        for (int b = sl; b < nblocks; b += 25) acc += (double)__ldcg(&partials[(size_t)b * 2 * LADDER_N + term]);
-        s_sum[term][sl] = acc;
-    }
-    __syncthreads();
-    if (tid < 2 * LADDER_N) {
-        double a = 0.0;
-        for (int i = 0; i < 25; ++i) a += s_sum[tid][i];
-        sums10[tid] = (float)a;
-    }
-    if (tid == 0) *ticket = 0u;
+    if (!red.reduce(partials, ticket)) return;
+    if (tid < 2 * LADDER_N) sums10[tid] = (float)red.total(tid);
 }
 
 __global__ void sil_select_kernel(const float* __restrict__ sums10, float* __restrict__ thr_out, float* __restrict__ mse_out) {
@@ -208,21 +172,16 @@ ffma_probe_kernel(long long iters, float* __restrict__ sink) {
 }
 
 // Tracking loss (mode 0): sums of masked absolute differences; dL/dplane = w * sign * mask.
-// The block that finishes last performs the final reduction of the per-block partials (fixed slice order,
-// fp64: deterministic regardless of which block is last) -- no second launch.  `ticket` must be zero on
-// entry and is reset by the last block.
 __global__ void __launch_bounds__(256)
 tracking_loss_kernel(const __grid_constant__ CamConst cam, VtgsLossConfig cfg, const float* __restrict__ image6,
                      const float* __restrict__ gt_rgb, const float* __restrict__ gt_depth,
                      float* __restrict__ dL_dimage4, float* __restrict__ partials, unsigned int* __restrict__ ticket,
                      float* __restrict__ loss_terms, const unsigned int* __restrict__ median_state) {
     VTGS_PDL_PROLOGUE();
-    __shared__ float s_part[8][LOSS_TERMS];
-    __shared__ double s_sum[LOSS_TERMS][64];
-    __shared__ bool s_last;
+    __shared__ LastBlockSum<LOSS_TERMS> red;
     const size_t P = (size_t)cam.W * cam.H;
-    const size_t row_begin = (size_t)cam.row0 * 16 * cam.W;
-    const size_t row_end = min(P, (size_t)cam.row1 * 16 * cam.W);
+    size_t row_begin, row_end;
+    band_pixel_range(cam, row_begin, row_end);
     // outlier mask: depth_error < 50 * median(depth_error) (NaN median: nothing passes)
     const float outlier_thr = median_state ? 50.0f * __uint_as_float(__ldcg(median_state + 259)) : 0.0f;
     const float sil_thres = cfg.sil_thres_dev ? __ldcg(cfg.sil_thres_dev) : cfg.sil_thres;
@@ -267,33 +226,11 @@ tracking_loss_kernel(const __grid_constant__ CamConst cam, VtgsLossConfig cfg, c
     }
     ld = warp_sum(ld); li = warp_sum(li); cnt = warp_sum(cnt);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    if (lane == 0) { s_part[warp][0] = ld; s_part[warp][1] = li; s_part[warp][2] = cnt; s_part[warp][3] = 0.f; }
-    __syncthreads();
-    if (tid < LOSS_TERMS) {
-        float s = 0.f;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) s += s_part[w][tid];
-        partials[(size_t)blockIdx.x * LOSS_TERMS + tid] = s;
-        __threadfence();
-    }
-    __syncthreads();
-    if (tid == 0) s_last = atomicAdd(ticket, 1u) == gridDim.x - 1;
-    __syncthreads();
-    if (!s_last) return;
-    __threadfence();
-    const int nblocks = gridDim.x;
-    const int term = tid & (LOSS_TERMS - 1), sl = tid >> 2;           // 64 slices, coalesced
-    double acc = 0.0;
-    for (int b = sl; b < nblocks; b += 64) acc += (double)__ldcg(&partials[(size_t)b * LOSS_TERMS + term]);
-    s_sum[term][sl] = acc;
-    __syncthreads();
+    if (lane == 0) { red.part[warp][0] = ld; red.part[warp][1] = li; red.part[warp][2] = cnt; red.part[warp][3] = 0.f; }
+    if (!red.reduce(partials, ticket)) return;
     if (tid == 0) {
         double tot[LOSS_TERMS];
-        for (int k = 0; k < LOSS_TERMS; ++k) {
-            double a = 0.0;
-            for (int i = 0; i < 64; ++i) a += s_sum[k][i];
-            tot[k] = a;
-        }
+        for (int k = 0; k < LOSS_TERMS; ++k) tot[k] = red.total(k);
         const double wim = (double)cfg.w_im * tot[1], wd = (double)cfg.w_depth * tot[0];
         loss_terms[0] = (float)(wim + wd);
         loss_terms[1] = (float)wim;
@@ -303,7 +240,6 @@ tracking_loss_kernel(const __grid_constant__ CamConst cam, VtgsLossConfig cfg, c
         loss_terms[5] = 0.0f;
         loss_terms[6] = fmaxf(fabsf(cfg.w_im), fabsf(cfg.w_depth));      // >= |dL/dplane| everywhere: VtgsParamGrads.dL_abs_bound
         loss_terms[7] = 0.0f;
-        *ticket = 0u;
     }
 }
 
@@ -426,30 +362,21 @@ ssim_forward_kernel(int W, int H, const SsimWindow win, const float* __restrict_
     if (lane == 0) { s_part[warp][0] = l1; s_part[warp][1] = ld; s_part[warp][2] = cnt; s_part[warp][3] = ss; }
     __syncthreads();
     if (tid < MAP_TERMS) {
-        float a = 0.f;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) a += s_part[w][tid];
         const size_t b = ((size_t)blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x;
-        partials[b * MAP_TERMS + tid] = a;
+        partials[b * MAP_TERMS + tid] = warp_order_sum(s_part, tid);
     }
 }
 
+// The slice stage of the fixed-order sum (common.cuh) over ssim_forward_kernel's partials, then the loss terms.
 __global__ void __launch_bounds__(1024)
 mapping_finalize_kernel(const float* __restrict__ partials, int nblocks, int W, int H, VtgsLossConfig cfg, float* __restrict__ loss_terms) {
     VTGS_PDL_PROLOGUE();
     __shared__ double s_sum[MAP_TERMS][256];
     __shared__ double s_tot[MAP_TERMS];
     const int tid = threadIdx.x;
-    const int term = tid & (MAP_TERMS - 1), sl = tid >> 2;
-    double acc = 0.0;
-    for (int b = sl; b < nblocks; b += 256) acc += (double)partials[(size_t)b * MAP_TERMS + term];
-    s_sum[term][sl] = acc;
+    slice_sums<MAP_TERMS, 1024, false>(partials, nblocks, s_sum);
     __syncthreads();
-    if (tid < MAP_TERMS) {
-        double a = 0.0;
-        for (int i = 0; i < 256; ++i) a += s_sum[tid][i];
-        s_tot[tid] = a;
-    }
+    if (tid < MAP_TERMS) s_tot[tid] = slices_total(s_sum, tid);
     __syncthreads();
     if (tid == 0) {
         const double n3 = 3.0 * (double)W * (double)H;
@@ -547,18 +474,23 @@ ssim_backward_kernel(int W, int H, const SsimWindow win, VtgsLossConfig cfg, con
 
 // ---- re-tie a section's Gaussians to its optimised pose (reference src/vtgaussian_slam.py:2706-2727) ----
 // pts <- inv([R(q)|t]) * (w2c_old * pts), q/t read from the device (the pose the optimiser just updated).
+// R of an unnormalised pose quaternion: F.normalize, then build_rotation's second normalisation.  Plain fp32 that the
+// compiler may contract, so not pose_from_quat's spec'd order: the two give different bits.
+__device__ __forceinline__ void retie_rotation(const float* __restrict__ q_un, float* R) {
+    const float u0 = q_un[0], u1 = q_un[1], u2 = q_un[2], u3 = q_un[3];
+    const float n1 = fmaxf(sqrtf(u0 * u0 + u1 * u1 + u2 * u2 + u3 * u3), 1e-12f);
+    const float q0 = u0 / n1, q1 = u1 / n1, q2 = u2 / n1, q3 = u3 / n1;
+    const float n2 = sqrtf(q0 * q0 + q1 * q1 + q2 * q2 + q3 * q3);
+    quat_to_R(q0 / n2, q1 / n2, q2 / n2, q3 / n2, R);
+}
+
 struct Mat34 { float m[12]; };
 __global__ void __launch_bounds__(256)
 retie_kernel(float* __restrict__ means3D, int64_t n, const Mat34 old, const float* __restrict__ q_un, const float* __restrict__ t) {
     const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
     if (i >= n) return;
-    const float u0 = q_un[0], u1 = q_un[1], u2 = q_un[2], u3 = q_un[3];
-    const float n1 = fmaxf(sqrtf(u0 * u0 + u1 * u1 + u2 * u2 + u3 * u3), 1e-12f);
-    float q0 = u0 / n1, q1 = u1 / n1, q2 = u2 / n1, q3 = u3 / n1;
-    const float n2 = sqrtf(q0 * q0 + q1 * q1 + q2 * q2 + q3 * q3);
-    q0 /= n2; q1 /= n2; q2 /= n2; q3 /= n2;
     float R[9];
-    quat_to_R(q0, q1, q2, q3, R);
+    retie_rotation(q_un, R);
     const float x = means3D[3 * i], y = means3D[3 * i + 1], z = means3D[3 * i + 2];
     const float cx = old.m[0] * x + old.m[1] * y + old.m[2] * z + old.m[3] - t[0];
     const float cy = old.m[4] * x + old.m[5] * y + old.m[6] * z + old.m[7] - t[1];
@@ -574,20 +506,8 @@ retie_kernel(float* __restrict__ means3D, int64_t n, const Mat34 old, const floa
 __device__ __forceinline__ void retie_row(float* __restrict__ means3D, int64_t i, const float* __restrict__ q_old,
                                           const float* __restrict__ t_old, const float* __restrict__ q_un, const float* __restrict__ t) {
     float Ro[9], Rn[9];
-    {
-        const float u0 = q_old[0], u1 = q_old[1], u2 = q_old[2], u3 = q_old[3];
-        const float n1 = fmaxf(sqrtf(u0 * u0 + u1 * u1 + u2 * u2 + u3 * u3), 1e-12f);
-        float q0 = u0 / n1, q1 = u1 / n1, q2 = u2 / n1, q3 = u3 / n1;
-        const float n2 = sqrtf(q0 * q0 + q1 * q1 + q2 * q2 + q3 * q3);
-        quat_to_R(q0 / n2, q1 / n2, q2 / n2, q3 / n2, Ro);
-    }
-    {
-        const float u0 = q_un[0], u1 = q_un[1], u2 = q_un[2], u3 = q_un[3];
-        const float n1 = fmaxf(sqrtf(u0 * u0 + u1 * u1 + u2 * u2 + u3 * u3), 1e-12f);
-        float q0 = u0 / n1, q1 = u1 / n1, q2 = u2 / n1, q3 = u3 / n1;
-        const float n2 = sqrtf(q0 * q0 + q1 * q1 + q2 * q2 + q3 * q3);
-        quat_to_R(q0 / n2, q1 / n2, q2 / n2, q3 / n2, Rn);
-    }
+    retie_rotation(q_old, Ro);
+    retie_rotation(q_un, Rn);
     const float x = means3D[3 * i], y = means3D[3 * i + 1], z = means3D[3 * i + 2];
     const float cx = Ro[0] * x + Ro[1] * y + Ro[2] * z + t_old[0] - t[0];
     const float cy = Ro[3] * x + Ro[4] * y + Ro[5] * z + t_old[1] - t[1];
@@ -652,14 +572,6 @@ retie_records_kernel(const __grid_constant__ RecordTables tabs, int world, int r
     }
 }
 
-static inline size_t band_pixels(const CamConst& cam) {
-    const size_t P = (size_t)cam.W * cam.H;
-    const size_t b = (size_t)cam.row0 * 16 * cam.W;
-    size_t e = (size_t)cam.row1 * 16 * cam.W;
-    if (e > P) e = P;
-    return e > b ? e - b : 0;
-}
-
 // ---- Adam -----------------------------------------------------------------------------------
 // beta^t by repeated squaring in fp64: a dozen DMULs (pow() is microseconds of serial fp64 on this part,
 // paid as a prologue by every block).
@@ -670,6 +582,16 @@ __device__ __forceinline__ double ipow(double b, int t) {
         b *= b;
     }
     return r;
+}
+
+// torch.optim.Adam's update of one element; step_size = lr / (1 - b1^t), bc2s = sqrt(1 - b2^t)
+__device__ __forceinline__ void adam_update(float& p, const float g, float& m, float& v, float step_size, float bc2s, float b1,
+                                            float b2, float eps) {
+    const float mi = m + (1.0f - b1) * (g - m);                 // exp_avg.lerp_(grad, 1 - beta1)
+    const float vi = b2 * v + (1.0f - b2) * g * g;              // exp_avg_sq.mul_(b2).addcmul_(g, g, 1 - b2)
+    m = mi; v = vi;
+    const float denom = sqrtf(vi) / bc2s + eps;
+    p = p - step_size * (mi / denom);
 }
 
 __global__ void __launch_bounds__(256)
@@ -686,13 +608,7 @@ adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restric
     }
     __syncthreads();
     const float step_size = s_c[0], bc2s = s_c[1];
-    auto upd = [&](float& pi, const float gi, float& mi_, float& vi_) {
-        const float mi = mi_ + (1.0f - b1) * (gi - mi_);            // exp_avg.lerp_(grad, 1 - beta1)
-        const float vi = b2 * vi_ + (1.0f - b2) * gi * gi;          // exp_avg_sq.mul_(b2).addcmul_(g, g, 1 - b2)
-        mi_ = mi; vi_ = vi;
-        const float denom = sqrtf(vi) / bc2s + eps;
-        pi = pi - step_size * (mi / denom);
-    };
+    auto upd = [&](float& pi, const float gi, float& mi, float& vi) { adam_update(pi, gi, mi, vi, step_size, bc2s, b1, b2, eps); };
     const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
     if (vec4) {                                                      // four elements per thread, 16-byte accesses
         if (4 * i >= n) return;
@@ -725,6 +641,19 @@ struct ShardedAdamArgs {
     int nseg, world, rank;
 };
 
+// The sharded kernels' step constants (thread 0 of each block): lr[s] / (1 - b1^t) per segment s, and sqrt(1 - b2^t)
+__device__ __forceinline__ void sharded_adam_consts(const ShardedAdamArgs& a, float b1, float b2, int t, float (&step)[4], float& bc2s) {
+    const double bc1 = 1.0 - ipow((double)b1, t);
+    for (int k = 0; k < a.nseg; ++k) step[k] = (float)((double)a.lr[k] / bc1);
+    bc2s = (float)sqrt(1.0 - ipow((double)b2, t));
+}
+// the segment of flat element e, whose learning rate it takes
+__device__ __forceinline__ int segment_of(const ShardedAdamArgs& a, int64_t e) {
+    int sg = 0;
+    while (sg + 1 < a.nseg && e >= a.seg_end[sg]) ++sg;
+    return sg;
+}
+
 // W: ranks (compile-time: the peer loads of one element are issued together), U: float4 per thread and trip, so that
 // about eight remote 16-byte loads are in flight per thread whatever the world size (an NVLink round trip is ~3 us)
 template <int W, int U>
@@ -734,10 +663,7 @@ sharded_adam_kernel(const __grid_constant__ ShardedAdamArgs a, int64_t param_off
                     const int32_t* __restrict__ step_dev, float* __restrict__ loss_out) {
     __shared__ float s_step[4], s_bc2s;
     if (threadIdx.x == 0) {
-        const int t = *step_dev;
-        const double bc1 = 1.0 - ipow((double)b1, t);
-        for (int k = 0; k < a.nseg; ++k) s_step[k] = (float)((double)a.lr[k] / bc1);
-        s_bc2s = (float)sqrt(1.0 - ipow((double)b2, t));
+        sharded_adam_consts(a, b1, b2, *step_dev, s_step, s_bc2s);
         if (blockIdx.x == 0) {
             float L = 0.0f;
             for (int k = 0; k < a.world; ++k) L += reinterpret_cast<const float*>(a.base[k])[loss_off];
@@ -757,14 +683,8 @@ sharded_adam_kernel(const __grid_constant__ ShardedAdamArgs a, int64_t param_off
         pdst[k] = reinterpret_cast<float4*>(a.pbase[kk]) + param_off / 4;
     }
     const float4* my_p = reinterpret_cast<const float4*>(a.base[a.rank]) + param_off / 4;   // identical everywhere: local copy
-    auto upd = [&](float& pi, const float gi, float& mi_, float& vi_, int64_t e) {
-        int sg = 0;
-        while (sg + 1 < a.nseg && e >= a.seg_end[sg]) ++sg;
-        const float mi = mi_ + (1.0f - b1) * (gi - mi_);
-        const float vi = b2 * vi_ + (1.0f - b2) * gi * gi;
-        mi_ = mi; vi_ = vi;
-        const float denom = sqrtf(vi) / bc2s + eps;
-        pi = pi - s_step[sg] * (mi / denom);
+    auto upd = [&](float& pi, const float gi, float& mi, float& vi, int64_t e) {
+        adam_update(pi, gi, mi, vi, s_step[segment_of(a, e)], bc2s, b1, b2, eps);
     };
     const int64_t stride = (int64_t)gridDim.x * 256;
     for (int64_t j0 = begin + (int64_t)blockIdx.x * 256 + threadIdx.x; j0 < end; j0 += stride * U) {
@@ -804,10 +724,7 @@ sharded_adam_mc_kernel(const __grid_constant__ ShardedAdamArgs a, uint64_t mc_ba
                        const int32_t* __restrict__ step_dev, float* __restrict__ loss_out) {
     __shared__ float s_step[4], s_bc2s;
     if (threadIdx.x == 0) {
-        const int t = *step_dev;
-        const double bc1 = 1.0 - ipow((double)b1, t);
-        for (int k = 0; k < a.nseg; ++k) s_step[k] = (float)((double)a.lr[k] / bc1);
-        s_bc2s = (float)sqrt(1.0 - ipow((double)b2, t));
+        sharded_adam_consts(a, b1, b2, *step_dev, s_step, s_bc2s);
         if (blockIdx.x == 0) {
             float L;
             asm volatile("multimem.ld_reduce.relaxed.sys.global.add.f32 %0, [%1];" : "=f"(L) : "l"(reinterpret_cast<const float*>(mc_base) + loss_off) : "memory");
@@ -821,14 +738,8 @@ sharded_adam_mc_kernel(const __grid_constant__ ShardedAdamArgs a, uint64_t mc_ba
     const float4* mc_g = reinterpret_cast<const float4*>(mc_base) + grad_off / 4;
     float4* mc_p = reinterpret_cast<float4*>(mc_base) + param_off / 4;
     const float4* my_p = reinterpret_cast<const float4*>(a.base[a.rank]) + param_off / 4;
-    auto upd = [&](float& pi, const float gi, float& mi_, float& vi_, int64_t e) {
-        int sg = 0;
-        while (sg + 1 < a.nseg && e >= a.seg_end[sg]) ++sg;
-        const float mi = mi_ + (1.0f - b1) * (gi - mi_);
-        const float vi = b2 * vi_ + (1.0f - b2) * gi * gi;
-        mi_ = mi; vi_ = vi;
-        const float denom = sqrtf(vi) / bc2s + eps;
-        pi = pi - s_step[sg] * (mi / denom);
+    auto upd = [&](float& pi, const float gi, float& mi, float& vi, int64_t e) {
+        adam_update(pi, gi, mi, vi, s_step[segment_of(a, e)], bc2s, b1, b2, eps);
     };
     constexpr int U = 4;
     const int64_t stride = (int64_t)gridDim.x * 256;
@@ -881,12 +792,9 @@ __global__ void tracking_update_kernel(float* __restrict__ cam_q, float* __restr
     float* v = adam + (k < 4 ? 4 + k : 11 + (k - 4));
     const double bc1 = 1.0 - ipow((double)b1, s_step), bc2 = 1.0 - ipow((double)b2, s_step);
     const float step_size = (float)((double)(k < 4 ? lr_rot : lr_trans) / bc1);
-    const float mi = *m + (1.0f - b1) * (g - *m);
-    const float vi = b2 * *v + (1.0f - b2) * g * g;
-    *m = mi; *v = vi;
-    const float denom = sqrtf(vi) / (float)sqrt(bc2) + eps;
-    const float pn = *p - step_size * (mi / denom);
-    *p = pn;
+    float pn = *p, mi = *m, vi = *v;
+    adam_update(pn, g, mi, vi, step_size, (float)sqrt(bc2), b1, b2, eps);
+    *m = mi; *v = vi; *p = pn;
     if (s_better && (flags & VTGS_TRACK_BOOK_POST_STEP)) best[1 + k] = pn;
 }
 
@@ -931,8 +839,9 @@ int vtgs_loss(const VtgsCamera* camera, const VtgsLossConfig* cfg, const float* 
                         gt_depth, maps, loss_terms, dL_dimage4);
     }
     if (cfg->mode != 0) { set_error("unknown loss mode"); return VTGS_E_INVALID; }
-    const size_t npx = band_pixels(cam);
-    const int nblocks = (int)((npx + 256 * LOSS_PX_PER_THREAD - 1) / (256 * LOSS_PX_PER_THREAD));
+    size_t pix_b, pix_e;
+    band_pixel_range(cam, pix_b, pix_e);
+    const int nblocks = (int)((pix_e - pix_b + 256 * LOSS_PX_PER_THREAD - 1) / (256 * LOSS_PX_PER_THREAD));
     if (nblocks > 0) {
         unsigned int* ticket = reinterpret_cast<unsigned int*>(scratch + (size_t)nblocks * LOSS_TERMS);
         const unsigned int* median_state = nullptr;
